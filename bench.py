@@ -2,7 +2,7 @@
 """Benchmark of the hot path: one U2 Conformer training step (fwd + bwd + hybrid CTC/attention loss + gradient all-reduce +
 fused clip/Adam) on synthetic 80-dim fbank batches.  Metric: audio-seconds per second (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c1|c3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c1|c3] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One JSON line on rank 0.  `value` = whole-job audio-s/s with the batch resident in HBM (CUDA-graph replay, CUDA-event timed,
@@ -20,6 +20,7 @@ step over (at most) 126 utterances of the batch.  `--impl reference` runs only t
 from __future__ import annotations
 
 import argparse
+import contextlib
 import json
 import os
 import sys
@@ -122,9 +123,12 @@ def build_reference_step(wl, device, dropout: float, batch):
             return torch.nn.functional.dropout(x, p, True) if p > 0 else x
     dp = TorchDropper() if dropout > 0 else None
 
+    # on the GPU the oracle's factory calls (masks, position tables) must follow its inputs there
+    on_device = contextlib.nullcontext() if device.type == "cpu" else torch.device(device)
+
     def step(autocast=False):
         opt.zero_grad(set_to_none=True)
-        with torch.autocast(device_type=device.type, dtype=torch.bfloat16, enabled=autocast):
+        with torch.autocast(device_type=device.type, dtype=torch.bfloat16, enabled=autocast), on_device:
             if device.type == "cpu":
                 loss = O.hybrid_loss(sd, cfg, xs, xlens, ys, ylens, wl["ctc_weight"], wl["smoothing"], True, {}, dp)["loss"]
             else:
@@ -198,7 +202,7 @@ def cpu_oracle_run(wl, steps: int, warmup: int, sample_batch: int = 2, dropout: 
     batch = synth_batch(sample_batch, wl["tmax"], wl["lmax"], dims.vocab_size, seed=42)
     if reference_root() is None:
         from oracle import u2_oracle as O
-        O.build_c_oracle()
+        O._clib()  # compile (if needed) and load the C lattice before the timed steps
     one, kind = build_reference_step(wl, torch.device("cpu"), dropout, batch)
     for _ in range(max(0, warmup)):
         one()
@@ -217,11 +221,10 @@ def run_reference(args, wl):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 10))
-    r = cpu_oracle_run(wl, steps, max(1, min(args.warmup, 2)), sample_batch=8, dropout=args.dropout)
+    r = cpu_oracle_run(wl, args.steps, max(1, min(args.warmup, 2)), sample_batch=8, dropout=args.dropout)
     line = {
         "impl": "reference", "metric": "audio-sec/sec train (Conformer fwd+bwd+CTC)", "value": r["value"], "unit": "audio-s/s",
-        "n_gpus": args.gpus, "steps": steps, "warmup": max(1, min(args.warmup, 2)), "ms_per_step": r["ms_per_step"],
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": max(1, min(args.warmup, 2)), "ms_per_step": r["ms_per_step"],
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": wl["desc"], "parallelism": "cpu", "frame_shift_ms": 10, "dropout": args.dropout},
         "cpu_baseline": {"value": r["value"], "unit": "audio-s/s", "cores": r["cores"], "kind": r["kind"], "sample": r["sample"]},
@@ -546,6 +549,7 @@ def measure_step(args, wl, dev, dropout: float, rank: int, world: int, want_e2e:
             e2e_step()
         res["ms_e2e"] = timed(e2e_step, steps)
         res["h2d"] = sum(t.numel() * t.element_size() for t in host)
+        res["loss_last"] = loss_host
     if sampler:
         sampler.stop_flag = True
         sampler.join(timeout=1.0)
@@ -652,6 +656,33 @@ def gpu_incumbent(wl, dev, dropout: float, host_batch):
     return out
 
 
+DUMP_SAMPLE = 4 << 20  # parameter / gradient elements written by --dump-outputs: 2 x 16 MB in float32
+
+
+def dump_outputs(out_dir: str, model, optimizer, loss) -> None:
+    """What a caller of the timed step holds after its last step, as DIR/<name>.npy: the loss the call returned, its
+    [loss, CTC term, attention term], the updated parameters and their gradients (the same seeded sample of DUMP_SAMPLE
+    elements of all parameters concatenated in state_dict order: the whole model is larger than the dump's 64 MB), the
+    BatchNorm running statistics and the optimizer's [updates so far, gradient norm, learning rate] of that step (float64).
+    Same arguments, same inputs: two builds can be compared array by array.  The names are listed in .gitignore."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    params = [p for _, p in model.named_parameters()]
+    n = sum(p.numel() for p in params)
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values.to(params[0].device)
+    arrays = {
+        "loss": loss.float(),
+        "loss_terms": model.last_losses.float(),
+        "params_sample": torch.cat([p.detach().reshape(-1) for p in params])[idx],
+        "grads_sample": torch.cat([p.grad.reshape(-1) for p in params])[idx],
+        "bn_running_stats": torch.cat([b.reshape(-1).float() for k, b in model.state_dict().items() if "running" in k]),
+        "optimizer_state": optimizer.state[:3].double(),
+    }
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
+
+
 def run_gpu(args, wl):
     import torch
     import torch.distributed as dist
@@ -677,6 +708,8 @@ def run_gpu(args, wl):
 
     r = measure_step(args, wl, dev, args.dropout, rank, world, want_e2e=True, want_clocks=True, steps=args.steps)
     ms, audio, dims, step = r["ms"], r["audio"], r["dims"], r["step"]
+    if args.dump_outputs and rank == 0:  # before anything below runs another step on the same model
+        dump_outputs(args.dump_outputs, step.model, step.optimizer, r["loss_last"])
 
     # roofline of the dominant kernel family (tcgen05 GEMM), measured live with CUDA events
     flops, gemm_ms, n_gemm, split = gemm_family_replay(step, r["batch"], split=True)
@@ -807,7 +840,14 @@ def main():
     ap.add_argument("--no-ddp-check", action="store_true", help="skip the NCCL gradient / buffer numeric check that runs first at N > 1")
     ap.add_argument("--check-ddp-shapes", action="store_true", help="N > 1: also run TrainStep with rank-dependent batch shapes (graph capture at different steps)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed (loss, sampled parameters and gradients, "
+                         "BatchNorm statistics, optimizer step count / gradient norm / learning rate) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl b200)")
     wl = dict(WORKLOADS[args.workload])
     for k in WORKLOADS:
         WORKLOADS[k]["desc"] = WORKLOADS[k]["desc"].replace("dropout 0 (U2Config default)", f"dropout {args.dropout}")

@@ -16,9 +16,11 @@ torch build for most ops, float64 is used for tight pins).
 from __future__ import annotations
 
 import ctypes
+import hashlib
 import math
 import os
 import subprocess
+import tempfile
 from dataclasses import dataclass
 from typing import Dict, Optional, Tuple
 
@@ -379,13 +381,28 @@ _CLIB = None
 
 
 def build_c_oracle(force: bool = False) -> str:
-    """gcc -O2 oracle/ctc_oracle.c -> oracle/_build/libctc_oracle.so (plain C, no deps)."""
+    """gcc -O2 oracle/ctc_oracle.c -> oracle/_build/libctc_oracle.so (plain C, no deps).  In a read-only tree whose library
+    is missing or older than its source, the library goes to a private per-user cache directory under the system's temporary
+    directory instead, named after a hash of the source: built once, reused by later processes."""
     out_dir = os.path.join(_HERE, "_build")
     so = os.path.join(out_dir, "libctc_oracle.so")
     src = os.path.join(_HERE, "ctc_oracle.c")
-    if force or not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(src):
-        os.makedirs(out_dir, exist_ok=True)
-        subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", "-fopenmp", "-o", so, src, "-lm"])
+    if not force and os.path.exists(so) and os.path.getmtime(so) >= os.path.getmtime(src):
+        return so
+    if not os.access(out_dir if os.path.isdir(out_dir) else _HERE, os.W_OK):
+        out_dir = os.path.join(tempfile.gettempdir(), f"ctc_oracle-{os.getuid()}")
+        os.makedirs(out_dir, mode=0o700, exist_ok=True)
+        st = os.stat(out_dir)
+        if st.st_uid != os.getuid() or st.st_mode & 0o077:  # a library loaded from here must be this user's own
+            raise RuntimeError(f"{out_dir} is not a private directory of this user")
+        with open(src, "rb") as f:
+            so = os.path.join(out_dir, f"libctc_oracle-{hashlib.sha256(f.read()).hexdigest()[:16]}.so")
+        if not force and os.path.exists(so):
+            return so
+    os.makedirs(out_dir, exist_ok=True)
+    tmp = f"{so}.{os.getpid()}.tmp"  # concurrent builders each write their own file; the rename is atomic
+    subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", "-fopenmp", "-o", tmp, src, "-lm"])
+    os.replace(tmp, so)
     return so
 
 

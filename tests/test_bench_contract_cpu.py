@@ -5,6 +5,7 @@ import json
 import os
 import subprocess
 import sys
+from types import SimpleNamespace
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -30,3 +31,37 @@ def test_reference_arm_prints_the_contract_line_on_rank_0_only():
     assert d["gpu_launches"] == 0
     other = _run({"RANK": "1"})
     assert other.returncode == 0 and other.stdout.strip() == ""
+
+
+def test_dump_outputs_writes_a_fixed_sample_of_the_step_results(tmp_path, monkeypatch):
+    """--dump-outputs: arrays named after what the step returns (float32; the optimizer's counters float64); the parameter /
+    gradient sample is the same seeded set of positions in every run, in state_dict order, and holds the model's own values."""
+    import numpy as np
+    import torch
+    import bench
+    torch.manual_seed(0)
+    model = torch.nn.Sequential(torch.nn.Linear(6, 5), torch.nn.BatchNorm1d(5), torch.nn.Linear(5, 3))
+    with torch.no_grad():
+        for p in model.parameters():  # distinct values: a sampled value identifies its position
+            p.uniform_(-1.0, 1.0)
+    model(torch.randn(4, 6)).sum().backward()
+    model.last_losses = torch.tensor([3.0, 2.0, 4.0])
+    opt = SimpleNamespace(state=torch.tensor([7.0, 1.5, 2e-4, 0.0, 1.0, 0.0, 0.0, 0.0]))  # [updates, grad norm, lr, ...]
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 17)
+    bench.dump_outputs(str(tmp_path / "a"), model, opt, torch.tensor(3.0))
+    bench.dump_outputs(str(tmp_path / "b"), model, opt, torch.tensor(3.0))
+    names = {"loss", "loss_terms", "params_sample", "grads_sample", "bn_running_stats", "optimizer_state"}
+    assert {p.name for p in (tmp_path / "a").iterdir()} == {n + ".npy" for n in names}
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in names}
+    for n in names:
+        assert got[n].dtype == (np.float64 if n == "optimizer_state" else np.float32), n
+        assert np.array_equal(got[n], np.load(tmp_path / "b" / f"{n}.npy")), n
+    assert got["loss"] == 3.0 and got["loss_terms"].tolist() == [3.0, 2.0, 4.0]
+    assert got["optimizer_state"].tolist() == opt.state[:3].double().tolist()
+    flat_p = torch.cat([p.detach().reshape(-1) for p in model.parameters()]).numpy()
+    flat_g = torch.cat([p.grad.reshape(-1) for p in model.parameters()]).numpy()
+    assert got["params_sample"].shape == got["grads_sample"].shape == (17,)
+    pos = [int(np.flatnonzero(flat_p == v)[0]) for v in got["params_sample"]]
+    assert pos == sorted(set(pos)) and np.array_equal(flat_g[pos], got["grads_sample"])
+    bn = model[1]
+    assert np.array_equal(got["bn_running_stats"], torch.cat([bn.running_mean, bn.running_var]).numpy())

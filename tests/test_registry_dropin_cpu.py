@@ -2,14 +2,21 @@
 (/root/reference/liteasr/models/__init__.py:53-86, criterions/__init__.py:28-56) loaded through ``oracle/ref_shims.py``.
 
 Runs in a fresh interpreter (import order matters: ``liteasr_b200.config`` derives its dataclasses from
-``liteasr.config.LiteasrDataclass`` when LiteASR is importable at that moment).  Skipped where the reference tree does not exist
-(the GPU box)."""
+``liteasr.config.LiteasrDataclass`` when LiteASR is importable at that moment).  Skipped where no copy of the upstream LiteASR
+source tree is found (``oracle/ref_shims.py``: ``LITEASR_REFERENCE_ROOT``).
+
+The state_dict half of that check also runs without the upstream tree, against what the unmodified reference model recorded
+when the golden files were generated (``oracle/make_golden.py``): its parameter names in ``named_parameters()`` order with
+their shapes (``f64.grads``) and its BatchNorm buffers (``f64.bn``, ``f64.nbt``), for three model sizes."""
+import json
 import os
 import subprocess
 import sys
 import textwrap
 
 import pytest
+
+from oracle import ref_shims
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -98,9 +105,29 @@ print("DROPIN-OK")
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/liteasr/nets"), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not ref_shims.reference_available(), reason="needs the upstream LiteASR source tree (LITEASR_REFERENCE_ROOT)")
 @pytest.mark.parametrize("dropout", [0.1])
 def test_integration_md_section1_against_unmodified_reference_registry(dropout):
     src = f"ROOT = {ROOT!r}\nDROPOUT = {dropout!r}\n" + textwrap.dedent(SCRIPT)
     r = subprocess.run([sys.executable, "-c", src], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0 and "DROPIN-OK" in r.stdout, r.stdout[-3000:] + r.stderr[-3000:]
+
+
+@pytest.mark.parametrize("case", ["tiny", "tiny_odd", "c1"])
+def test_state_dict_schema_matches_the_reference_recording(case):
+    """Parameter names, order and shapes and the BatchNorm buffers of the product's U2 are the unmodified reference model's, as
+    recorded in tests/golden/u2_<case>.json (enc / dec layers 2 / 2, 1 / 1 and 4 / 6).  The recording holds no dtypes and no
+    position tables, so those two stay with the live check above."""
+    from liteasr_b200.models.u2 import U2, U2Config
+    with open(os.path.join(ROOT, "tests", "golden", f"u2_{case}.json")) as f:
+        g = json.load(f)
+    rec = g["f64"]
+    model = U2(U2Config(**g["dims"]))
+    assert [(k, list(p.shape)) for k, p in model.named_parameters()] == [(k, v["shape"]) for k, v in rec["grads"].items()]
+    sd = model.state_dict()
+    for group in (rec["bn"], rec["nbt"]):
+        assert [k for k in sd if k in group] == list(group)
+    assert all(list(sd[k].shape) == v["shape"] for k, v in rec["bn"].items())
+    # the sinusoid position tables are the only entries the recording does not list
+    recorded = set(rec["grads"]) | set(rec["bn"]) | set(rec["nbt"])
+    assert all(k.endswith(".pe.pe") for k in sd if k not in recorded)

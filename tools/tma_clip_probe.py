@@ -1,5 +1,5 @@
-import torch, sys
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from liteasr_b200 import ops
 for cdt in (torch.bfloat16, torch.float32):
     for n in (299, 297, 290):
