@@ -283,6 +283,11 @@ int lasr_scale_by_scalar(void* x, int dtype, int64_t n, const float* scalar, voi
  * ------------------------------------------------------------------------------------------------ */
 int lasr_glu_dwconv_fwd(const void* y2, int dtype, int64_t ldy, const float* w, const float* bias, float* z, float* partial,
                         int B, int T, int d, void* stream);
+/* glu_dwconv_fwd_lens: the same with per-utterance lengths lens (B,) int64 (sub-sampled frames, clamped to [0,T]): GLU outputs
+ * of rows t >= lens[b] read as zero, the Conv1d zero padding of a batch-1 call on the utterance cut to lens[b] frames.  Rows
+ * t < lens[b] of z then do not depend on the padded rows; rows t >= lens[b] hold finite values.  Inference only: no backward. */
+int lasr_glu_dwconv_fwd_lens(const void* y2, int dtype, int64_t ldy, const float* w, const float* bias, float* z, float* partial,
+                             int B, int T, int d, const int64_t* lens, void* stream);
 int lasr_bn_finalize(const float* partial, int nblk, int d, int64_t count, float eps, float momentum, float* mean, float* rstd,
                      float* running_mean, float* running_var, int64_t* num_batches_tracked, int training, void* stream);
 int lasr_bn_swish_fwd(const float* z, const float* mean, const float* rstd, const float* gamma, const float* beta, void* a,
@@ -326,7 +331,11 @@ int lasr_conv2_wgrad(const void* dy2p, const void* h1p, float* dw2k, int B, int 
  * (dscores = p*(dp - sum p*dp)*scale; dbd = inverse shift of dscores, NULL for plain attention).
  * ac/bd/dprobs (B,H,Tq,ld) of s_dtype: fp32, or bf16 when probs are bf16 (what torch autocast's matmul hands to the softmax;
  * halves the score traffic); probs/dscores/dbd fp32|bf16 (B,H,Tq,ld); columns [Tk,ld) are zeroed.
- * mask_mode: 0 none | 1 klen=lens[b] | 2 klen=lens[b]+1 | 3 klen=#{j: 4j<lens[b]} (encoder sub-sampled mask).
+ * mask_mode: 0 none | 1 klen=lens[b] | 2 klen=lens[b]+1 | 3 klen=#{j: 4j<lens[b]} (encoder sub-sampled mask) |
+ *            4 klen=lens[b] with the legacy shift run over klen instead of Tk (forward only, no backward counterpart):
+ *              bdshift[i,j] = bd[i, klen-1-(i-j)] (j <= i) | 0 (j == i+1) | bd[i+1, j-i-2] (i+1 < j < klen), keys j >= klen -1e38;
+ *              rows i < klen then equal the maskless batch-1 call on the utterance cut to klen frames (per-utterance inference
+ *              on a padded batch), rows i >= klen get finite values without the rel-pos term.
  * ------------------------------------------------------------------------------------------------ */
 int lasr_attn_softmax_fwd(const void* ac, const void* bd, int s_dtype, void* probs, int p_dtype, const int64_t* lens, int mask_mode,
                           int causal, float scale, int B, int H, int Tq, int Tk, int ld, void* stream);
@@ -392,6 +401,14 @@ int lasr_zero(void* ptr, size_t bytes, void* stream);
  *   ctc_prefix_beam_search : HOST function (no device work): u2.py:224-261 on host copies of top_val / top_idx for ONE
  *                     utterance; float64 arithmetic in the reference's operation order, insertion-ordered prefix map, stable
  *                     sort.  Outputs up to `beam` hypotheses best first: tokens (beam,max_len) padded -1, lengths, scores.
+ *   ctc_prefix_beam_search_batch : the same search on the DEVICE for a ragged batch in one launch, no host synchronisation,
+ *                     deterministic.  top_val / top_idx (B*Tmax, K) as logsoftmax_topk emits them (utterance b at rows
+ *                     [b*Tmax, b*Tmax + frames[b])), frames (B,) int64 (clamped to [0,Tmax]).  Outputs: tokens
+ *                     (B,beam,max_len) padded -1 (max_len >= Tmax), lengths (B,beam), float64 scores (B,beam) (-inf beyond
+ *                     the count), hypothesis counts (B,).  1 <= K <= 64, 1 <= beam <= 32.  workspace: at least
+ *                     ctc_prefix_beam_search_batch_workspace(B, Tmax, beam) bytes (the prefix-node pools).  Float64 with CUDA's
+ *                     exp / log (<= 1 ulp): scores may differ from the host function's in the last bits, and two hypotheses
+ *                     whose scores lie within a few ulps may come out in the other order.
  * ------------------------------------------------------------------------------------------------ */
 int lasr_logsoftmax_topk(const void* logits, int dtype, int64_t ld, int64_t rows, int V, int K, float* lse, float* logp_full,
                          int64_t ldf, float* top_val, int32_t* top_idx, void* stream);
@@ -399,6 +416,10 @@ int lasr_gather_logp(const void* logits, int dtype, int64_t ld, const float* lse
                      void* stream);
 int lasr_ctc_prefix_beam_search(const float* topk_logp, const int32_t* topk_idx, int frames, int K, int beam, int blank,
                                 int32_t* out_tokens, int32_t* out_lens, double* out_scores, int max_len, int32_t* n_out);
+size_t lasr_ctc_prefix_beam_search_batch_workspace(int B, int Tmax, int beam);
+int lasr_ctc_prefix_beam_search_batch(const float* top_val, const int32_t* top_idx, const int64_t* frames, int B, int Tmax, int K, int beam,
+                                      int blank, int32_t* out_tokens, int32_t* out_lens, double* out_scores, int32_t* out_n, int max_len,
+                                      void* workspace, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * SpecAugment on a padded batch (utils/transform/spec_augment.py:19-125; SURVEY 8f N3), out of place.

@@ -55,6 +55,7 @@ def lib() -> C.CDLL:
         _lib = C.CDLL(LIB_PATH)
         _lib.lasr_last_error.restype = C.c_char_p
         _lib.lasr_ctc_workspace_bytes.restype = C.c_size_t
+        _lib.lasr_ctc_prefix_beam_search_batch_workspace.restype = C.c_size_t
         _lib.lasr_launch_count.restype = C.c_ulonglong
     return _lib
 

@@ -7,7 +7,9 @@
 //         bdshift[i,j] = bd[i, Tk-1-(i-j)] (j <= i) | 0 (j == i+1) | bd[i+1, j-i-2] (j > i+1)      (quirk Q1)
 //   bwd : ds = p * (dp - sum_j p*dp) * scale  -> dac ; dbd = the same values scattered through the inverse shift (same pass)
 // Key mask: key j of batch b is valid iff j < klen(b);  klen mode: 0 none, 1 lens[b], 2 lens[b]+1,
-// 3 #{j : 4j < lens[b]} (the encoder's mask[:, :-2:2][:, :-2:2] of a padding mask, nets/transformer_encoder.py:118).
+// 3 #{j : 4j < lens[b]} (the encoder's mask[:, :-2:2][:, :-2:2] of a padding mask, nets/transformer_encoder.py:118),
+// 4 lens[b] with the legacy shift taken over klen instead of Tk (per-utterance inference on a padded batch: every valid row equals
+// the maskless batch-1 call on the utterance cut to its length; rows i >= klen get finite values without the rel-pos term).
 // Masked scores are -1e38 exactly like masked_fill (no -inf, no post-softmax zeroing: quirk Q4).
 #include "common.cuh"
 
@@ -39,7 +41,7 @@ template <> __device__ __forceinline__ float2 load_pair<bf16>(const bf16* p) {
 
 // One warp per score row; lane l owns the column pairs (2l + 64e, 2l + 64e + 1), e < NP (Tk <= 64 NP): 64-bit loads of ac,
 // 32/64-bit stores of the probabilities, NP sized to the problem so the kernel runs at full occupancy.  ld must be even.
-template <typename TP, typename TS, int NP>
+template <typename TP, typename TS, int NP, bool RAGGED = false>
 __global__ void __launch_bounds__(256) attn_softmax_fwd_kernel(const TS* __restrict__ ac, const TS* __restrict__ bd,
                                                                TP* __restrict__ probs, const int64_t* __restrict__ lens,
                                                                int mask_mode, int causal, float scale, int B, int H, int Tq,
@@ -50,7 +52,7 @@ __global__ void __launch_bounds__(256) attn_softmax_fwd_kernel(const TS* __restr
     if (row >= (long)B * H * Tq) return;
     const int i = (int)(row % Tq);
     const int b = (int)(row / ((long)H * Tq));
-    const int klen = key_len(lens, mask_mode, b, Tk);
+    const int klen = RAGGED ? key_len(lens, 1, b, Tk) : key_len(lens, mask_mode, b, Tk);
     const TS* ar = ac + row * ld;
     const TS* br = bd ? bd + row * ld : nullptr;  // bd row i of the same (b,h); row i+1 is br + ld
     float2 s[NP];
@@ -62,7 +64,13 @@ __global__ void __launch_bounds__(256) attn_softmax_fwd_kernel(const TS* __restr
         if (j < Tk) {
             float2 v = load_pair<TS>(ar + j);
             const bool two = j + 1 < Tk;
-            if (br) {
+            if (RAGGED) {
+                // the shift over klen: bd[i, klen-1-(i-j)] (j <= i) | 0 (j == i+1) | bd[i+1, j-i-2] (i+1 < j < klen)
+                if (br && i < klen) {
+                    if (j < klen) v.x += (j <= i) ? to_f32<TS>(br[klen - 1 - i + j]) : ((j > i + 1) ? to_f32<TS>(br[ld + j - i - 2]) : 0.f);
+                    if (j + 1 < klen) v.y += (j + 1 <= i) ? to_f32<TS>(br[klen - i + j]) : ((j > i) ? to_f32<TS>(br[ld + j - i - 1]) : 0.f);
+                }
+            } else if (br) {
                 // legacy rel_shift: bd[i, Tk-1-(i-j)] (j <= i) | 0 (j == i+1) | bd[i+1, j-i-2] (j > i+1)
                 v.x += (j <= i) ? to_f32<TS>(br[Tk - 1 - i + j]) : ((j > i + 1) ? to_f32<TS>(br[ld + j - i - 2]) : 0.f);
                 if (two) v.y += (j + 1 <= i) ? to_f32<TS>(br[Tk - i + j]) : ((j > i) ? to_f32<TS>(br[ld + j - i - 1]) : 0.f);
@@ -165,16 +173,36 @@ using namespace lasr;
         else launch_pdl(KERNEL<TP, TS, SM_MAXP>, grid, 256, 0, st, __VA_ARGS__);             \
     } while (0)
 
+// mask mode 4: the RAGGED instantiations of the forward kernel
+#define LASR_SM_DISPATCH_RAGGED(TP, TS, ...)                                                               \
+    do {                                                                                                    \
+        if (Tk <= 64) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 1, true>, grid, 256, 0, st, __VA_ARGS__);          \
+        else if (Tk <= 128) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 2, true>, grid, 256, 0, st, __VA_ARGS__);    \
+        else if (Tk <= 320) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 5, true>, grid, 256, 0, st, __VA_ARGS__);    \
+        else if (Tk <= 448) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 7, true>, grid, 256, 0, st, __VA_ARGS__);    \
+        else launch_pdl(attn_softmax_fwd_kernel<TP, TS, SM_MAXP, true>, grid, 256, 0, st, __VA_ARGS__);             \
+    } while (0)
+
 int lasr_attn_softmax_fwd(const void* ac, const void* bd, int s_dtype, void* probs, int p_dtype, const int64_t* lens, int mask_mode,
                           int causal, float scale, int B, int H, int Tq, int Tk, int ld, void* stream) {
     LASR_REQUIRE(ac && probs && B > 0 && H > 0 && Tq > 0 && Tk > 0 && ld >= Tk && ld <= 64 * SM_MAXP && ld % 2 == 0,
                  "attn_softmax_fwd: bad args (Tk <= ld <= 1024, ld even)");
     LASR_REQUIRE(!bd || Tq == Tk, "attn_softmax_fwd: rel_shift needs Tq == Tk");
-    LASR_REQUIRE(mask_mode >= 0 && mask_mode <= 3 && (mask_mode == 0 || lens), "attn_softmax_fwd: bad mask mode");
+    LASR_REQUIRE(mask_mode >= 0 && mask_mode <= 4 && (mask_mode == 0 || lens), "attn_softmax_fwd: bad mask mode");
     LASR_REQUIRE(((uintptr_t)ac & 7) == 0 && ((uintptr_t)probs & 7) == 0, "attn_softmax_fwd: unaligned");
     const long rows = (long)B * H * Tq;
     cudaStream_t st = (cudaStream_t)stream;
     const int grid = ceil_div(rows, 8);
+    if (mask_mode == 4) {
+        if (p_dtype == LASR_F32 && s_dtype == LASR_F32)
+            LASR_SM_DISPATCH_RAGGED(float, float, (const float*)ac, (const float*)bd, (float*)probs, lens, mask_mode, causal, scale, B, H, Tq, Tk, ld);
+        else if (p_dtype == LASR_BF16 && s_dtype == LASR_F32)
+            LASR_SM_DISPATCH_RAGGED(bf16, float, (const float*)ac, (const float*)bd, (bf16*)probs, lens, mask_mode, causal, scale, B, H, Tq, Tk, ld);
+        else if (p_dtype == LASR_BF16 && s_dtype == LASR_BF16)
+            LASR_SM_DISPATCH_RAGGED(bf16, bf16, (const bf16*)ac, (const bf16*)bd, (bf16*)probs, lens, mask_mode, causal, scale, B, H, Tq, Tk, ld);
+        else { set_error("attn_softmax_fwd: unsupported dtype combination"); return LASR_ERR_UNSUPPORTED; }
+        return check_launch("attn_softmax_fwd");
+    }
     if (p_dtype == LASR_F32 && s_dtype == LASR_F32)
         LASR_SM_DISPATCH(attn_softmax_fwd_kernel, float, float, (const float*)ac, (const float*)bd, (float*)probs, lens, mask_mode, causal, scale, B, H, Tq, Tk, ld);
     else if (p_dtype == LASR_BF16 && s_dtype == LASR_F32)

@@ -199,6 +199,16 @@ __device__ __noinline__ void ctl_pv_mma_store(const Ctl& c, const CUtensorMap* m
     bulk_commit();
 }
 
+// mask mode 4 (RAGGED): klen = lens[b] and the flat re-view runs over klen instead of T -- bd row r written at r (klen+1) + 1 + c
+// for c < klen only (columns >= klen are products of real P rows here), shifted row read at r klen + j -- so that every valid
+// row equals the batch-1 call on the utterance cut to klen frames.  Query rows >= klen drop the rel-pos term (their reads
+// would reach flat positions no bd row of the tile wrote) and keep finite values.
+__device__ __forceinline__ int ragged_len(const Params& p, int tt) {
+    const long l = p.lens[(tt / p.tiles) / p.H];
+    return (int)(l < p.T ? (l < 0 ? 0 : l) : p.T);
+}
+
+template <bool RAGGED>
 __global__ void __launch_bounds__(THREADS, 1)
 rel_attn_fwd_kernel(const __grid_constant__ CUtensorMap m_qu, const __grid_constant__ CUtensorMap m_qv,
                     const __grid_constant__ CUtensorMap m_k, const __grid_constant__ CUtensorMap m_v,
@@ -288,18 +298,19 @@ rel_attn_fwd_kernel(const __grid_constant__ CUtensorMap m_qu, const __grid_const
             epi_barrier();
             FA_STAMP(2);
             const int r0 = (tt % p.tiles) * TOUT;
-            const int off = r * (T + 1) + r0 - T;  // flat position of the padded zero of bd row g
+            const int W = RAGGED ? ragged_len(p, tt) : T;  // length the shift runs over
+            const int off = r * (W + 1) + r0 - W;  // flat position of the padded zero of bd row g
             if (part == 0) flat[off] = 0;
             uint16_t* dst = flat + off + 1 + cb;
-            // T odd: the row stride T + 1 is even, so every lane of the warp has the same 4-byte alignment and pairs of
+            // W odd: the row stride W + 1 is even, so every lane of the warp has the same 4-byte alignment and pairs of
             // halves go out as 32-bit stores (the phase is bound by shared-memory store wavefronts)
-            const int par = (T & 1) ? ((off + 1 + cb) & 1) : 2;  // 0 aligned | 1 off by one half | 2 per-lane (scalar stores)
+            const int par = (W & 1) ? ((off + 1 + cb) & 1) : 2;  // 0 aligned | 1 off by one half | 2 per-lane (scalar stores)
 #pragma unroll
             for (int ch = 0; ch < PARTW / CH; ++ch) {
                 const int c0 = cb + ch * CH;
                 const float* v = sv + ch * CH;
                 uint16_t* d = dst + ch * CH;
-                if (c0 + CH <= T) {  // warp-uniform
+                if (c0 + CH <= W) {  // warp-uniform
                     if (par == 0) {
 #pragma unroll
                         for (int e = 0; e < CH; e += 2) *reinterpret_cast<uint32_t*>(d + e) = f16x2_sat(v[e] * c2, v[e + 1] * c2);
@@ -316,12 +327,12 @@ rel_attn_fwd_kernel(const __grid_constant__ CUtensorMap m_qu, const __grid_const
                             d[e + 1] = (uint16_t)(h2 >> 16);
                         }
                     }
-                } else if (c0 < T) {  // columns >= T are zero products of the zero-filled P rows: they must not reach the next row's slots
+                } else if (c0 < W) {  // columns >= W (zero products of the zero-filled P rows when W = T) must not reach the next row's slots
 #pragma unroll
                     for (int e = 0; e < CH; e += 2) {
                         const uint32_t h2 = f16x2_sat(v[e] * c2, v[e + 1] * c2);
-                        if (c0 + e < T) d[e] = (uint16_t)(h2 & 0xffffu);
-                        if (c0 + e + 1 < T) d[e + 1] = (uint16_t)(h2 >> 16);
+                        if (c0 + e < W) d[e] = (uint16_t)(h2 & 0xffffu);
+                        if (c0 + e + 1 < W) d[e + 1] = (uint16_t)(h2 >> 16);
                     }
                 }
             }
@@ -363,14 +374,17 @@ rel_attn_fwd_kernel(const __grid_constant__ CUtensorMap m_qu, const __grid_const
             // shifted row r starts at half r T + cb of the flat buffer: aligned 32-bit loads from the word below and a funnel
             // shift by the lane's own parity (row stride T may be odd) instead of 16-bit loads
             int klen = T;
-            if (p.mask_mode != 0 && p.lens) {
+            if (RAGGED) {
+                klen = ragged_len(p, tt);
+            } else if (p.mask_mode != 0 && p.lens) {
                 const long l = p.lens[(tt / p.tiles) / p.H];
                 long k = l;
                 if (p.mask_mode == 2) k = l + 1;
                 else if (p.mask_mode == 3) k = (l + 3) / 4;
                 klen = (int)(k < T ? (k < 0 ? 0 : k) : T);
             }
-            const int h0 = r * T + cb;
+            const int h0 = r * (RAGGED ? klen : T) + cb;
+            const bool qpad = RAGGED && (tt % p.tiles) * TOUT + r >= klen;  // padded query row: no rel-pos term
             const int fpar = h0 & 1;
             const uint32_t* src = reinterpret_cast<const uint32_t*>(flat + (h0 - fpar));
             const uint32_t fsh = 16u * (uint32_t)fpar;
@@ -385,7 +399,8 @@ rel_attn_fwd_kernel(const __grid_constant__ CUtensorMap m_qu, const __grid_const
 #pragma unroll
                 for (int k = 0; k < CH / 2; ++k) {
                     const uint32_t pr = __funnelshift_r(w[k], w[k + 1], fsh);
-                    const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&pr));
+                    float2 f = __half22float2(*reinterpret_cast<const __half2*>(&pr));
+                    if (RAGGED && qpad) f = make_float2(0.f, 0.f);
                     float s0 = fmaf(v[2 * k], c2, f.x), s1 = fmaf(v[2 * k + 1], c2, f.y);
                     if (!clean) {
                         const int j = j0 + 2 * k;
@@ -560,7 +575,7 @@ int lasr_rel_attn_fwd(const void* qu, const void* qv, long ldq, const void* k, c
         return LASR_ERR_UNSUPPORTED;
     }
     LASR_REQUIRE(ld >= T && ld % 8 == 0 && ld <= fa::TKMAX, "rel_attn_fwd: ld must be a multiple of 8 in [T, %d]", fa::TKMAX);
-    LASR_REQUIRE(mask_mode >= 0 && mask_mode <= 3 && (mask_mode == 0 || lens), "rel_attn_fwd: bad mask mode");
+    LASR_REQUIRE(mask_mode >= 0 && mask_mode <= 4 && (mask_mode == 0 || lens), "rel_attn_fwd: bad mask mode");
     LASR_REQUIRE(ldo % 8 == 0 && (reinterpret_cast<uintptr_t>(o) & 15) == 0 && (reinterpret_cast<uintptr_t>(probs) & 15) == 0,
                  "rel_attn_fwd: O and probs must be 16-byte aligned");
     const long d = (long)H * dk;
@@ -574,7 +589,8 @@ int lasr_rel_attn_fwd(const void* qu, const void* qv, long ldq, const void* k, c
     if ((rc = fa::make_map(&m_probs, probs, ld, T, ld, (long)B * H, (long)T * ld, fa::TOUT, true)) != LASR_OK) return rc;
     static bool configured = false;
     if (!configured) {
-        if (cudaFuncSetAttribute(fa::rel_attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fa::SMEM_BYTES) != cudaSuccess)
+        if (cudaFuncSetAttribute(fa::rel_attn_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fa::SMEM_BYTES) != cudaSuccess ||
+            cudaFuncSetAttribute(fa::rel_attn_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fa::SMEM_BYTES) != cudaSuccess)
             return check_launch("rel_attn_fwd smem attr");
         configured = true;
     }
@@ -594,8 +610,12 @@ int lasr_rel_attn_fwd(const void* qu, const void* qv, long ldq, const void* k, c
     }
     const long total = (long)p.tiles * H * B;
     const int grid = (int)(total < sms ? total : sms);  // persistent: one CTA per SM walks the (batch, head, row tile) list
-    launch_pdl(fa::rel_attn_fwd_kernel, dim3((unsigned)grid), dim3(fa::THREADS), (size_t)fa::SMEM_BYTES,
-               (cudaStream_t)stream, m_qu, m_qv, m_k, m_v, m_p, m_probs, p);
+    if (mask_mode == 4)
+        launch_pdl(fa::rel_attn_fwd_kernel<true>, dim3((unsigned)grid), dim3(fa::THREADS), (size_t)fa::SMEM_BYTES,
+                   (cudaStream_t)stream, m_qu, m_qv, m_k, m_v, m_p, m_probs, p);
+    else
+        launch_pdl(fa::rel_attn_fwd_kernel<false>, dim3((unsigned)grid), dim3(fa::THREADS), (size_t)fa::SMEM_BYTES,
+                   (cudaStream_t)stream, m_qu, m_qv, m_k, m_v, m_p, m_probs, p);
     return check_launch("rel_attn_fwd");
 }
 

@@ -35,11 +35,19 @@ template <> __device__ __forceinline__ void st2<bf16>(bf16* p, float a, float b)
 }
 
 // ---------------------------------------------------------------- fwd 1
-template <typename TD>
+// LENS (lasr_glu_dwconv_fwd_lens): GLU outputs of rows t >= lens[b] read as zero -- the Conv1d zero padding the batch-1 call on
+// the utterance cut to lens[b] frames sees -- so that rows t < lens[b] do not depend on the padded rows.
+__device__ __forceinline__ int valid_rows(const int64_t* lens, int b, int T) {
+    const long l = lens[b];
+    return (int)(l < T ? (l < 0 ? 0 : l) : T);
+}
+
+template <typename TD, bool LENS = false>
 __global__ void __launch_bounds__(128) glu_dwconv_fwd_generic(const TD* __restrict__ y2, long ldy, const float* __restrict__ w,
                                                              const float* __restrict__ bias, float* __restrict__ z,
-                                                             float* __restrict__ partial, int T, int d) {
+                                                             float* __restrict__ partial, int T, int d, const int64_t* __restrict__ lens) {
     const int b = blockIdx.y, chunk = blockIdx.x, nchunk = gridDim.x;
+    const int Tv = LENS ? valid_rows(lens, b, T) : T;
     const int t0 = chunk * TCH, t1 = min(T, t0 + TCH);
     float* part = partial + ((long)(b * nchunk + chunk)) * 2 * d;
     for (int c = threadIdx.x * 2; c < d; c += blockDim.x * 2) {
@@ -50,7 +58,7 @@ __global__ void __launch_bounds__(128) glu_dwconv_fwd_generic(const TD* __restri
         float s0 = 0.f, s1 = 0.f, q0 = 0.f, q1 = 0.f;
         for (int tt = t0 - HALO; tt < t1 + HALO; ++tt) {
             float g0 = 0.f, g1 = 0.f;
-            if (tt >= 0 && tt < T) {
+            if (tt >= 0 && tt < Tv) {
                 const TD* row = y2 + ((long)b * T + tt) * ldy;
                 const float2 v = ld2<TD>(row + c), gt = ld2<TD>(row + d + c);
                 g0 = v.x * sigmoidf_(gt.x);
@@ -228,10 +236,10 @@ template <> __device__ __forceinline__ float4 ld4c<bf16>(const bf16* p) {
 
 // ---------------------------------------------------------------- fwd 1 (fast)
 // partial rows keep the 32-step granularity of the ABI: a CTA writes one row per 32-step half of its tile.
-template <typename TD>
+template <typename TD, bool LENS = false>
 __global__ void __launch_bounds__(256, 4) glu_dwconv_fwd_kernel(const TD* __restrict__ y2, long ldy, const float* __restrict__ w,
                                                                 const float* __restrict__ bias, float* __restrict__ z,
-                                                                float* __restrict__ partial, int T, int d) {
+                                                                float* __restrict__ partial, int T, int d, const int64_t* __restrict__ lens) {
     LASR_PDL_SYNC();
     __shared__ __align__(16) float gt[FWIN][FC];
     __shared__ float wt[FC * KW];
@@ -249,7 +257,7 @@ __global__ void __launch_bounds__(256, 4) glu_dwconv_fwd_kernel(const TD* __rest
             const int r = rbase + 16 * it, tt = t0 - HALO + r;
             v[it] = make_float4(0.f, 0.f, 0.f, 0.f);
             gate[it] = v[it];
-            if (r < FWIN && tt >= 0 && tt < T && cok) {
+            if (r < FWIN && tt >= 0 && tt < (LENS ? valid_rows(lens, b, T) : T) && cok) {
                 const TD* row = y2 + ((long)b * T + tt) * ldy + c0 + cv;
                 v[it] = ld4c<TD>(row);
                 gate[it] = ld4c<TD>(row + d);
@@ -338,9 +346,10 @@ __device__ __forceinline__ uint32_t pack_bf2(float a, float b) {
 __device__ __forceinline__ float bf16lo(uint32_t u) { return __uint_as_float(u << 16); }
 __device__ __forceinline__ float bf16hi(uint32_t u) { return __uint_as_float(u & 0xffff0000u); }
 
+template <bool LENS = false>
 __global__ void __launch_bounds__(256, 4) glu_dwconv_fwd_stream_kernel(const bf16* __restrict__ y2, long ldy, const float* __restrict__ w,
                                                                        const float* __restrict__ bias, float* __restrict__ z,
-                                                                       float* __restrict__ partial, int T, int d) {
+                                                                       float* __restrict__ partial, int T, int d, const int64_t* __restrict__ lens) {
     LASR_PDL_SYNC();
     __shared__ __align__(16) bf16 raw[SSTG][2][SR][SCH];
     __shared__ __align__(16) float ring[SRING][SCH];
@@ -348,12 +357,13 @@ __global__ void __launch_bounds__(256, 4) glu_dwconv_fwd_stream_kernel(const bf1
     __shared__ float red[2][4][SCH];
     const int b = blockIdx.y, c0 = blockIdx.x * SCH, tid = threadIdx.x;
     const int nch = (T + SR - 1) / SR;
+    const int Tv = LENS ? valid_rows(lens, b, T) : T;
     const int lrow = tid >> 3, lpc = (tid & 7) * 8;     // loader / GLU role: one row, 8 channels
     const int c = tid & (SCH - 1), rg = tid >> 6;       // convolution role: one channel, 8 rows
     const bf16* src0 = y2 + (long)b * T * ldy + c0 + lpc;
     auto issue = [&](int j) {
         const int t = j * SR + lrow;
-        const bool ok = j < nch && t < T;
+        const bool ok = j < nch && t < Tv;
         const bf16* sp = src0 + (long)(ok ? t : 0) * ldy;
         cp_async16(&raw[j % SSTG][0][lrow][lpc], sp, ok);
         cp_async16(&raw[j % SSTG][1][lrow][lpc], sp + d, ok);
@@ -700,30 +710,44 @@ using namespace lasr;
 static inline bool fast_d(int d) { return d % 4 == 0; }
 static inline bool pow2_rows(int d) { const int v = d / 4; return d % 4 == 0 && v >= 1 && v <= 256 && (v & (v - 1)) == 0; }
 
-/* partial: B * ceil(T/32) * 2 * d floats */
-int lasr_glu_dwconv_fwd(const void* y2, int dtype, int64_t ldy, const float* w, const float* bias, float* z, float* partial,
-                        int B, int T, int d, void* stream) {
+extern "C++" {
+template <bool LENS>
+static int glu_dwconv_fwd_launch(const void* y2, int dtype, int64_t ldy, const float* w, const float* bias, float* z, float* partial,
+                                 int B, int T, int d, const int64_t* lens, void* stream) {
     LASR_REQUIRE(y2 && w && bias && z && partial && B > 0 && T > 0 && d > 0 && d % 2 == 0 && ldy % 2 == 0, "glu_dwconv_fwd: bad args");
     cudaStream_t st = (cudaStream_t)stream;
     const bool fast = fast_d(d) && ldy % 4 == 0 && ((uintptr_t)y2 & 15) == 0 && ((uintptr_t)z & 15) == 0;
     static int stream_on = -1;  // LASR_CONVMOD_STREAM=0: developer switch back to the tiled kernels
     if (stream_on < 0) { const char* e = getenv("LASR_CONVMOD_STREAM"); stream_on = e ? atoi(e) : 1; }
     if (stream_on && dtype == LASR_BF16 && d % SCH == 0 && ldy % 8 == 0 && ((uintptr_t)y2 & 15) == 0) {
-        launch_pdl(glu_dwconv_fwd_stream_kernel, dim3(d / SCH, B), 256, 0, st, (const bf16*)y2, ldy, w, bias, z, partial, T, d);
+        launch_pdl(glu_dwconv_fwd_stream_kernel<LENS>, dim3(d / SCH, B), 256, 0, st, (const bf16*)y2, ldy, w, bias, z, partial, T, d, lens);
         return check_launch("glu_dwconv_fwd");
     }
     if (fast) {
         dim3 grid(ceil_div(T, FT), B, ceil_div(d, FC));
-        if (dtype == LASR_F32) launch_pdl(glu_dwconv_fwd_kernel<float>, grid, 256, 0, st, (const float*)y2, ldy, w, bias, z, partial, T, d);
-        else if (dtype == LASR_BF16) launch_pdl(glu_dwconv_fwd_kernel<bf16>, grid, 256, 0, st, (const bf16*)y2, ldy, w, bias, z, partial, T, d);
+        if (dtype == LASR_F32) launch_pdl(glu_dwconv_fwd_kernel<float, LENS>, grid, 256, 0, st, (const float*)y2, ldy, w, bias, z, partial, T, d, lens);
+        else if (dtype == LASR_BF16) launch_pdl(glu_dwconv_fwd_kernel<bf16, LENS>, grid, 256, 0, st, (const bf16*)y2, ldy, w, bias, z, partial, T, d, lens);
         else { set_error("glu_dwconv_fwd: bad dtype"); return LASR_ERR_UNSUPPORTED; }
     } else {
         dim3 grid(ceil_div(T, TCH), B);
-        if (dtype == LASR_F32) glu_dwconv_fwd_generic<float><<<grid, 128, 0, st>>>((const float*)y2, ldy, w, bias, z, partial, T, d);
-        else if (dtype == LASR_BF16) glu_dwconv_fwd_generic<bf16><<<grid, 128, 0, st>>>((const bf16*)y2, ldy, w, bias, z, partial, T, d);
+        if (dtype == LASR_F32) glu_dwconv_fwd_generic<float, LENS><<<grid, 128, 0, st>>>((const float*)y2, ldy, w, bias, z, partial, T, d, lens);
+        else if (dtype == LASR_BF16) glu_dwconv_fwd_generic<bf16, LENS><<<grid, 128, 0, st>>>((const bf16*)y2, ldy, w, bias, z, partial, T, d, lens);
         else { set_error("glu_dwconv_fwd: bad dtype"); return LASR_ERR_UNSUPPORTED; }
     }
     return check_launch("glu_dwconv_fwd");
+}
+}  // extern "C++"
+
+/* partial: B * ceil(T/32) * 2 * d floats */
+int lasr_glu_dwconv_fwd(const void* y2, int dtype, int64_t ldy, const float* w, const float* bias, float* z, float* partial,
+                        int B, int T, int d, void* stream) {
+    return glu_dwconv_fwd_launch<false>(y2, dtype, ldy, w, bias, z, partial, B, T, d, nullptr, stream);
+}
+
+int lasr_glu_dwconv_fwd_lens(const void* y2, int dtype, int64_t ldy, const float* w, const float* bias, float* z, float* partial,
+                             int B, int T, int d, const int64_t* lens, void* stream) {
+    LASR_REQUIRE(lens, "glu_dwconv_fwd_lens: lens is required");
+    return glu_dwconv_fwd_launch<true>(y2, dtype, ldy, w, bias, z, partial, B, T, d, lens, stream);
 }
 
 int lasr_bn_finalize(const float* partial, int nblk, int d, int64_t count, float eps, float momentum, float* mean, float* rstd,

@@ -8,6 +8,8 @@
 //                               sequential dictionary algorithm in float64 Python arithmetic in the reference; it is restated
 //                               here in C++ with the same operation order (libm exp/log, left-to-right sums, insertion-ordered
 //                               map, stable sort), so n-best lists and scores are bit-identical given the same log-probs.
+//   lasr_ctc_prefix_beam_search_batch (device) the same search for a ragged batch in one launch, one warp per utterance;
+//                               float64 with CUDA's exp / log, so scores may differ from the host's in the last bits.
 #include <cmath>
 #include <cstring>
 #include <algorithm>
@@ -15,6 +17,8 @@
 #include <string>
 #include <unordered_map>
 #include <vector>
+
+#include <math_constants.h>
 
 #include "common.cuh"
 
@@ -114,6 +118,260 @@ static std::string key_of(const std::vector<int32_t>& p) {
     return std::string(reinterpret_cast<const char*>(p.data()), p.size() * sizeof(int32_t));
 }
 
+// ---------------------------------------------------------------------------------------------
+// device: CTC prefix beam search over a ragged batch, one warp (one CTA) per utterance
+// ---------------------------------------------------------------------------------------------
+// The host function below restated operation for operation.  A prefix is a node (parent, token) of a per-utterance pool; only
+// hypotheses that survive a prune get one, at id t * beam + rank.  Per frame:
+//   1. contributions in the host's loop order (j over the K classes, h over the beam), placed by a warp scan: each carries the
+//      key of the entry it updates -- h' < beam for a prefix already in the beam (h itself, or h' = h + s when such a
+//      hypothesis exists), beam + pair for a new extension (top_idx holds distinct classes, so those are all distinct)
+//   2. lane h' folds the contributions of key h' in loop order through the same log_add; an extension has one contribution
+//   3. entries are numbered by first touch; rank = stable descending sort by log_add(pb, pnb); rank < beam survives
+// Exact arithmetic: float64 with CUDA's exp / log (<= 1 ulp, not glibc's), so scores may differ from the host's in the last
+// bits and two hypotheses within a few ulps of each other may swap.
+constexpr int PB_MAX_BEAM = 32, PB_MAX_K = 64;
+
+// log_add of (a0, a1) or (a0, a1, a2): the host's operation order with scalar arguments (no local-memory array)
+__device__ __forceinline__ double log_add_d(double a0, double a1, double a2, bool three) {
+    const double ninf = -CUDART_INF;
+    if (a0 == ninf && a1 == ninf && (!three || a2 == ninf)) return ninf;
+    double a_max = fmax(a0, a1);
+    if (three) a_max = fmax(a_max, a2);
+    double s = 0.0;
+    s += exp(a0 - a_max);
+    s += exp(a1 - a_max);
+    if (three) s += exp(a2 - a_max);
+    return a_max + log(s);
+}
+
+struct PbBeam {  // one hypothesis of the beam
+    double pb, pnb;
+    int node, len, last;  // node -1 = empty prefix; last = its final token (-1 if empty)
+};
+
+// Shared-memory layout of one CTA (sizes from K and beam)
+struct PbSmem {
+    PbBeam* cur;
+    PbBeam* nxt;
+    int* ckey;       // [2 K beam]  entry key of a contribution
+    int* cmeta;      // [2 K beam]  field (bit 0: 0 pb / 1 pnb) | term count (bit 1: 3 terms) | pair index << 2
+    double* cterm;   // [2 K beam][2]
+    int* cflag;      // [2 K beam]  entry id of a first touch, -1 otherwise
+    double* ev;      // [K beam + beam][3]  pb, pnb, score of each entry
+    int* ekey;       // [K beam + beam]     key of the entry, and the contribution that created it (new extensions)
+    int* esrc;
+};
+
+__host__ __device__ inline size_t pb_smem_bytes(int K, int beam) {
+    const size_t nc = 2 * (size_t)K * beam, ne = (size_t)K * beam + beam;
+    return 2 * beam * sizeof(PbBeam) + nc * (3 * sizeof(int) + 2 * sizeof(double)) + ne * (3 * sizeof(double) + 2 * sizeof(int)) + 64;
+}
+
+// prefix(a) == prefix(b) for two nodes of equal length: equal ids end the walk (a prefix can own two nodes when it was pruned
+// and re-created while one of its extensions survived)
+__device__ __forceinline__ bool same_prefix(const int2* pool, int a, int b) {
+    while (a != b) {
+        if (a < 0 || b < 0) return false;
+        const int2 na = pool[a], nb = pool[b];
+        if (na.y != nb.y) return false;
+        a = na.x;
+        b = nb.x;
+    }
+    return true;
+}
+
+__global__ void __launch_bounds__(32) ctc_prefix_beam_search_kernel(const float* __restrict__ top_val, const int* __restrict__ top_idx,
+                                                                    const int64_t* __restrict__ frames, int Tmax, int K, int beam,
+                                                                    int blank, int2* __restrict__ pool_all, int32_t* __restrict__ out_tokens,
+                                                                    int32_t* __restrict__ out_lens, double* __restrict__ out_scores,
+                                                                    int32_t* __restrict__ out_n, int max_len) {
+    extern __shared__ __align__(16) uint8_t pb_raw[];
+    const int b = blockIdx.x, lane = threadIdx.x;
+    const int nc_max = 2 * K * beam, ne_max = K * beam + beam;
+    PbSmem S;
+    {
+        uint8_t* p = pb_raw;
+        S.cur = reinterpret_cast<PbBeam*>(p); p += beam * sizeof(PbBeam);
+        S.nxt = reinterpret_cast<PbBeam*>(p); p += beam * sizeof(PbBeam);
+        S.cterm = reinterpret_cast<double*>(p); p += (size_t)nc_max * 2 * sizeof(double);
+        S.ev = reinterpret_cast<double*>(p); p += (size_t)ne_max * 3 * sizeof(double);
+        S.ckey = reinterpret_cast<int*>(p); p += nc_max * sizeof(int);
+        S.cmeta = reinterpret_cast<int*>(p); p += nc_max * sizeof(int);
+        S.cflag = reinterpret_cast<int*>(p); p += nc_max * sizeof(int);
+        S.ekey = reinterpret_cast<int*>(p); p += ne_max * sizeof(int);
+        S.esrc = reinterpret_cast<int*>(p);
+    }
+    long nf = frames[b];
+    nf = nf < 0 ? 0 : (nf > Tmax ? Tmax : nf);
+    int2* pool = pool_all + (long)b * Tmax * beam;
+    const float* tv = top_val + (long)b * Tmax * K;
+    const int* ti = top_idx + (long)b * Tmax * K;
+    if (lane == 0) S.cur[0] = PbBeam{0.0, -CUDART_INF, -1, 0, -1};
+    int nh = 1;
+    __syncwarp();
+    for (int t = 0; t < nf; ++t) {
+        // ---- 1. contributions in loop order
+        const int npairs = K * nh;
+        int nc = 0;
+        for (int q0 = 0; q0 < npairs; q0 += 32) {
+            const int q = q0 + lane;
+            int cnt = 0, s = -1, h = 0;
+            double ps = 0.0;
+            if (q < npairs) {
+                const int j = q / nh;
+                h = q - j * nh;
+                s = ti[(long)t * K + j];
+                ps = (double)tv[(long)t * K + j];
+                if (s >= 0) cnt = (s != blank && s == S.cur[h].last) ? 2 : 1;
+            }
+            int incl = cnt;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int v = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += v;
+            }
+            int pos = nc + incl - cnt;
+            if (cnt > 0) {
+                const PbBeam hy = S.cur[h];
+                if (s == blank) {  // *  -> *   (pb)
+                    S.ckey[pos] = h; S.cmeta[pos] = 0 | 2 | (q << 2);
+                    S.cterm[2 * pos] = hy.pb + ps; S.cterm[2 * pos + 1] = hy.pnb + ps;
+                } else {
+                    if (cnt == 2) {  // *s -> *s  (pnb)
+                        S.ckey[pos] = h; S.cmeta[pos] = 1 | (q << 2);
+                        S.cterm[2 * pos] = hy.pnb + ps;
+                        ++pos;
+                    }
+                    // the extension prefix(h) + s: a hypothesis of the beam already, or a new entry
+                    int key = beam + q;
+                    for (int h2 = 0; h2 < nh; ++h2) {
+                        const PbBeam& o = S.cur[h2];
+                        if (o.len == hy.len + 1 && o.last == s && same_prefix(pool, pool[o.node].x, hy.node)) { key = h2; break; }
+                    }
+                    S.ckey[pos] = key;
+                    if (cnt == 2) {  // *s-s -> *ss  (pnb, two terms)
+                        S.cmeta[pos] = 1 | (q << 2);
+                        S.cterm[2 * pos] = hy.pb + ps;
+                    } else {         // *  -> *s  (pnb, three terms)
+                        S.cmeta[pos] = 1 | 2 | (q << 2);
+                        S.cterm[2 * pos] = hy.pb + ps; S.cterm[2 * pos + 1] = hy.pnb + ps;
+                    }
+                }
+            }
+            nc += __shfl_sync(0xffffffffu, incl, 31);
+        }
+        __syncwarp();
+        // ---- 2. folds in loop order: lane h' for the beam's own prefixes, any lane for a new extension
+        double fpb = -CUDART_INF, fpnb = -CUDART_INF;
+        int first = 0x7fffffff;
+        if (lane < nh) {
+            for (int c = 0; c < nc; ++c) {
+                if (S.ckey[c] != lane) continue;
+                first = min(first, c);
+                const int m = S.cmeta[c];
+                const double r = log_add_d((m & 1) ? fpnb : fpb, S.cterm[2 * c], S.cterm[2 * c + 1], (m & 2) != 0);
+                if (m & 1) fpnb = r; else fpb = r;
+            }
+        }
+        for (int c = lane; c < nc; c += 32) S.cflag[c] = S.ckey[c] >= beam ? 1 : 0;
+        __syncwarp();
+        if (lane < nh && first != 0x7fffffff) S.cflag[first] = 1;
+        __syncwarp();
+        // entry ids = scan of the first-touch flags
+        int ne = 0;
+        for (int c0 = 0; c0 < nc; c0 += 32) {
+            const int c = c0 + lane;
+            const int f = c < nc ? S.cflag[c] : 0;
+            int incl = f;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int v = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += v;
+            }
+            if (f) {
+                const int e = ne + incl - 1;
+                const int key = S.ckey[c];
+                S.ekey[e] = key;
+                S.esrc[e] = c;
+                if (key >= beam) {
+                    const int m = S.cmeta[c];
+                    S.ev[3 * e] = -CUDART_INF;
+                    S.ev[3 * e + 1] = log_add_d(-CUDART_INF, S.cterm[2 * c], S.cterm[2 * c + 1], (m & 2) != 0);
+                }
+            }
+            ne += __shfl_sync(0xffffffffu, incl, 31);
+        }
+        __syncwarp();
+        // the folds of the beam's own prefixes live in lanes h': publish them at the entry of their first touch
+        if (lane < nh && first != 0x7fffffff) {
+            int e = 0;
+            for (; e < ne; ++e) if (S.esrc[e] == first) break;
+            S.ev[3 * e] = fpb;
+            S.ev[3 * e + 1] = fpnb;
+        }
+        __syncwarp();
+        for (int e = lane; e < ne; e += 32) {
+            S.ev[3 * e + 2] = log_add_d(S.ev[3 * e], S.ev[3 * e + 1], 0.0, false);
+        }
+        __syncwarp();
+        // ---- 3. stable descending sort by score (ties: first touch first); the best `beam` survive
+        const int nkeep = min(beam, ne);
+        for (int e = lane; e < ne; e += 32) {
+            const double sc = S.ev[3 * e + 2];
+            int rank = 0;
+            for (int e2 = 0; e2 < ne && rank < beam; ++e2) {
+                const double s2 = S.ev[3 * e2 + 2];
+                rank += (s2 > sc || (s2 == sc && e2 < e)) ? 1 : 0;
+            }
+            if (rank < beam) {
+                const int key = S.ekey[e];
+                PbBeam nh_;
+                nh_.pb = S.ev[3 * e];
+                nh_.pnb = S.ev[3 * e + 1];
+                if (key < beam) {
+                    const PbBeam& o = S.cur[key];
+                    nh_.node = o.node; nh_.len = o.len; nh_.last = o.last;
+                } else {
+                    const int q = S.cmeta[S.esrc[e]] >> 2;
+                    const int j = q / nh, h = q - j * nh;
+                    const int s = ti[(long)t * K + j];
+                    const int id = t * beam + rank;
+                    pool[id] = make_int2(S.cur[h].node, s);
+                    nh_.node = id; nh_.len = S.cur[h].len + 1; nh_.last = s;
+                }
+                S.nxt[rank] = nh_;
+            }
+        }
+        __syncwarp();
+        for (int i = lane; i < nkeep; i += 32) S.cur[i] = S.nxt[i];
+        nh = nkeep;
+        __syncwarp();
+    }
+    // ---- output: tokens by walking the parent links
+    for (int i = lane; i < beam; i += 32) {
+        int32_t* row = out_tokens + ((long)b * beam + i) * max_len;
+        if (i < nh) {
+            const PbBeam hy = S.cur[i];
+            const int len = min(hy.len, max_len);
+            for (int j = len; j < max_len; ++j) row[j] = -1;
+            int nd = hy.node;
+            for (int j = hy.len - 1; j >= 0; --j) {
+                const int2 n = pool[nd];
+                if (j < max_len) row[j] = n.y;
+                nd = n.x;
+            }
+            out_lens[(long)b * beam + i] = hy.len;
+            out_scores[(long)b * beam + i] = log_add_d(hy.pb, hy.pnb, 0.0, false);
+        } else {
+            for (int j = 0; j < max_len; ++j) row[j] = -1;
+            out_lens[(long)b * beam + i] = 0;
+            out_scores[(long)b * beam + i] = -CUDART_INF;
+        }
+    }
+    if (lane == 0) out_n[b] = nh;
+}
+
 }  // namespace lasr
 
 extern "C" {
@@ -137,6 +395,28 @@ int lasr_gather_logp(const void* logits, int dtype, int64_t ld, const float* lse
     else if (dtype == LASR_BF16) gather_logp_kernel<bf16><<<ceil_div(rows, 256), 256, 0, st>>>((const bf16*)logits, ld, lse, tokens, out, rows, V);
     else { set_error("gather_logp: bad dtype"); return LASR_ERR_UNSUPPORTED; }
     return check_launch("gather_logp");
+}
+
+size_t lasr_ctc_prefix_beam_search_batch_workspace(int B, int Tmax, int beam) {
+    return (B > 0 && Tmax > 0 && beam > 0) ? (size_t)B * Tmax * beam * sizeof(int2) : 0;
+}
+
+int lasr_ctc_prefix_beam_search_batch(const float* top_val, const int32_t* top_idx, const int64_t* frames, int B, int Tmax, int K, int beam,
+                                      int blank, int32_t* out_tokens, int32_t* out_lens, double* out_scores, int32_t* out_n, int max_len,
+                                      void* workspace, size_t ws_bytes, void* stream) {
+    LASR_REQUIRE(top_val && top_idx && frames && out_tokens && out_lens && out_scores && out_n && B > 0 && Tmax > 0 && max_len >= Tmax,
+                 "ctc_prefix_beam_search_batch: bad args (max_len must be >= Tmax)");
+    LASR_REQUIRE(K >= 1 && K <= PB_MAX_K && beam >= 1 && beam <= PB_MAX_BEAM, "ctc_prefix_beam_search_batch: needs 1 <= K <= %d, 1 <= beam <= %d",
+                 PB_MAX_K, PB_MAX_BEAM);
+    LASR_REQUIRE(workspace && ws_bytes >= lasr_ctc_prefix_beam_search_batch_workspace(B, Tmax, beam),
+                 "ctc_prefix_beam_search_batch: workspace too small");
+    const size_t smem = pb_smem_bytes(K, beam);
+    if (smem > 48 * 1024 &&
+        cudaFuncSetAttribute(ctc_prefix_beam_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        return check_launch("ctc_prefix_beam_search_batch smem attr");
+    ctc_prefix_beam_search_kernel<<<B, 32, smem, (cudaStream_t)stream>>>(top_val, top_idx, frames, Tmax, K, beam, blank, (int2*)workspace,
+                                                                         out_tokens, out_lens, out_scores, out_n, max_len);
+    return check_launch("ctc_prefix_beam_search_batch");
 }
 
 /* HOST function: topk_logp / topk_idx are host arrays (frames, K), row-major, classes in the order the device kernel emits

@@ -7,9 +7,17 @@
                               reference's operation order (``lasr_ctc_prefix_beam_search``).
 * ``attention_rescore``       models/u2.py:269-317: one decoder pass over the padded n-best, the (beam, L, V) log-softmax is never
                               materialised (row log-sum-exp + ``lasr_gather_logp``), scores summed left to right in fp32.
-* ``inference_batch``         the same result for a list of utterances: encoders run one by one (bit-identical to the batch-1
-                              reference call: BatchNorm running statistics, no padding), ONE decoder pass rescoring every n-best
-                              of every utterance (memory padded + masked by its true length).
+* ``decode_batch``            a padded batch in ONE encoder pass with per-utterance semantics (attention mask mode 4 and the
+                              length-aware depthwise conv: every valid row equals the maskless batch-1 call on the utterance cut
+                              to its length), one top-K over all rows, the prefix search for every utterance in one device launch
+                              (``lasr_ctc_prefix_beam_search_batch``), one copy of the n-best to the host, ONE decoder pass
+                              rescoring every n-best of every utterance (memory masked by its sub-sampled length).
+* ``inference_batch``         a list of utterances through the same encoder pass and top-K, with the host search per utterance:
+                              token- and score-identical to calling ``attention_rescore`` one by one.
+
+``greedy_ctc(xs, xlens)`` keeps the reference's padded-batch semantics (mask mode 3, the padded rows inside the depthwise conv
+window), so its tokens can differ from those of a batch-1 call; ``decode_batch(...)["greedy"]`` has per-utterance semantics and
+equals ``greedy_ctc(x_b, None)`` on each utterance.
 
 Everything runs under ``torch.no_grad()`` on the hand-written CUDA kernels; there is no CPU fallback.
 """
@@ -47,6 +55,15 @@ def _encode(model, xs: Tensor, xlens: Optional[Tensor]):
     return enc.out, head.out, enc.Tp
 
 
+def _greedy_rows(ids, n: int, blank: int) -> List[int]:
+    """Frame ids -> greedy CTC tokens: the first n frames, repeats collapsed, blanks dropped."""
+    row = ids[:n]
+    keep = np.ones(len(row), dtype=bool)
+    keep[1:] = row[1:] != row[:-1]
+    keep &= row != blank
+    return [int(v) for v in row[keep]]
+
+
 @torch.no_grad()
 def greedy_ctc(model, xs: Tensor, xlens: Optional[Tensor] = None) -> Tuple[List[List[int]], Tensor]:
     """xs (B,T,F); xlens (B,) or None (maskless, every frame decoded).  -> (token lists, frame ids (B,T') int32)."""
@@ -58,14 +75,7 @@ def greedy_ctc(model, xs: Tensor, xlens: Optional[Tensor] = None) -> Tuple[List[
     ids = idx.view(B, Tp)
     host = ids.cpu().numpy()
     n = [Tp] * B if xlens is None else [int(v) for v in model.get_pred_len(xlens.cpu())]
-    out = []
-    for b in range(B):
-        row = host[b, : n[b]]
-        keep = np.ones(len(row), dtype=bool)
-        keep[1:] = row[1:] != row[:-1]
-        keep &= row != model.blank
-        out.append([int(v) for v in row[keep]])
-    return out, ids
+    return [_greedy_rows(host[b], n[b], model.blank) for b in range(B)], ids
 
 
 @torch.no_grad()
@@ -87,10 +97,11 @@ def ctc_prefix_beam_search(model, x: Tensor, beam: int = BEAM):
 
 
 @torch.no_grad()
-def _rescore(model, nbest: Sequence[Sequence[Tuple[tuple, float]]], mems: Sequence[Tensor]):
-    """One decoder pass over every hypothesis of every utterance.  nbest[u] = [(prefix, ctc score)], mems[u] = (1,T'_u,d).
-    -> per utterance (best index, [scores])."""
-    dev = mems[0].device
+def _rescore(model, nbest: Sequence[Sequence[Tuple[tuple, float]]], mem: Tensor, mlens: Optional[Tensor]):
+    """One decoder pass over every hypothesis of every utterance.  nbest[u] = [(prefix, ctc score)]; mem (n,T',d) fp32 holds the
+    encoder output each of the n hypotheses attends to, mlens (n,) its key lengths (None: every key, memory_mask=None as in
+    models/u2.py:297).  -> per utterance (best index, [scores])."""
+    dev = mem.device
     st, eng, _ = F.bind(model, dev)
     F.bind(model.decoder, dev)
     flat = [(u, hy) for u, hyps in enumerate(nbest) for hy in hyps]
@@ -107,20 +118,6 @@ def _rescore(model, nbest: Sequence[Sequence[Tuple[tuple, float]]], mems: Sequen
             toks[i, 1:L + 1] = hy[0]
             look[i, :L] = hy[0]
         look[i, L] = model.eos
-    tmax = max(m.shape[1] for m in mems)
-    d = mems[0].shape[2]
-    single = len(mems) == 1
-    if single:
-        mem = mems[0].expand(n, tmax, d).contiguous()            # h.repeat(len(hyps), 1, 1)  (models/u2.py:273)
-        mlens = None                                              # memory_mask=None (:297)
-    else:
-        mem = torch.zeros((n, tmax, d), dtype=torch.float32, device=dev)
-        ml = np.zeros(n, dtype=np.int64)
-        for i, (u, _) in enumerate(flat):
-            t = mems[u].shape[1]
-            mem[i, :t] = mems[u][0]
-            ml[i] = t
-        mlens = torch.from_numpy(ml).to(dev)
     model.decoder.pe.ensure(lmax + 1, dev)
     c = eng.decoder_fwd(model.decoder, torch.from_numpy(toks).to(dev), torch.from_numpy(ylens).to(dev), mem, mlens, mem_mask_mode=1)
     V = model.vocab_size
@@ -145,21 +142,81 @@ def _rescore(model, nbest: Sequence[Sequence[Tuple[tuple, float]]], mems: Sequen
 def attention_rescore(model, x: Tensor, beam: int = BEAM, return_details: bool = False):
     """models/u2.py:269-317 for one utterance x (1,T,F) -> best hypothesis (list of token ids)."""
     hyps, h = _prefix_search(model, x, beam)
-    (best, scores), = _rescore(model, [hyps], [h])
+    (best, scores), = _rescore(model, [hyps], h.expand(len(hyps), -1, -1).contiguous(), None)  # h.repeat(len(hyps), 1, 1) (u2.py:273)
     if return_details:
         return dict(best=list(hyps[best][0]), hyps=hyps, scores=scores)
     return list(hyps[best][0])
 
 
+@torch.no_grad()
+def _ragged_topk(model, xs: Tensor, xlens, beam: int):
+    """Per-utterance encoder pass over a padded batch + one top-K over every row.
+    -> (h (B,T'max,d) fp32, top_val / top_idx (B*T'max, K), T'_b list, T'_b device tensor, T'max)."""
+    if model.training:
+        raise RuntimeError("inference runs on the BatchNorm running statistics: call model.eval() first")
+    if xs.dim() != 3:
+        raise ValueError("xs must be a padded batch (B, T, F)")
+    B, T = xs.shape[0], xs.shape[1]
+    lens = [int(v) for v in torch.as_tensor(xlens).reshape(-1).cpu()]
+    if len(lens) != B:
+        raise ValueError(f"xlens has {len(lens)} entries for a batch of {B}")
+    for n in lens:
+        if n > T:
+            raise ValueError(f"xlens holds {n} frames, more than the {T} of the padded batch")
+        if n < 7:
+            raise ValueError(f"an utterance of {n} frames has no frame after sub-sampling (needs >= 7)")
+    tps = [int(model.get_pred_len(n)) for n in lens]
+    dev = xs.device
+    sub = torch.tensor(tps, dtype=torch.int64).to(dev)
+    st, eng, _ = F.bind(model, dev)
+    F.bind(model.encoder, dev)
+    F.bind(model.ctc, dev)
+    st.refresh_operands(force=True)
+    enc = eng.encoder_fwd(model.encoder, xs.contiguous().float(), None, False, sub_lens=sub)
+    head = eng.ctc_head_fwd(model.ctc, enc.out)
+    k = min(beam, model.vocab_size)
+    tv, ti, _, _ = ops.logsoftmax_topk(head.out, k, vocab=model.vocab_size)
+    return enc.out, tv, ti, tps, sub, enc.Tp
+
+
+@torch.no_grad()
+def _rescore_padded(model, nbest, h: Tensor, tps: Sequence[int]):
+    """``_rescore`` with the padded encoder output as memory: hypothesis i of utterance u reads h[u], keys j < T'_u."""
+    dev = h.device
+    utt = [u for u, hyps in enumerate(nbest) for _ in hyps]
+    idx = torch.tensor(utt, dtype=torch.int64).to(dev)
+    return _rescore(model, nbest, h.index_select(0, idx), torch.tensor([tps[u] for u in utt], dtype=torch.int64).to(dev))
+
+
+def decode_batch(model, xs: Tensor, xlens, beam: int = BEAM):
+    """Decode a padded batch xs (B,T,F) fp32 with lengths xlens (B,): the batch-1 inference of every utterance (models/u2.py:
+    221-317 on xs[b, :xlens[b]]) in one encoder pass, one top-K, one device prefix search and one decoder pass.
+    -> one dict per utterance: ``best`` (token list), ``hyps`` [(prefix tuple, CTC score)], ``scores`` (rescoring scores) and
+    ``greedy`` (greedy CTC tokens of the same rows, = ``greedy_ctc(x_b, None)``).  CTC scores are float64 with CUDA's exp / log:
+    they may differ from the host search's in the last bits (see ``lasr_ctc_prefix_beam_search_batch``).
+    Raises RuntimeError in training mode, ValueError for an utterance shorter than 7 frames or longer than T."""
+    h, tv, ti, tps, sub, Tp = _ragged_topk(model, xs, xlens, beam)
+    toks, lens, scores, count = ops.ctc_prefix_beam_search_batch(tv, ti, sub, Tp, beam=beam, blank=model.blank)
+    toks, lens, scores, count, top1 = (t.cpu().numpy() for t in (toks, lens, scores, count, ti[:, 0].view(-1, Tp)))
+    nbest = [[(tuple(int(x) for x in toks[b, i, : lens[b, i]]), float(scores[b, i])) for i in range(count[b])] for b in range(len(tps))]
+    res = _rescore_padded(model, nbest, h, tps)
+    return [dict(best=list(hy[bi][0]), hyps=hy, scores=sc, greedy=_greedy_rows(top1[b], tps[b], model.blank))
+            for b, (hy, (bi, sc)) in enumerate(zip(nbest, res))]
+
+
 def inference_batch(model, xs_list: Sequence[Tensor], beam: int = BEAM, return_details: bool = False):
-    """Decode a list of utterances (each (T_u,F) or (1,T_u,F)); token-identical to calling ``attention_rescore`` one by one."""
-    nbest, mems = [], []
-    for x in xs_list:
-        x = x if x.dim() == 3 else x.unsqueeze(0)
-        hyps, h = _prefix_search(model, x, beam)
-        nbest.append(hyps)
-        mems.append(h)
-    res = _rescore(model, nbest, mems)
+    """Decode a list of utterances (each (T_u,F) or (1,T_u,F)); token-identical to calling ``attention_rescore`` one by one.
+    The utterances share one per-utterance encoder pass and one top-K; the prefix search runs on the host per utterance, so
+    that the CTC scores are bit-identical to the batch-1 path's (``decode_batch`` runs it on the device instead)."""
+    utts = [x[0] if x.dim() == 3 else x for x in xs_list]
+    lens = [u.shape[0] for u in utts]
+    xs = torch.zeros((len(utts), max(lens), utts[0].shape[1]), dtype=torch.float32, device=utts[0].device)
+    for i, u in enumerate(utts):
+        xs[i, : lens[i]] = u
+    h, tv, ti, tps, _, Tp = _ragged_topk(model, xs, torch.tensor(lens), beam)
+    tv, ti = tv.view(len(utts), Tp, -1).cpu().numpy(), ti.view(len(utts), Tp, -1).cpu().numpy()
+    nbest = [ops.ctc_prefix_beam_search_host(tv[b, : tps[b]], ti[b, : tps[b]], beam=beam, blank=model.blank) for b in range(len(utts))]
+    res = _rescore_padded(model, nbest, h, tps)
     if return_details:
         return [dict(best=list(h[b][0]), hyps=h, scores=s) for h, (b, s) in zip(nbest, res)]
     return [list(h[b][0]) for h, (b, _) in zip(nbest, res)]

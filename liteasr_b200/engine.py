@@ -321,7 +321,8 @@ class Engine:
     # ------------------------------------------------------------------------------------------
     # relative-position self-attention block (nets/conformer_layer.py:107-128, nets/attention.py:120-154)
     # ------------------------------------------------------------------------------------------
-    def rel_mha_fwd(self, x, pfx_norm, pfx, pos, B, T, H, xlens, d_att=None, d_out=None) -> NS:
+    def rel_mha_fwd(self, x, pfx_norm, pfx, pos, B, T, H, xlens, d_att=None, d_out=None, sub_lens=None) -> NS:
+        """sub_lens: sub-sampled lengths -> mask mode 4 (per-utterance shift, inference only) instead of xlens' mode 3."""
         d = x.shape[1]
         dk = d // H
         ln = self.layernorm(x, pfx_norm, self.adt)
@@ -333,7 +334,10 @@ class Engine:
         qv = _empty((B * T, d), self.adt, self.dev)
         ops.pos_bias_fwd(q, self.st.p(pfx + ".pos_bias_u").view(-1), self.st.p(pfx + ".pos_bias_v").view(-1), qu, qv)
         p = self.linear(pos, pfx + ".linear_pos", self.adt, bias=False)
-        core = self.attn_core_fwd(qu, k, v, B, H, T, T, dk, xlens, 3 if xlens is not None else 0, 0, qv=qv, p=p, drop=d_att)
+        if sub_lens is not None:
+            core = self.attn_core_fwd(qu, k, v, B, H, T, T, dk, sub_lens, 4, 0, qv=qv, p=p, drop=d_att)
+        else:
+            core = self.attn_core_fwd(qu, k, v, B, H, T, T, dk, xlens, 3 if xlens is not None else 0, 0, qv=qv, p=p, drop=d_att)
         out = self.linear(core.o, pfx + ".linear_o", torch.float32, res=x, drop=d_out)
         return NS(out=out, ln=ln, qkv=qkv, core=core, pos=pos, pfx=pfx, d=d, d_out=d_out)
 
@@ -410,14 +414,19 @@ class Engine:
     # ------------------------------------------------------------------------------------------
     # convolution block (nets/conformer_layer.py:49-56, nets/conformer_convolution.py:44-57)
     # ------------------------------------------------------------------------------------------
-    def conv_fwd(self, x, pfx_norm, pfx, B, T, bn_mod, training, d_out=None) -> NS:
+    def conv_fwd(self, x, pfx_norm, pfx, B, T, bn_mod, training, d_out=None, sub_lens=None) -> NS:
+        """sub_lens: sub-sampled lengths -> rows t >= sub_lens[b] enter the depthwise conv as zeros (inference only)."""
         st, d = self.st, x.shape[1]
         ln = self.layernorm(x, pfx_norm, self.adt)
         y2 = self.linear(ln.y, None, self.adt, w=st.w(pfx + ".pointwise_conv1.weight"), bias_t=st.p(pfx + ".pointwise_conv1.bias"))
         z = _empty((B * T, d), torch.float32, self.dev)
         nblk = B * ((T + 31) // 32)
         partial = _empty((nblk, 2, d), torch.float32, self.dev)
-        ops.glu_dwconv_fwd(y2, st.p(pfx + ".depthwise_conv.weight").view(d, KW), st.p(pfx + ".depthwise_conv.bias"), z, partial, B, T, d)
+        if sub_lens is not None:
+            ops.glu_dwconv_fwd_lens(y2, st.p(pfx + ".depthwise_conv.weight").view(d, KW), st.p(pfx + ".depthwise_conv.bias"), z, partial, B,
+                                    T, d, sub_lens)
+        else:
+            ops.glu_dwconv_fwd(y2, st.p(pfx + ".depthwise_conv.weight").view(d, KW), st.p(pfx + ".depthwise_conv.bias"), z, partial, B, T, d)
         mean = _empty((d,), torch.float32, self.dev)
         rstd = _empty((d,), torch.float32, self.dev)
         if bn_mod.momentum is None:  # cumulative moving average: never configured by the reference (conformer_convolution.py:41)
@@ -556,9 +565,14 @@ class Engine:
     # ------------------------------------------------------------------------------------------
     # encoder (nets/transformer_encoder.py:107-127; use_rel=True, arch=conformer, activation=swish)
     # ------------------------------------------------------------------------------------------
-    def encoder_fwd(self, enc, xs, xlens, training: bool, rng=None) -> NS:
+    def encoder_fwd(self, enc, xs, xlens, training: bool, rng=None, sub_lens=None) -> NS:
         """xs (B,T,F) fp32, xlens (B,) int64 or None (maskless inference call).  Returns ctx with ctx.out (B,T',d) fp32.
-        rng: RNG snapshot of this pass (dropout.RngState.begin_pass) -- dropout is applied iff training and rng is given."""
+        rng: RNG snapshot of this pass (dropout.RngState.begin_pass) -- dropout is applied iff training and rng is given.
+        sub_lens (B,) int64 device tensor of sub-sampled lengths T'_b (xlens must be None): per-utterance inference on a padded
+        batch -- rows t < T'_b of utterance b equal the maskless batch-1 call on xs[b, :T_b] (attention mask mode 4, the
+        length-aware depthwise conv), rows t >= T'_b hold finite values.  Eval only: training keeps the padded-batch semantics."""
+        if sub_lens is not None and (training or xlens is not None):
+            raise RuntimeError("encoder_fwd: per-utterance lengths are an inference-only, maskless mode (training=False, xlens=None)")
         d, H = enc.h_dim, enc.n_head
         B = xs.shape[0]
         pfx = enc._lasr_prefix
@@ -581,9 +595,10 @@ class Engine:
             c1 = self.ffn_fwd(x, lp + ".feed_forward_macaron_norm", lp + ".feed_forward_macaron", ACT_SWISH, 0.5,
                               DR.drop(rng, E, i, DR.ENC_FFM_INNER, p_ffm), DR.drop(rng, E, i, DR.ENC_FFM_OUT, p_out))
             c2 = self.rel_mha_fwd(c1.out, lp + ".self_attn_norm", lp + ".self_attn", pos, B, Tp, H, xlens,
-                                  DR.drop(rng, E, i, DR.ENC_ATT_PROB, layer.self_attn.dropout_rate), DR.drop(rng, E, i, DR.ENC_ATT_OUT, p_out))
+                                  DR.drop(rng, E, i, DR.ENC_ATT_PROB, layer.self_attn.dropout_rate), DR.drop(rng, E, i, DR.ENC_ATT_OUT, p_out),
+                                  sub_lens=sub_lens)
             c3 = self.conv_fwd(c2.out, lp + ".conv_norm", lp + ".conv", B, Tp, layer.conv.norm, training,
-                               DR.drop(rng, E, i, DR.ENC_CONV_OUT, p_out))
+                               DR.drop(rng, E, i, DR.ENC_CONV_OUT, p_out), sub_lens=sub_lens)
             c4 = self.ffn_fwd(c3.out, lp + ".feed_forward_norm", lp + ".feed_forward", ACT_SWISH, 0.5,
                               DR.drop(rng, E, i, DR.ENC_FF_INNER, p_ff), DR.drop(rng, E, i, DR.ENC_FF_OUT, p_out))
             c5 = self.layernorm(c4.out, lp + ".final_norm", torch.float32)

@@ -366,6 +366,14 @@ def glu_dwconv_fwd(y2, w, bias, z, partial, B, T, d):
                                               _ptr(partial), _i(B), _i(T), _i(d), _stream()), "glu_dwconv_fwd")
 
 
+def glu_dwconv_fwd_lens(y2, w, bias, z, partial, B, T, d, lens):
+    """glu_dwconv_fwd with GLU rows t >= lens[b] (int64 (B,), sub-sampled frames) read as zero: per-utterance inference."""
+    _require_cuda(y2, lens)
+    assert lens.dtype == torch.int64 and lens.numel() == B and lens.is_contiguous()
+    _lib.check(_lib.lib().lasr_glu_dwconv_fwd_lens(_ptr(y2), _i(dtype_code(y2)), _l(y2.stride(0)), _ptr(w), _ptr(bias), _ptr(z),
+                                                   _ptr(partial), _i(B), _i(T), _i(d), _ptr(lens), _stream()), "glu_dwconv_fwd_lens")
+
+
 def bn_finalize(partial, nblk, d, count, mean, rstd, running_mean, running_var, nbt, training, eps=1e-5, momentum=0.1):
     _lib.check(_lib.lib().lasr_bn_finalize(_ptr(partial), _i(nblk), _i(d), _l(count), _f(eps), _f(momentum), _ptr(mean), _ptr(rstd),
                                            _ptr(running_mean), _ptr(running_var), _ptr(nbt), _i(training), _stream()), "bn_finalize")
@@ -573,3 +581,28 @@ def ctc_prefix_beam_search_host(top_val, top_idx, beam: int = 10, blank: int = 0
                                                       toks.ctypes.data_as(_P), lens.ctypes.data_as(_P), scores.ctypes.data_as(_P),
                                                       _i(max_len), C.byref(n)), "ctc_prefix_beam_search")
     return [(tuple(int(x) for x in toks[i, : lens[i]]), float(scores[i])) for i in range(n.value)]
+
+
+def ctc_prefix_beam_search_batch(top_val: torch.Tensor, top_idx: torch.Tensor, frames: torch.Tensor, Tmax: int, beam: int = 10,
+                                 blank: int = 0):
+    """DEVICE prefix search over a ragged batch (one launch, no host synchronisation).  top_val / top_idx (B*Tmax, K) as
+    ``logsoftmax_topk`` returns them, frames (B,) int64 on the device.  -> (tokens (B,beam,Tmax) int32 padded -1, lengths (B,beam)
+    int32, scores (B,beam) float64, counts (B,) int32), all on the device."""
+    _require_cuda(top_val, top_idx, frames)
+    assert top_val.dtype == torch.float32 and top_idx.dtype == torch.int32 and frames.dtype == torch.int64
+    assert top_val.is_contiguous() and top_idx.is_contiguous() and frames.is_contiguous() and top_val.shape == top_idx.shape
+    B = frames.numel()
+    K = top_val.shape[1]
+    assert top_val.shape[0] == B * Tmax
+    dev = top_val.device
+    toks = torch.empty((B, beam, Tmax), dtype=torch.int32, device=dev)
+    lens = torch.empty((B, beam), dtype=torch.int32, device=dev)
+    scores = torch.empty((B, beam), dtype=torch.float64, device=dev)
+    count = torch.empty(B, dtype=torch.int32, device=dev)
+    L = _lib.lib()
+    ws_bytes = int(L.lasr_ctc_prefix_beam_search_batch_workspace(_i(B), _i(Tmax), _i(beam)))
+    ws = torch.empty(max(ws_bytes, 8), dtype=torch.uint8, device=dev)
+    _lib.check(L.lasr_ctc_prefix_beam_search_batch(_ptr(top_val), _ptr(top_idx), _ptr(frames), _i(B), _i(Tmax), _i(K), _i(beam), _i(blank),
+                                                   _ptr(toks), _ptr(lens), _ptr(scores), _ptr(count), _i(Tmax), _ptr(ws),
+                                                   C.c_size_t(ws.numel()), _stream()), "ctc_prefix_beam_search_batch")
+    return toks, lens, scores, count
