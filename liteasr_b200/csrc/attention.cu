@@ -39,7 +39,7 @@ template <> __device__ __forceinline__ float2 load_pair<bf16>(const bf16* p) {
     return make_float2(__low2float(h), __high2float(h));
 }
 
-// One warp per score row; lane l owns the column pairs (2l + 64e, 2l + 64e + 1), e < NP (Tk <= 64 NP): 64-bit loads of ac,
+// One warp per score row; lane l owns the column pairs (2l + 64e, 2l + 64e + 1), e < NP (ld <= 64 NP): 64-bit loads of ac,
 // 32/64-bit stores of the probabilities, NP sized to the problem so the kernel runs at full occupancy.  ld must be even.
 template <typename TP, typename TS, int NP, bool RAGGED = false>
 __global__ void __launch_bounds__(256) attn_softmax_fwd_kernel(const TS* __restrict__ ac, const TS* __restrict__ bd,
@@ -164,22 +164,24 @@ __global__ void __launch_bounds__(256) attn_softmax_bwd_kernel(const TP* __restr
 extern "C" {
 using namespace lasr;
 
+// NP is chosen from the row width ld, not from Tk: a lane writes only columns j < 64 NP, and every column of [Tk, ld) must be
+// zeroed.  The bucket edges are multiples of 64, so ld = ceil(Tk, 8) or ceil(Tk, 64) selects the same NP as Tk would.
 #define LASR_SM_DISPATCH(KERNEL, TP, TS, ...)                                        \
     do {                                                                             \
-        if (Tk <= 64) launch_pdl(KERNEL<TP, TS, 1>, grid, 256, 0, st, __VA_ARGS__);          \
-        else if (Tk <= 128) launch_pdl(KERNEL<TP, TS, 2>, grid, 256, 0, st, __VA_ARGS__);    \
-        else if (Tk <= 320) launch_pdl(KERNEL<TP, TS, 5>, grid, 256, 0, st, __VA_ARGS__);    \
-        else if (Tk <= 448) launch_pdl(KERNEL<TP, TS, 7>, grid, 256, 0, st, __VA_ARGS__);    \
+        if (ld <= 64) launch_pdl(KERNEL<TP, TS, 1>, grid, 256, 0, st, __VA_ARGS__);          \
+        else if (ld <= 128) launch_pdl(KERNEL<TP, TS, 2>, grid, 256, 0, st, __VA_ARGS__);    \
+        else if (ld <= 320) launch_pdl(KERNEL<TP, TS, 5>, grid, 256, 0, st, __VA_ARGS__);    \
+        else if (ld <= 448) launch_pdl(KERNEL<TP, TS, 7>, grid, 256, 0, st, __VA_ARGS__);    \
         else launch_pdl(KERNEL<TP, TS, SM_MAXP>, grid, 256, 0, st, __VA_ARGS__);             \
     } while (0)
 
 // mask mode 4: the RAGGED instantiations of the forward kernel
 #define LASR_SM_DISPATCH_RAGGED(TP, TS, ...)                                                               \
     do {                                                                                                    \
-        if (Tk <= 64) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 1, true>, grid, 256, 0, st, __VA_ARGS__);          \
-        else if (Tk <= 128) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 2, true>, grid, 256, 0, st, __VA_ARGS__);    \
-        else if (Tk <= 320) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 5, true>, grid, 256, 0, st, __VA_ARGS__);    \
-        else if (Tk <= 448) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 7, true>, grid, 256, 0, st, __VA_ARGS__);    \
+        if (ld <= 64) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 1, true>, grid, 256, 0, st, __VA_ARGS__);          \
+        else if (ld <= 128) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 2, true>, grid, 256, 0, st, __VA_ARGS__);    \
+        else if (ld <= 320) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 5, true>, grid, 256, 0, st, __VA_ARGS__);    \
+        else if (ld <= 448) launch_pdl(attn_softmax_fwd_kernel<TP, TS, 7, true>, grid, 256, 0, st, __VA_ARGS__);    \
         else launch_pdl(attn_softmax_fwd_kernel<TP, TS, SM_MAXP, true>, grid, 256, 0, st, __VA_ARGS__);             \
     } while (0)
 

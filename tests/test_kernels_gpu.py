@@ -122,49 +122,95 @@ def test_conv_module_middle_fwd_bwd(B, T, d, dtype):
     assert _close(cs, dy2.float().sum(0), 1e-3 if dtype == torch.float32 else 3e-2)
 
 
-def _rel_shift(x):
-    """nets/attention.py:99-118 (legacy, no zero_triu)."""
-    b, h, t1, t2 = x.shape
-    zp = torch.zeros(b, h, t1, 1, device=x.device, dtype=x.dtype)
-    xp = torch.cat([zp, x], dim=-1).view(b, h, t2 + 1, t1)
-    return xp[:, :, 1:].view_as(x)
+# ---------------------------------------------------------------------------------------------------------------------------------
+# attention softmax (csrc/attention.cu) against a float64 reference evaluated from the same rounded inputs the kernel reads
+#
+# Element-wise bounds (u = 2^-24, S = the largest |scaled logit| of the call):
+#   forward, fp32 probs : |p - ref| <= ref * u * (6 S + 60)   (logit add / subtract, two expf at <= 2 ulp, 1/sum, the row sum over
+#                                                             at most 2 NP + 5 sequential adds with NP <= 16)
+#   forward, bf16 probs : one more rounding, + 2^-8 * ref
+#   backward            : ds = p (dp - D) scale with D = sum_j p_j dp_j; the fp32 row dot product is off by at most
+#                         (2 NP + 8) u sum_j |p_j dp_j|, the three roundings of the element by 2^-22 |p scale| (|dp| + |D|);
+#                         bf16 outputs add 2^-8 |ref|.  dbd holds the same values moved through the inverse shift.
+# Columns [Tk, ld) of probs / dscores / dbd must be exactly 0 (the buffers start as NaN).
+# ---------------------------------------------------------------------------------------------------------------------------------
+U32 = 2.0 ** -24
+DTYPES = [(torch.float32, torch.float32), (torch.float32, torch.bfloat16), (torch.bfloat16, torch.bfloat16)]  # (scores, probs)
 
 
-@pytest.mark.parametrize("B,H,T", [(2, 2, 7), (3, 4, 124), (2, 4, 299), (1, 8, 399)])
-@pytest.mark.parametrize("pdt", [torch.float32, torch.bfloat16])
-def test_attn_softmax_relshift_fwd_bwd(B, H, T, pdt):
+def _np_bucket(ld):
+    return 1 if ld <= 64 else 2 if ld <= 128 else 5 if ld <= 320 else 7 if ld <= 448 else 16
+
+
+def _key_len(lens, mode, B, Tk):
+    if mode == 0:
+        return torch.full((B,), Tk, dtype=torch.int64)
+    k = lens.cpu() + (1 if mode == 2 else 0)
+    if mode == 3:
+        k = (lens.cpu() + 3) // 4
+    return k.clamp(0, Tk)
+
+
+def _softmax_case(B, H, Tq, Tk, ld, sdt, pdt, mode, causal, rel, lens, seed, scale=0.125):
+    """Run lasr_attn_softmax_fwd and _bwd once (rel: with the legacy rel_shift of bd) and check every output element."""
     from liteasr_b200 import ops
-    g = torch.Generator(device="cuda").manual_seed(B * H * T)
-    ld = (T + 7) // 8 * 8
-    ac = torch.zeros(B, H, T, ld, device="cuda")
-    bd = torch.zeros(B, H, T, ld, device="cuda")
-    ac[..., :T] = torch.randn(B, H, T, T, generator=g, device="cuda") * 3
-    bd[..., :T] = torch.randn(B, H, T, T, generator=g, device="cuda") * 3
-    lens = torch.randint(max(1, 4 * T - 11), 4 * T + 1, (B,), generator=g, device="cuda")   # raw frame counts: klen = ceil(l/4)
-    lens[0] = 4 * T
-    scale = 0.125
-    acr = ac[..., :T].clone().requires_grad_(True)
-    bdr = bd[..., :T].clone().requires_grad_(True)
-    klen = (lens + 3) // 4
-    mask = torch.arange(T, device="cuda")[None, :] >= klen[:, None]
-    sc = ((acr + _rel_shift(bdr)) * scale).masked_fill(mask[:, None, None, :], -1e38)
-    pr = torch.softmax(sc, -1)
-    probs = torch.full((B, H, T, ld), 9.0, device="cuda", dtype=pdt)
-    ops.attn_softmax_fwd(ac, bd, probs, lens, 3, 0, scale, T)
-    tol = 1e-5 if pdt == torch.float32 else 1e-2
-    assert _close(probs[..., :T], pr, tol)
-    assert (probs[..., T:] == 0).all()
-    dp = torch.zeros(B, H, T, ld, device="cuda")
-    dp[..., :T] = torch.randn(B, H, T, T, generator=g, device="cuda")
-    pr.backward(dp[..., :T])
-    # feed the kernel the exact probabilities it would have saved
-    dsc = torch.empty(B, H, T, ld, device="cuda", dtype=pdt)
-    dbd = torch.empty(B, H, T, ld, device="cuda", dtype=pdt)
-    ops.attn_softmax_bwd(probs, dp, dsc, dbd, scale, T)
-    tolb = 1e-4 if pdt == torch.float32 else 3e-2
-    assert _close(dsc[..., :T], acr.grad, tolb)
-    assert _close(dbd[..., :T], bdr.grad, tolb)
-    assert (dsc[..., T:] == 0).all()
+    from oracle.u2_oracle import rel_shift
+    g = torch.Generator(device="cuda").manual_seed(seed)
+    nan = float("nan")
+    ac = torch.full((B, H, Tq, ld), nan, device="cuda", dtype=sdt)   # padding columns are never read as scores
+    ac[..., :Tk] = (torch.randn(B, H, Tq, Tk, generator=g, device="cuda") * 3).to(sdt)
+    bd = None
+    if rel:
+        bd = torch.full((B, H, Tq, ld), nan, device="cuda", dtype=sdt)
+        bd[..., :Tk] = (torch.randn(B, H, Tq, Tk, generator=g, device="cuda") * 3).to(sdt)
+    probs = torch.full((B, H, Tq, ld), nan, device="cuda", dtype=pdt)
+    ops.attn_softmax_fwd(ac, bd, probs, lens, mode, causal, scale, Tk)
+
+    # float64 reference (masked_fill(-1e38) + softmax: a row without keys is uniform 1/Tk, quirk Q4)
+    s = ac[..., :Tk].double().cpu()
+    if rel:
+        s = s + rel_shift(bd[..., :Tk].double().cpu())
+    s = s * scale
+    S = float(s.abs().max())
+    j = torch.arange(Tk)
+    mask = (j[None, :] >= _key_len(lens, mode, B, Tk)[:, None])[:, None, None, :]
+    if causal:
+        mask = mask | (j[None, :] > torch.arange(Tq)[:, None])[None, None]
+    ref = torch.softmax(s.masked_fill(mask, -1e38), -1)
+    got = probs.double().cpu()
+    bound = ref * U32 * (6 * S + 60)
+    if pdt == torch.bfloat16:
+        bound = bound + 2.0 ** -8 * ref
+    assert not torch.isnan(got).any(), "probs: element left unwritten or NaN"
+    err = (got[..., :Tk] - ref).abs()
+    assert (err <= bound).all(), f"probs: worst excess {float((err - bound).max()):.3g}"
+    assert (got[..., Tk:] == 0).all(), "probs: padding columns not zeroed"
+
+    # backward from the probabilities the kernel saved and dprobs of the score dtype
+    dp = torch.full((B, H, Tq, ld), nan, device="cuda", dtype=sdt)
+    dp[..., :Tk] = torch.randn(B, H, Tq, Tk, generator=g, device="cuda").to(sdt)
+    dsc = torch.full((B, H, Tq, ld), nan, device="cuda", dtype=pdt)
+    dbd = torch.full((B, H, Tq, ld), nan, device="cuda", dtype=pdt) if rel else None
+    ops.attn_softmax_bwd(probs, dp, dsc, dbd, scale, Tk)
+    p64, g64 = got[..., :Tk], dp[..., :Tk].double().cpu()
+    D = (p64 * g64).sum(-1, keepdim=True)
+    ds_ref = p64 * (g64 - D) * scale
+    a = p64.abs() * abs(scale)
+    ds_bound = a * ((2 * _np_bucket(ld) + 8) * U32 * (p64 * g64).abs().sum(-1, keepdim=True) + 2.0 ** -22 * (g64.abs() + D.abs()))
+    if pdt == torch.bfloat16:
+        ds_bound = ds_bound + 2.0 ** -8 * (ds_ref.abs() + ds_bound)
+    outs = [("dscores", dsc, ds_ref, ds_bound)]
+    if rel:
+        x = torch.zeros(B, H, Tq, Tk, dtype=torch.float64, requires_grad=True)
+        dbd_ref, dbd_bound = (torch.autograd.grad(rel_shift(x), x, t)[0] for t in (ds_ref, ds_bound))
+        outs.append(("dbd", dbd, dbd_ref, dbd_bound))
+    for name, out, r, bnd in outs:
+        o = out.double().cpu()
+        assert not torch.isnan(o).any(), f"{name}: element left unwritten or NaN"
+        e = (o[..., :Tk] - r).abs()
+        assert (e <= bnd).all(), f"{name}: worst excess {float((e - bnd).max()):.3g}"
+        assert (o[..., Tk:] == 0).all(), f"{name}: padding columns not zeroed"
+    return got
 
 
 def test_attn_softmax_plain_causal_and_cross():
@@ -181,6 +227,52 @@ def test_attn_softmax_plain_causal_and_cross():
     mask = (j[None, None, :] > j[None, :, None]) | (j[None, None, :] >= (ylens + 1)[:, None, None])
     ref = torch.softmax((ac[..., :Tk] * 0.5).masked_fill(mask[:, None], -1e38), -1)
     assert _close(probs[..., :Tk], ref, 1e-5)
+
+
+# T covers both sides of every NP bucket edge (64, 128, 320, 448) and the largest bucket (T' up to 1024)
+@pytest.mark.parametrize("T", [7, 64, 65, 128, 129, 320, 321, 448, 449, 700, 1000])
+@pytest.mark.parametrize("sdt,pdt", DTYPES)
+@pytest.mark.parametrize("mode", [0, 1, 3])
+def test_attn_softmax_relshift_fwd_bwd(T, sdt, pdt, mode):
+    """Encoder self-attention (rel_shift of bd, Tq = Tk) at ld = ceil(T, 8) as the engine allocates it.  With a key mask the
+    second utterance has no keys at all: every score of its rows is -1e38 and the softmax is uniform 1/Tk, like the reference."""
+    B, H = 3, (2 if T <= 448 else 1)
+    ld = (T + 7) // 8 * 8
+    g = torch.Generator().manual_seed(T * 7 + mode)
+    lens = None
+    if mode == 1:
+        lens = torch.tensor([T + 5, 0, int(torch.randint(1, T, (1,), generator=g)) if T > 1 else 1])
+    elif mode == 3:                                           # raw frame counts: klen = ceil(l / 4)
+        lens = torch.tensor([4 * T, 0, int(torch.randint(1, 4 * T - 3, (1,), generator=g))])
+    lens = lens.cuda() if lens is not None else None
+    probs = _softmax_case(B, H, T, T, ld, sdt, pdt, mode, 0, True, lens, seed=T + 100 * mode)
+    if mode:
+        assert torch.allclose(probs[1, ..., :T].double().cpu(), torch.full((H, T, T), 1.0 / T, dtype=torch.float64), rtol=2.0 ** -8, atol=0)
+
+
+@pytest.mark.parametrize("sdt,pdt", DTYPES)
+@pytest.mark.parametrize("Tq,Tk", [(1, 299), (41, 299), (1, 449), (41, 449)])
+def test_attn_softmax_cross_attention(Tq, Tk, sdt, pdt):
+    """Decoder source attention: Tq = L + 1 queries against T' encoder frames, encoder key mask (mode 3), no rel-pos term."""
+    ld = (Tk + 7) // 8 * 8
+    lens = torch.tensor([4 * Tk, 0, 4 * Tk - 13, 5], device="cuda")
+    _softmax_case(4, 2, Tq, Tk, ld, sdt, pdt, 3, 0, False, lens, seed=Tq * Tk)
+
+
+@pytest.mark.parametrize("sdt,pdt", DTYPES)
+def test_attn_softmax_decoder_self_attention(sdt, pdt):
+    """Decoder self-attention: causal and keys j < ylen + 1 (mode 2), Tq = Tk = 41, no rel-pos term."""
+    lens = torch.tensor([40, 0, 17, 3], device="cuda")
+    _softmax_case(4, 2, 41, 41, 48, sdt, pdt, 2, 1, False, lens, seed=41)
+
+
+@pytest.mark.parametrize("sdt,pdt", DTYPES)
+@pytest.mark.parametrize("Tk,ld", [(99, 100), (449, 450), (100, 128), (321, 384), (100, 200), (300, 512)])
+def test_attn_softmax_padding_columns(Tk, ld, sdt, pdt):
+    """include/lasr.h: columns [Tk, ld) of probs, dscores and dbd are zeroed for any even ld <= 1024, including a row buffer
+    wider than the bucket that Tk alone would pick ((100, 200), (300, 512))."""
+    lens = torch.tensor([4 * Tk, 4 * Tk - 9], device="cuda")
+    _softmax_case(2, 2, Tk, Tk, ld, sdt, pdt, 3, 0, True, lens, seed=Tk + ld)
 
 
 @pytest.mark.parametrize("rows,d", [(37674, 256), (1000, 512), (77, 64), (5166, 144)])
