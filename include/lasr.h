@@ -336,6 +336,10 @@ int lasr_conv2_wgrad(const void* dy2p, const void* h1p, float* dw2k, int B, int 
  *              bdshift[i,j] = bd[i, klen-1-(i-j)] (j <= i) | 0 (j == i+1) | bd[i+1, j-i-2] (i+1 < j < klen), keys j >= klen -1e38;
  *              rows i < klen then equal the maskless batch-1 call on the utterance cut to klen frames (per-utterance inference
  *              on a padded batch), rows i >= klen get finite values without the rel-pos term.
+ * Row width: ld even, Tk <= ld <= 16384 (T' = 16384 sub-sampled frames, about 10.9 minutes of audio at a 10 ms frame shift);
+ * a larger ld returns LASR_ERR_BAD_ARG with a message naming the bound.  ld <= 1024 runs one warp per row, wider rows one
+ * 512-thread CTA per row (B*H*Tq <= 2^31 - 1 rows); element offsets are 64-bit, so a tensor may exceed 2^31 elements.
+ * A row's results do not depend on ld within either range.
  * ------------------------------------------------------------------------------------------------ */
 int lasr_attn_softmax_fwd(const void* ac, const void* bd, int s_dtype, void* probs, int p_dtype, const int64_t* lens, int mask_mode,
                           int causal, float scale, int B, int H, int Tq, int Tk, int ld, void* stream);
