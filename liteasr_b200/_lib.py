@@ -9,6 +9,7 @@ import re
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("LASR_LIB_PATH") or os.path.join(_HERE, "liblasr.so")  # LASR_LIB_PATH: developer A/B builds
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "lasr.h")
+ALIGN_HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "lasr_align.h")
 
 F32, BF16 = 0, 1
 ACT_NONE, ACT_RELU, ACT_SWISH, ACT_MUL = 0, 1, 2, 3
@@ -37,9 +38,9 @@ class GemmArgs(C.Structure):
 _lib = None
 
 
-def declared_symbols() -> list:
-    """Every function name declared in include/lasr.h (used by the symbol-export test)."""
-    with open(HEADER_PATH) as f:
+def declared_symbols(header: str = HEADER_PATH) -> list:
+    """Every function name declared in include/lasr.h, or in ``header`` (used by the symbol-export tests)."""
+    with open(header) as f:
         src = f.read()
     src = re.sub(r"/\*.*?\*/", "", src, flags=re.S)
     return sorted(set(re.findall(r"\b(lasr_[a-z0-9_]+)\s*\(", src)))
@@ -56,6 +57,7 @@ def lib() -> C.CDLL:
         _lib.lasr_last_error.restype = C.c_char_p
         _lib.lasr_ctc_workspace_bytes.restype = C.c_size_t
         _lib.lasr_ctc_prefix_beam_search_batch_workspace.restype = C.c_size_t
+        _lib.lasr_ctc_forced_align_workspace.restype = C.c_size_t
         _lib.lasr_launch_count.restype = C.c_ulonglong
     return _lib
 

@@ -14,6 +14,9 @@
                               rescoring every n-best of every utterance (memory masked by its sub-sampled length).
 * ``inference_batch``         a list of utterances through the same encoder pass and top-K, with the host search per utterance:
                               token- and score-identical to calling ``attention_rescore`` one by one.
+* ``align``                   CTC Viterbi forced alignment of known transcripts on the same encoder pass: the most likely CTC
+                              path per utterance in one device launch (``lasr_ctc_forced_align``), token spans in frames and
+                              seconds (defined from nets/ctc.py:25-26; the reference ships no aligner).
 
 ``greedy_ctc(xs, xlens)`` keeps the reference's padded-batch semantics (mask mode 3, the padded rows inside the depthwise conv
 window), so its tokens can differ from those of a batch-1 call; ``decode_batch(...)["greedy"]`` has per-utterance semantics and
@@ -149,9 +152,9 @@ def attention_rescore(model, x: Tensor, beam: int = BEAM, return_details: bool =
 
 
 @torch.no_grad()
-def _ragged_topk(model, xs: Tensor, xlens, beam: int):
-    """Per-utterance encoder pass over a padded batch + one top-K over every row.
-    -> (h (B,T'max,d) fp32, top_val / top_idx (B*T'max, K), T'_b list, T'_b device tensor, T'max)."""
+def _ragged_encode(model, xs: Tensor, xlens):
+    """Per-utterance encoder pass over a padded batch + the CTC head.
+    -> (h (B,T'max,d) fp32, CTC logits (B*T'max, >=V) 2-D view, T'_b list, T'_b device tensor, T'max)."""
     if model.training:
         raise RuntimeError("inference runs on the BatchNorm running statistics: call model.eval() first")
     if xs.dim() != 3:
@@ -174,9 +177,17 @@ def _ragged_topk(model, xs: Tensor, xlens, beam: int):
     st.refresh_operands(force=True)
     enc = eng.encoder_fwd(model.encoder, xs.contiguous().float(), None, False, sub_lens=sub)
     head = eng.ctc_head_fwd(model.ctc, enc.out)
+    return enc.out, head.out, tps, sub, enc.Tp
+
+
+@torch.no_grad()
+def _ragged_topk(model, xs: Tensor, xlens, beam: int, want_lse: bool = False):
+    """``_ragged_encode`` + one top-K over every row (and, with want_lse, the row log-sum-exp from the same launch).
+    -> (h (B,T'max,d) fp32, top_val / top_idx (B*T'max, K), T'_b list, T'_b device tensor, T'max, CTC logits, lse or None)."""
+    h, logits, tps, sub, Tp = _ragged_encode(model, xs, xlens)
     k = min(beam, model.vocab_size)
-    tv, ti, _, _ = ops.logsoftmax_topk(head.out, k, vocab=model.vocab_size)
-    return enc.out, tv, ti, tps, sub, enc.Tp
+    tv, ti, lse, _ = ops.logsoftmax_topk(logits, k, vocab=model.vocab_size, want_lse=want_lse)
+    return h, tv, ti, tps, sub, Tp, logits, lse
 
 
 @torch.no_grad()
@@ -188,20 +199,104 @@ def _rescore_padded(model, nbest, h: Tensor, tps: Sequence[int]):
     return _rescore(model, nbest, h.index_select(0, idx), torch.tensor([tps[u] for u in utt], dtype=torch.int64).to(dev))
 
 
-def decode_batch(model, xs: Tensor, xlens, beam: int = BEAM):
+def decode_batch(model, xs: Tensor, xlens, beam: int = BEAM, timestamps: bool = False):
     """Decode a padded batch xs (B,T,F) fp32 with lengths xlens (B,): the batch-1 inference of every utterance (models/u2.py:
     221-317 on xs[b, :xlens[b]]) in one encoder pass, one top-K, one device prefix search and one decoder pass.
     -> one dict per utterance: ``best`` (token list), ``hyps`` [(prefix tuple, CTC score)], ``scores`` (rescoring scores) and
     ``greedy`` (greedy CTC tokens of the same rows, = ``greedy_ctc(x_b, None)``).  CTC scores are float64 with CUDA's exp / log:
     they may differ from the host search's in the last bits (see ``lasr_ctc_prefix_beam_search_batch``).
+    ``timestamps=True`` adds ``timestamps``: ``align``'s ``tokens`` for ``best`` (token, first frame, last frame, start s, end s
+    at a 10 ms frame shift), from the same encoder pass and CTC logits (one more device launch); the other keys do not change.
     Raises RuntimeError in training mode, ValueError for an utterance shorter than 7 frames or longer than T."""
-    h, tv, ti, tps, sub, Tp = _ragged_topk(model, xs, xlens, beam)
+    h, tv, ti, tps, sub, Tp, logits, lse = _ragged_topk(model, xs, xlens, beam, want_lse=timestamps)
     toks, lens, scores, count = ops.ctc_prefix_beam_search_batch(tv, ti, sub, Tp, beam=beam, blank=model.blank)
     toks, lens, scores, count, top1 = (t.cpu().numpy() for t in (toks, lens, scores, count, ti[:, 0].view(-1, Tp)))
     nbest = [[(tuple(int(x) for x in toks[b, i, : lens[b, i]]), float(scores[b, i])) for i in range(count[b])] for b in range(len(tps))]
     res = _rescore_padded(model, nbest, h, tps)
-    return [dict(best=list(hy[bi][0]), hyps=hy, scores=sc, greedy=_greedy_rows(top1[b], tps[b], model.blank))
-            for b, (hy, (bi, sc)) in enumerate(zip(nbest, res))]
+    out = [dict(best=list(hy[bi][0]), hyps=hy, scores=sc, greedy=_greedy_rows(top1[b], tps[b], model.blank))
+           for b, (hy, (bi, sc)) in enumerate(zip(nbest, res))]
+    if timestamps:
+        best = [o["best"] for o in out]
+        ys = np.full((len(best), max(len(b) for b in best)), -1, dtype=np.int64)
+        for b, hy in enumerate(best):
+            ys[b, : len(hy)] = hy
+        al = _align_rows(model, logits, lse, ys, [len(b) for b in best], sub, tps, Tp, 0.01)
+        for o, a in zip(out, al):
+            o["timestamps"] = a["tokens"]
+    return out
+
+
+# ----------------------------------------------------------------------------------------------
+# forced alignment
+# ----------------------------------------------------------------------------------------------
+SUBSAMPLE = 4          # input frames per encoder frame (nets/subsampling.py: two stride-2 convolutions)
+MAX_ALIGN_LABELS = 16383
+
+
+def span_seconds(first: int, last: int, frame_shift: float = 0.01) -> Tuple[float, float]:
+    """Encoder frames [first, last] -> (start, end) in seconds: encoder frame t stands for input frames [4t, 4t + 4), so
+    start = 4 * first * frame_shift and end = 4 * (last + 1) * frame_shift."""
+    return SUBSAMPLE * first * frame_shift, SUBSAMPLE * (last + 1) * frame_shift
+
+
+def _align_rows(model, logits: Tensor, lse: Tensor, ys: np.ndarray, ylens: Sequence[int], sub: Tensor, tps: Sequence[int], Tp: int,
+                frame_shift: float):
+    """Forced alignment of the ragged CTC logits against host targets ys (B, Lmax) int64 padded -1 -> one dict per utterance."""
+    dev = logits.device
+    state, _, score, spans = ops.ctc_forced_align(logits, lse, torch.from_numpy(ys).to(dev), torch.tensor(list(ylens), dtype=torch.int64).to(dev),
+                                                  sub, Tp, model.blank, vocab=model.vocab_size)
+    state, score, spans = state.cpu().numpy(), score.cpu().numpy(), spans.cpu().numpy()
+    out = []
+    for b, (L, T) in enumerate(zip(ylens, tps)):
+        sc = float(score[b])
+        if sc == -np.inf:
+            out.append(dict(score=sc, path=[], tokens=[]))
+            continue
+        st = state[b, :T].astype(np.int64)
+        y = ys[b, :L]
+        path = np.full(T, model.blank, dtype=np.int64)
+        odd = (st & 1) == 1
+        path[odd] = y[st[odd] >> 1]
+        toks = [(tok, f0, f1, *span_seconds(f0, f1, frame_shift)) for tok, (f0, f1) in zip(y.tolist(), spans[b, :L].tolist())]
+        out.append(dict(score=sc, path=path.tolist(), tokens=toks))
+    return out
+
+
+def align(model, xs: Tensor, xlens, ys, ylens, frame_shift: float = 0.01):
+    """CTC Viterbi forced alignment of known transcripts (include/lasr_align.h): the single most likely CTC path of each
+    transcript over log_softmax(ctc_lo(encoder(x))) (nets/ctc.py:25-26; the reference ships no aligner, this definition is
+    ours).  xs (B,T,F) fp32 padded with lengths xlens (B,); ys (B,Lmax) int64 padded -1 with lengths ylens (B,): the training
+    batch contract.  The encoder pass is ``decode_batch``'s (per-utterance semantics), so each result equals ``align`` on the
+    utterance alone.
+    -> one dict per utterance: ``score`` (float, the path's summed fp32 log-probability; -inf when the T'_b encoder frames
+    cannot hold the transcript: T'_b < L + the number of adjacent repeated tokens), ``path`` (T'_b token ids, the blank id on
+    blank frames; [] when infeasible) and ``tokens`` [(token, first frame, last frame, start s, end s)] ([] when infeasible).
+    Frames are encoder frames: frame t covers input frames [4t, 4t + 4) at ``frame_shift`` seconds each, so start_s =
+    4 * first * frame_shift and end_s = 4 * (last + 1) * frame_shift.
+    Raises RuntimeError in training mode; ValueError for an utterance shorter than 7 frames or longer than T, a token that is
+    blank, negative or >= V, a transcript longer than 16383 tokens, or ylens larger than Lmax."""
+    if model.training:
+        raise RuntimeError("inference runs on the BatchNorm running statistics: call model.eval() first")
+    y = torch.as_tensor(ys).cpu()
+    if y.dim() != 2 or y.dtype != torch.int64:
+        raise ValueError("ys must be a padded (B, Lmax) int64 batch")
+    y = y.numpy()
+    lens = [int(v) for v in torch.as_tensor(ylens).reshape(-1).cpu()]
+    if len(lens) != y.shape[0] or y.shape[0] != xs.shape[0]:
+        raise ValueError(f"ys / ylens hold {y.shape[0]} / {len(lens)} transcripts for a batch of {xs.shape[0]}")
+    V = model.vocab_size
+    for b, L in enumerate(lens):
+        if L < 0 or L > y.shape[1]:
+            raise ValueError(f"ylens[{b}] = {L} outside [0, Lmax = {y.shape[1]}]")
+        if L > MAX_ALIGN_LABELS:
+            raise ValueError(f"a transcript of {L} tokens exceeds the aligner's limit of {MAX_ALIGN_LABELS}")
+        row = y[b, :L]
+        bad = (row < 0) | (row >= V) | (row == model.blank)
+        if bad.any():
+            raise ValueError(f"ys[{b}] holds token {int(row[bad][0])}: tokens must lie in [0, {V}) and differ from blank {model.blank}")
+    _, logits, tps, sub, Tp = _ragged_encode(model, xs, xlens)
+    _, _, lse, _ = ops.logsoftmax_topk(logits, 0, vocab=V, want_lse=True)
+    return _align_rows(model, logits, lse, np.ascontiguousarray(y[:, : max(lens, default=0)]), lens, sub, tps, Tp, frame_shift)
 
 
 def inference_batch(model, xs_list: Sequence[Tensor], beam: int = BEAM, return_details: bool = False):
@@ -213,7 +308,7 @@ def inference_batch(model, xs_list: Sequence[Tensor], beam: int = BEAM, return_d
     xs = torch.zeros((len(utts), max(lens), utts[0].shape[1]), dtype=torch.float32, device=utts[0].device)
     for i, u in enumerate(utts):
         xs[i, : lens[i]] = u
-    h, tv, ti, tps, _, Tp = _ragged_topk(model, xs, torch.tensor(lens), beam)
+    h, tv, ti, tps, _, Tp, _, _ = _ragged_topk(model, xs, torch.tensor(lens), beam)
     tv, ti = tv.view(len(utts), Tp, -1).cpu().numpy(), ti.view(len(utts), Tp, -1).cpu().numpy()
     nbest = [ops.ctc_prefix_beam_search_host(tv[b, : tps[b]], ti[b, : tps[b]], beam=beam, blank=model.blank) for b in range(len(utts))]
     res = _rescore_padded(model, nbest, h, tps)

@@ -606,3 +606,30 @@ def ctc_prefix_beam_search_batch(top_val: torch.Tensor, top_idx: torch.Tensor, f
                                                    _ptr(toks), _ptr(lens), _ptr(scores), _ptr(count), _i(Tmax), _ptr(ws),
                                                    C.c_size_t(ws.numel()), _stream()), "ctc_prefix_beam_search_batch")
     return toks, lens, scores, count
+
+
+def ctc_forced_align(logits: torch.Tensor, lse: torch.Tensor, targets: torch.Tensor, tgt_len: torch.Tensor, frames: torch.Tensor, Tmax: int,
+                     blank: int = 0, *, vocab: Optional[int] = None):
+    """DEVICE CTC Viterbi forced alignment of a ragged batch (include/lasr_align.h, one launch, no host synchronisation).
+    logits (B*Tmax, >=V) fp32 | bf16 2-D view (utterance b at rows [b*Tmax, b*Tmax + frames[b])), lse (B*Tmax,) fp32 as
+    ``logsoftmax_topk(..., want_lse=True)`` returns it, targets (B, lmax) int64 padded -1, tgt_len / frames (B,) int64.
+    -> (state (B,Tmax) int32, frame_logp (B,Tmax) fp32, score (B,) fp32, spans (B,lmax,2) int32), all on the device."""
+    _require_cuda(logits, lse, targets, tgt_len, frames)
+    assert logits.dim() == 2 and logits.stride(1) == 1 and lse.dtype == torch.float32 and lse.is_contiguous()
+    assert targets.dtype == torch.int64 and tgt_len.dtype == torch.int64 and frames.dtype == torch.int64 and targets.dim() == 2
+    B, lmax = targets.shape
+    assert tgt_len.numel() == B and frames.numel() == B and logits.shape[0] == B * Tmax and lse.numel() == B * Tmax
+    V = logits.shape[1] if vocab is None else vocab
+    dev = logits.device
+    targets, tgt_len, frames = targets.contiguous(), tgt_len.contiguous(), frames.contiguous()
+    state = torch.empty((B, Tmax), dtype=torch.int32, device=dev)
+    logp = torch.empty((B, Tmax), dtype=torch.float32, device=dev)
+    score = torch.empty(B, dtype=torch.float32, device=dev)
+    spans = torch.empty((B, lmax, 2), dtype=torch.int32, device=dev)
+    L = _lib.lib()
+    ws_bytes = int(L.lasr_ctc_forced_align_workspace(_i(B), _i(Tmax), _i(lmax)))
+    ws = torch.empty(max(ws_bytes, 8), dtype=torch.uint8, device=dev)
+    _lib.check(L.lasr_ctc_forced_align(_ptr(logits), _i(dtype_code(logits)), _l(logits.stride(0)), _ptr(lse), _ptr(targets), _ptr(tgt_len),
+                                       _ptr(frames), _i(B), _i(Tmax), _i(lmax), _i(V), _i(blank), _ptr(state), _ptr(logp), _ptr(score),
+                                       _ptr(spans), _ptr(ws), C.c_size_t(ws.numel()), _stream()), "ctc_forced_align")
+    return state, logp, score, spans
