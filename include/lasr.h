@@ -91,18 +91,6 @@ typedef struct lasr_gemm_args {
      * Lets a ragged N (T' = 299 attention scores in a 304-wide buffer) run entirely on the vector epilogue; the consumer
      * ignores those padding columns.  No bias/res/aux/dact/colsum. */
     int32_t n_store;
-    /* recompute (optional, with act = swish|relu and colsum allowed; no bias/res/aux/dact):
-     *   C = alpha * (A.B^T) * act'(A2.B2^T + bias2)
-     * The pre-activation of the forward Linear (A2 (M,K) row-major = its input, B2 (N,K) row-major = its weight, bias2 its bias)
-     * is RECOMPUTED on the tensor cores into a second TMEM accumulator of the same tile instead of being saved by the forward
-     * pass and read back: the FFN forward then writes one (M,N) tensor instead of two and this GEMM reads (M,K) instead of (M,N)
-     * (nets/feed_forward.py:18-19 backward; N = 2048 against K = 256 at C2).  Needs k2 == K of this GEMM's own contraction
-     * length in 64-blocks, bf16 operands and C, no batching. */
-    const void* a2;
-    const void* b2;
-    const float* bias2;
-    int64_t lda2, ldb2;
-    int32_t k2;
     /* dropout on the output (optional; the reference's nn.Dropout sites that sit right behind a Linear: nets/feed_forward.py:19,
      * nets/conformer_layer.py:42,54,63,125, nets/transformer_layer.py:48,58,174, nets/positional_encoding.py:75, and -- as the
      * backward of nets/ctc.py:29 -- the input gradient of ctc_lo):
@@ -111,7 +99,7 @@ typedef struct lasr_gemm_args {
      * (row, column) -- see the "dropout" section below; drop_thr = round(p * 32768) <= 0x7c00 (0 = off), drop_scale = 32768 / (32768 - thr).
      * drop_mark_aux = 1: dropped elements of `aux` (the saved pre-activation) receive -1e30, whose act'() is exactly 0, so the
      * activation-backward GEMM (dact = aux) applies the SAME mask without regenerating it (its alpha carries drop_scale).
-     * Unbatched GEMMs only; not with accumulate / dact / n_store / recompute. */
+     * Unbatched GEMMs only; not with accumulate / dact / n_store. */
     const void* drop_state;
     uint32_t drop_site;
     uint32_t drop_thr;

@@ -29,7 +29,6 @@ class GemmArgs(C.Structure):
         ("alpha", C.c_float), ("act", C.c_int32), ("accumulate", C.c_int32), ("split_k", C.c_int32),
         ("dact", C.c_void_p), ("lddact", C.c_int64), ("colsum", C.c_void_p), ("cs1", C.c_int64), ("cs2", C.c_int64),
         ("n_store", C.c_int32),
-        ("a2", C.c_void_p), ("b2", C.c_void_p), ("bias2", C.c_void_p), ("lda2", C.c_int64), ("ldb2", C.c_int64), ("k2", C.c_int32),
         ("drop_state", C.c_void_p), ("drop_site", C.c_uint32), ("drop_thr", C.c_uint32), ("drop_scale", C.c_float),
         ("drop_mark_aux", C.c_int32), ("aux_deriv", C.c_int32),
     ]

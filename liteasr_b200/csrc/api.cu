@@ -34,7 +34,7 @@ int gemm_simt_dispatch(const lasr_gemm_args* a, cudaStream_t st);
 
 extern "C" {
 
-int lasr_version(void) { return 1; }
+int lasr_version(void) { return 2; }
 int lasr_arch(void) { return 100; }
 const char* lasr_last_error(void) { return lasr::g_err; }
 unsigned long long lasr_launch_count(void) { return lasr::g_launches; }
@@ -53,20 +53,15 @@ int lasr_gemm(const lasr_gemm_args* a, void* stream) {
                      "gemm: dact needs act = swish|relu|mul and no bias/res/aux");
     else
         LASR_REQUIRE(a->act != LASR_ACT_MUL, "gemm: act = mul needs dact");
-    if (a->aux_deriv) LASR_REQUIRE(a->aux && a->act == LASR_ACT_SWISH && !a->a2, "gemm: aux_deriv needs aux and act = swish");
-    if (a->a2)
-        LASR_REQUIRE(a->b2 && a->ab_dtype == LASR_BF16 && a->c_dtype == LASR_BF16 && !a->bias && !a->res && !a->aux && !a->dact &&
-                         !a->accumulate && !a->n_store && a->batch1 == 1 && a->batch2 == 1 && !a->trans_a && a->k2 > 0 &&
-                         (a->k2 + 63) / 64 == (a->k + 63) / 64 && (a->act == LASR_ACT_SWISH || a->act == LASR_ACT_RELU),
-                     "gemm: recompute needs bf16 operands and C, act = swish|relu, equal K block counts, no batching and no other epilogue operand");
+    if (a->aux_deriv) LASR_REQUIRE(a->aux && a->act == LASR_ACT_SWISH, "gemm: aux_deriv needs aux and act = swish");
     if (a->split_k > 1) LASR_REQUIRE(a->accumulate, "gemm: split_k > 1 requires accumulate");
     if (a->n_store)
         LASR_REQUIRE(a->n_store >= a->n && a->n_store <= a->ldc && !a->bias && !a->res && !a->aux && !a->dact && !a->colsum && !a->accumulate,
                      "gemm: n_store must satisfy n <= n_store <= ldc and excludes every epilogue operand");
     if (a->drop_thr)
         LASR_REQUIRE(a->drop_state && a->drop_thr <= 0x7c00u && a->batch1 == 1 && a->batch2 == 1 && !a->accumulate && !a->dact && !a->n_store &&
-                         !a->a2 && !a->colsum,
-                     "gemm: dropout needs drop_state, thr = round(p * 32768) <= 0x7c00, an unbatched GEMM and no accumulate / dact / n_store / recompute / colsum");
+                         !a->colsum,
+                     "gemm: dropout needs drop_state, thr = round(p * 32768) <= 0x7c00, an unbatched GEMM and no accumulate / dact / n_store / colsum");
     cudaStream_t st = (cudaStream_t)stream;
     if (a->ab_dtype == LASR_BF16) return gemm_tc_dispatch(a, st);
     if (a->ab_dtype == LASR_F32) {

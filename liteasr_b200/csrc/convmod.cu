@@ -717,9 +717,7 @@ static int glu_dwconv_fwd_launch(const void* y2, int dtype, int64_t ldy, const f
     LASR_REQUIRE(y2 && w && bias && z && partial && B > 0 && T > 0 && d > 0 && d % 2 == 0 && ldy % 2 == 0, "glu_dwconv_fwd: bad args");
     cudaStream_t st = (cudaStream_t)stream;
     const bool fast = fast_d(d) && ldy % 4 == 0 && ((uintptr_t)y2 & 15) == 0 && ((uintptr_t)z & 15) == 0;
-    static int stream_on = -1;  // LASR_CONVMOD_STREAM=0: developer switch back to the tiled kernels
-    if (stream_on < 0) { const char* e = getenv("LASR_CONVMOD_STREAM"); stream_on = e ? atoi(e) : 1; }
-    if (stream_on && dtype == LASR_BF16 && d % SCH == 0 && ldy % 8 == 0 && ((uintptr_t)y2 & 15) == 0) {
+    if (dtype == LASR_BF16 && d % SCH == 0 && ldy % 8 == 0 && ((uintptr_t)y2 & 15) == 0) {
         launch_pdl(glu_dwconv_fwd_stream_kernel<LENS>, dim3(d / SCH, B), 256, 0, st, (const bf16*)y2, ldy, w, bias, z, partial, T, d, lens);
         return check_launch("glu_dwconv_fwd");
     }

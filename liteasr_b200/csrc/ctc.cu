@@ -13,8 +13,6 @@
 //        grad[t,b,label_k] -= s * occ_label  (red.add; only rows t < in_len[b], only L+1 addresses per row).
 // Physical traffic is therefore ~1 read + 1 write of the (T,B,V) tensor plus O(T*B*L) lattice state,
 // instead of the ~7 dense passes of log_softmax + ctc_loss + their backward kernels.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace lasr {
@@ -48,10 +46,6 @@ template <> struct Vec4<bf16> {
     }
 };
 
-
-__device__ __forceinline__ void red_sub(float* p, float v) { atomicAdd(p, -v); }
-__device__ __forceinline__ void red_sub(bf16* p, float v) { atomicAdd(p, __float2bfloat16_rn(-v)); }
-
 struct CtcDenseParams {
     const void* logits;
     void* grad;
@@ -63,10 +57,6 @@ struct CtcDenseParams {
     int T, B, V, lmax, blank;
     float grad_scale;
     const float* upstream;
-    // two-pass pipeline (see ctc_launch): utterance group [b0, b0 + nb), per-row log-sum-exp, lattice occupancies
-    int b0, nb;
-    float* lse;            // (T, B) natural-log units
-    const float2* occ;     // (B, T, lmax+1): (blank, label) state occupancies written by the lattice
 };
 
 // GROUP threads cooperate on one row; each holds NI chunks of 4 consecutive classes in registers.
@@ -173,155 +163,6 @@ __global__ void __launch_bounds__(256) ctc_softmax_gather_kernel(const CtcDenseP
                     if (c + j < p.V) gout[c + j] = from_f32<T>(0.f);
             }
         }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// two-pass pipeline kernels.  PASS 1: per row log-sum-exp + compact lattice inputs, no gradient write.
-// PASS 3: grad = s * (exp(x - lse) - occupancy), the occupancy of the row's L+1 classes subtracted with red.add right
-// after the row is written (the sectors are still in L2: no DRAM read-modify-write, unlike a separate scatter pass).
-// Rows are (t, b) with b in the utterance group [b0, b0 + nb).
-// ---------------------------------------------------------------------------------------------
-template <typename T, int GROUP, int NI, int PASS>
-__global__ void __launch_bounds__(256) ctc_pass_kernel(const CtcDenseParams p) {
-    constexpr int ROWS = 256 / GROUP;
-    __shared__ float red[ROWS][8];
-    const int g = threadIdx.x / GROUP, gl = threadIdx.x % GROUP;
-    const long row = (long)blockIdx.x * ROWS + g;
-    const bool row_ok = row < (long)p.T * p.nb;
-    const int t = row_ok ? (int)(row / p.nb) : 0, b = p.b0 + (row_ok ? (int)(row % p.nb) : 0);
-    const int Tb = (int)p.in_len[b];
-    const bool live = row_ok && t < Tb;
-    const T* x = reinterpret_cast<const T*>(p.logits) + (long)t * p.st + (long)b * p.sb;
-    typedef typename Vec4<T>::type V4;
-    float v[NI][4];
-    if (live) {
-#pragma unroll
-        for (int i = 0; i < NI; ++i) {
-            const int c = (i * GROUP + gl) * 4;
-            if (c + 3 < p.V) {
-                const V4 raw = *reinterpret_cast<const V4*>(x + c);
-                Vec4<T>::unpack(raw, v[i]);
-            } else {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) v[i][j] = (c + j < p.V) ? to_f32<T>(x[c + j]) : -INFINITY;
-            }
-        }
-    }
-    if (PASS == 1) {
-        float mx = -INFINITY;
-        if (live) {
-#pragma unroll
-            for (int i = 0; i < NI; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) mx = fmaxf(mx, v[i][j]);
-        }
-        mx = warp_max(mx);
-        if (GROUP != 32) {
-            if ((threadIdx.x & 31) == 0) red[0][threadIdx.x >> 5] = mx;
-            __syncthreads();
-            mx = red[0][0];
-#pragma unroll
-            for (int w = 1; w < 8; ++w) mx = fmaxf(mx, red[0][w]);
-            __syncthreads();
-        }
-        float sum = 0.f;
-        if (live) {
-#pragma unroll
-            for (int i = 0; i < NI; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) sum += expf(v[i][j] - mx);  // exp(-inf) = 0 for the padded tail
-        }
-        sum = warp_sum(sum);
-        if (GROUP != 32) {
-            if ((threadIdx.x & 31) == 0) red[0][threadIdx.x >> 5] = sum;
-            __syncthreads();
-            sum = 0.f;
-#pragma unroll
-            for (int w = 0; w < 8; ++w) sum += red[0][w];
-        }
-        if (!live) return;
-        const float lse = mx + logf(sum);
-        if (gl == 0) p.lse[(long)t * p.B + b] = lse;
-        const int L = (int)p.tgt_len[b];
-        float* le = p.lp_ext + ((long)b * p.T + t) * (p.lmax + 1);
-        const int64_t* tg = p.targets + (long)b * p.lmax;
-        const float xb = to_f32<T>(x[p.blank]);
-        for (int k2 = gl; k2 <= L; k2 += GROUP)  // log2 units: the lattice runs on ex2 / lg2 directly
-            le[k2] = LOG2E * ((k2 == 0) ? (xb - lse) : (to_f32<T>(x[(int)tg[k2 - 1]]) - xb));
-    } else {
-        T* gout = reinterpret_cast<T*>(p.grad) + (long)t * p.gst + (long)b * p.gsb;
-        float s = p.grad_scale;
-        if (p.upstream) s *= __ldg(p.upstream);
-        float bsum = 0.f;
-        const int L = live ? min((int)p.tgt_len[b], p.lmax) : 0;
-        const float2* oc = p.occ + ((long)b * p.T + t) * (p.lmax + 1);
-        float2 myocc[(GROUP == 32) ? 8 : 4];  // this thread's share of the row's L+1 occupancies (lmax + 1 <= 1024 = 256 * 4)
-        if (live) {
-            const float lse = p.lse[(long)t * p.B + b];
-#pragma unroll
-            for (int e = 0; e < ((GROUP == 32) ? 8 : 4); ++e) {
-                const int k = gl + e * GROUP;
-                myocc[e] = (k <= L) ? __ldcg(oc + k) : make_float2(0.f, 0.f);
-            }
-#pragma unroll
-            for (int i = 0; i < NI; ++i) {
-                const int c = (i * GROUP + gl) * 4;
-                float o[4];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) o[j] = s * expf(v[i][j] - lse);
-                if (c + 3 < p.V) {
-                    *reinterpret_cast<V4*>(gout + c) = Vec4<T>::pack(o);
-                } else {
-#pragma unroll
-                    for (int j = 0; j < 4; ++j)
-                        if (c + j < p.V) gout[c + j] = from_f32<T>(o[j]);
-                }
-            }
-        } else if (row_ok) {
-            float z[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-            for (int i = 0; i < NI; ++i) {
-                const int c = (i * GROUP + gl) * 4;
-                if (c + 3 < p.V) {
-                    *reinterpret_cast<V4*>(gout + c) = Vec4<T>::pack(z);
-                } else {
-#pragma unroll
-                    for (int j = 0; j < 4; ++j)
-                        if (c + j < p.V) gout[c + j] = from_f32<T>(0.f);
-                }
-            }
-        }
-        __syncthreads();  // the row's plain stores are ordered before the red.adds of other threads of the CTA
-        if (live) {
-            const int64_t* tg = p.targets + (long)b * p.lmax;
-            // GROUP == 32 with lmax + 1 > 256 cannot hold the row's occupancies in 8 registers per lane: loop instead
-            if (GROUP == 32 && p.lmax + 1 > 256) {
-                for (int k = gl; k <= L; k += 32) {
-                    const float2 o = __ldcg(oc + k);
-                    bsum += o.x;
-                    if (k < L) red_sub(gout + (int)tg[k], s * o.y);
-                }
-            } else {
-#pragma unroll
-                for (int e = 0; e < ((GROUP == 32) ? 8 : 4); ++e) {
-                    const int k = gl + e * GROUP;
-                    if (k <= L) {
-                        bsum += myocc[e].x;
-                        if (k < L) red_sub(gout + (int)tg[k], s * myocc[e].y);
-                    }
-                }
-            }
-        }
-        bsum = warp_sum(bsum);
-        if (GROUP != 32) {
-            if ((threadIdx.x & 31) == 0) red[0][threadIdx.x >> 5] = bsum;
-            __syncthreads();
-            bsum = 0.f;
-#pragma unroll
-            for (int w = 0; w < 8; ++w) bsum += red[0][w];
-        }
-        if (live && gl == 0) red_sub(gout + p.blank, s * bsum);
     }
 }
 
@@ -576,275 +417,6 @@ __global__ void __launch_bounds__(32 * NW) ctc_lattice_warp_kernel(const float* 
     }
 }
 
-// ---------------------------------------------------------------------------------------------
-// K_B', meet-in-the-middle lattice with the gradient scatter inside the sweeps (default path).
-// CTAs 2b (alpha) and 2b+1 (beta) of utterance b sweep towards each other and meet at row m = T_b / 2 (ONE flag exchange per
-// utterance).  At the meeting both know alpha_m and beta_m, hence the total log-likelihood (log-sum over the states of row m);
-// from there on the alpha CTA walks rows m .. T_b-1, where beta is already in memory, and the beta CTA rows m-1 .. 0, where
-// alpha is: each forms the occupancy 2^(alpha + beta - e - tot) of its own state pairs right after the recursion step and
-// subtracts it from the gradient row with red.add.  The separate scatter kernel (a second pass over alpha, beta and 201
-// scattered sectors of every gradient row: 0.36 ms of the 1.15 ms at T=1600, V=5000) disappears into the issue slots the
-// latency-bound recursion leaves idle.  CTA pairs are adjacent in launch order, so a waiting CTA's partner is always resident
-// or next in line; the wait traps after LASR_DEVICE_TIMEOUT_CYCLES instead of hanging.
-// ---------------------------------------------------------------------------------------------
-
-template <typename GT, int R, int PFW, int NW, bool OCC>
-struct MeetLattice {
-    const float* lpb;
-    float2* own;
-    const float2* partner;
-    GT* gb;
-    long gst;
-    int W, tid, lane, warp, blank;
-    float s, tot;
-    bool feasible;
-    int kcol[R], kidx[R], cls[R];
-    bool v_bl[R], v_lb[R], skip[R];
-    float s_bl[R], s_lb[R];
-    float (*edge)[2][NW];
-    float2* occ;  // OCC: occupancies (blank, label) of row t replace alpha_t in the alpha array (read by the final gradient pass)
-
-    __device__ __forceinline__ void scatter(int t, const float2 (&pp)[R], const float (&e)[R]) {
-        GT* g = gb + (long)t * gst;
-        const float qnan = __int_as_float(0x7fc00000);
-        float bsum = 0.f;
-#pragma unroll
-        for (int r = 0; r < R; ++r) {
-            float o_bl = fex2(s_bl[r] + pp[r].x - tot);
-            float o_lb = fex2(s_lb[r] + pp[r].y - e[r] - tot);
-            if (!feasible) { o_bl = qnan; o_lb = qnan; }
-            if (OCC) {
-                if (tid * R + r < W) occ[(long)t * W + tid * R + r] = make_float2(v_bl[r] ? o_bl : 0.f, v_lb[r] ? o_lb : 0.f);
-            } else {
-                if (v_lb[r]) red_sub(g + cls[r], s * o_lb);
-                bsum += v_bl[r] ? o_bl : 0.f;
-            }
-        }
-        if (!OCC) {
-            bsum = warp_sum(bsum);
-            if (lane == 0) red_sub(g + blank, s * bsum);
-        }
-    }
-
-    // n recursion steps starting at row t_first in sweep direction; PH2: also scatter every row (partner rows prefetched)
-    template <bool BETA, bool PH2>
-    __device__ __forceinline__ void run(int t_first, int n) {
-        if (n <= 0) return;  // CTA-uniform
-        constexpr int DIR = BETA ? -1 : 1;
-        const float NEG = LNEG;
-        float cl[PFW][R], nl[PFW][R];
-        float2 pc[PFW][R], pn[PFW][R];
-#pragma unroll
-        for (int i = 0; i < PFW; ++i) {
-            const long t = t_first + DIR * min(i, n - 1);
-#pragma unroll
-            for (int r = 0; r < R; ++r) {
-                cl[i][r] = lpb[t * W + kcol[r]];
-                if (PH2) pc[i][r] = __ldcg(partner + t * W + kidx[r]);
-            }
-        }
-        for (int j0 = 0; j0 < n; j0 += PFW) {
-#pragma unroll
-            for (int i = 0; i < PFW; ++i) {
-                const long t = t_first + DIR * min(j0 + PFW + i, n - 1);
-#pragma unroll
-                for (int r = 0; r < R; ++r) {
-                    nl[i][r] = lpb[t * W + kcol[r]];
-                    if (PH2) pn[i][r] = __ldcg(partner + t * W + kidx[r]);
-                }
-            }
-#pragma unroll
-            for (int i = 0; i < PFW; ++i) {
-                if (j0 + i < n) {  // CTA-uniform
-                    const int t = t_first + DIR * (j0 + i);
-                    float n_bl[R], n_lb[R];
-                    if (!BETA) {
-                        float up = __shfl_up_sync(0xffffffffu, s_lb[R - 1], 1);
-                        if (lane == 0) up = (NW > 1 && warp > 0) ? edge[(t - 1) & 1][0][warp - 1] : NEG;
-#pragma unroll
-                        for (int r = 0; r < R; ++r) {
-                            const float prev = (r == 0) ? up : s_lb[r - 1];   // alpha_{t-1}(2k-1)
-                            n_bl[r] = lse2q(s_bl[r], prev);
-                            n_lb[r] = cl[i][r] + lse3q(s_lb[r], s_bl[r], skip[r] ? prev : NEG);
-                        }
-#pragma unroll
-                        for (int r = 0; r < R; ++r) { s_bl[r] = n_bl[r]; s_lb[r] = n_lb[r]; }
-                    } else {
-                        float d1 = __shfl_down_sync(0xffffffffu, s_bl[0], 1);  // beta_{t+1}(2k+2) of the next thread's first pair
-                        float d2 = __shfl_down_sync(0xffffffffu, s_lb[0], 1);  // beta_{t+1}(2k+3)
-                        if (lane == 31) {
-                            const bool has = NW > 1 && warp + 1 < NW;
-                            d1 = has ? edge[(t + 1) & 1][0][warp + 1] : NEG;
-                            d2 = has ? edge[(t + 1) & 1][1][warp + 1] : NEG;
-                        }
-#pragma unroll
-                        for (int r = 0; r < R; ++r) {
-                            const float x1 = (r == R - 1) ? d1 : s_bl[r + 1];
-                            const float x2 = (r == R - 1) ? d2 : s_lb[r + 1];
-                            n_bl[r] = lse2q(s_bl[r], s_lb[r]);
-                            n_lb[r] = cl[i][r] + lse3q(s_lb[r], x1, skip[r] ? x2 : NEG);
-                        }
-                        // dead LABEL states must be forced: their emission column was never written by the gather kernel
-#pragma unroll
-                        for (int r = 0; r < R; ++r) { s_bl[r] = n_bl[r]; s_lb[r] = v_lb[r] ? n_lb[r] : NEG; }
-                    }
-                    if (!(PH2 && OCC)) {  // past the meeting nobody reads this sweep's values from memory
-#pragma unroll
-                        for (int r = 0; r < R; ++r)
-                            if (tid * R + r < W) own[(long)t * W + tid * R + r] = make_float2(s_bl[r], s_lb[r]);
-                    }
-                    if (NW > 1) {
-                        if (!BETA) {
-                            if (lane == 31) edge[t & 1][0][warp] = s_lb[R - 1];
-                        } else if (lane == 0) {
-                            edge[t & 1][0][warp] = s_bl[0];
-                            edge[t & 1][1][warp] = s_lb[0];
-                        }
-                        __syncthreads();
-                    }
-                    if (PH2) scatter(t, pc[i], cl[i]);
-                }
-            }
-#pragma unroll
-            for (int i = 0; i < PFW; ++i)
-#pragma unroll
-                for (int r = 0; r < R; ++r) {
-                    cl[i][r] = nl[i][r];
-                    if (PH2) pc[i][r] = pn[i][r];
-                }
-        }
-    }
-};
-
-template <typename GT, int R, int PFW, int NW, bool OCC>
-__global__ void __launch_bounds__(32 * NW) ctc_lattice_meet_kernel(const float* __restrict__ lp_ext, float2* al, float2* be,
-                                                                   const int64_t* __restrict__ targets,
-                                                                   const int64_t* __restrict__ in_len,
-                                                                   const int64_t* __restrict__ tgt_len, float* __restrict__ nll,
-                                                                   float* __restrict__ tot_out, int* flags, void* grad, long gst,
-                                                                   long gsb, int blank, float grad_scale, const float* upstream,
-                                                                   int T, int lmax, int b0) {
-    __shared__ float edge[2][2][NW];
-    __shared__ float scratch[32];
-    const int b = b0 + (blockIdx.x >> 1), tid = threadIdx.x;
-    const bool is_beta = (blockIdx.x & 1) != 0;
-    const int Tb = min((int)in_len[b], T), L = min((int)tgt_len[b], lmax);
-    const int W = lmax + 1;
-    if (Tb <= 0) {
-        if (!is_beta && tid == 0) { nll[b] = (L == 0) ? 0.f : INFINITY; tot_out[b] = (L == 0) ? 0.f : -INFINITY; }
-        return;
-    }
-    const int64_t* tg = targets + (long)b * lmax;
-    const float NEG = LNEG;
-    MeetLattice<GT, R, PFW, NW, OCC> lt;
-    lt.lpb = lp_ext + (long)b * T * W;
-    lt.own = (is_beta ? be : al) + (long)b * T * W;
-    lt.partner = (is_beta ? al : be) + (long)b * T * W;
-    lt.gb = reinterpret_cast<GT*>(grad) + (long)b * gsb;
-    lt.gst = gst;
-    lt.W = W; lt.tid = tid; lt.lane = tid & 31; lt.warp = tid >> 5; lt.blank = blank;
-    lt.s = grad_scale * (upstream ? __ldg(upstream) : 1.f);
-    lt.edge = edge;
-    lt.occ = al + (long)b * T * W;
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-        const int k = tid * R + r;
-        lt.kcol[r] = min(k, lmax - 1) + 1;
-        lt.kidx[r] = min(k, W - 1);
-        lt.v_bl[r] = k <= L;
-        lt.v_lb[r] = k < L;
-        const long my = (k < L) ? tg[k] : -1;
-        lt.cls[r] = (k < L) ? (int)my : 0;
-        if (!is_beta) lt.skip[r] = (k >= 1 && k < L) && (tg[k - 1] != my);   // alpha: 2k-1 -> 2k+1 allowed
-        else lt.skip[r] = (k + 1 < L) && (tg[k + 1] != my);                    // beta : 2k+1 -> 2k+3 allowed
-    }
-    const int m = Tb >> 1;  // meeting row
-    double csum = 0.0;
-    if (!is_beta) {
-        // C = sum_t lp_t(blank) (double, log2 units): the normalisation offset of the blank-normalised recursion
-        if (lt.warp == 0) {
-            for (int t = lt.lane; t < Tb; t += 32) csum += (double)lt.lpb[(long)t * W];
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) csum += __shfl_xor_sync(0xffffffffu, csum, o);
-        }
-#pragma unroll
-        for (int r = 0; r < R; ++r) {
-            const int k = tid * R + r;
-            lt.s_bl[r] = (k == 0) ? 0.f : NEG;
-            lt.s_lb[r] = (k == 0 && L > 0) ? lt.lpb[lt.kcol[r]] : NEG;
-            if (k < W) lt.own[k] = make_float2(lt.s_bl[r], lt.s_lb[r]);
-        }
-        if (NW > 1) {
-            if (lt.lane == 31) edge[0][0][lt.warp] = lt.s_lb[R - 1];
-            __syncthreads();
-        }
-        lt.template run<false, false>(1, m);  // rows 1 .. m
-    } else {
-        const int t = Tb - 1;
-#pragma unroll
-        for (int r = 0; r < R; ++r) {
-            const int k = tid * R + r;
-            const float ld_ = lt.lpb[(long)t * W + lt.kcol[r]];
-            lt.s_bl[r] = (k == L) ? 0.f : NEG;
-            lt.s_lb[r] = (L > 0 && k == L - 1) ? ld_ : NEG;
-            if (k < W) lt.own[(long)t * W + k] = make_float2(lt.s_bl[r], lt.s_lb[r]);
-        }
-        if (NW > 1) {
-            if (lt.lane == 0) { edge[t & 1][0][lt.warp] = lt.s_bl[0]; edge[t & 1][1][lt.warp] = lt.s_lb[0]; }
-            __syncthreads();
-        }
-        lt.template run<true, false>(Tb - 2, Tb - 1 - m);  // rows Tb-2 .. m
-    }
-    // ---- meeting: publish "my rows up to m are in memory", wait for the partner's
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) {
-        int* mine = flags + 2 * b + (is_beta ? 1 : 0);
-        const int* theirs = flags + 2 * b + (is_beta ? 0 : 1);
-        asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(mine), "r"(1) : "memory");
-        int v = 0;
-        const long long t0 = clock64();
-        do {
-            asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(theirs) : "memory");
-            if (v == 0 && clock64() - t0 > LASR_DEVICE_TIMEOUT_CYCLES) __trap();  // never hang the box
-        } while (v == 0);
-    }
-    __syncthreads();
-    // ---- total log-likelihood from row m: tot = log2 sum_s 2^(alpha_m(s) + beta_m(s) - e_m(s))
-    float2 pm[R];
-    float em[R];
-    {
-        float x[2 * R], mx = 4.f * NEG;
-#pragma unroll
-        for (int r = 0; r < R; ++r) {
-            pm[r] = __ldcg(lt.partner + (long)m * W + lt.kidx[r]);
-            em[r] = lt.lpb[(long)m * W + lt.kcol[r]];
-            x[2 * r] = lt.v_bl[r] ? lt.s_bl[r] + pm[r].x : 4.f * NEG;
-            x[2 * r + 1] = lt.v_lb[r] ? lt.s_lb[r] + pm[r].y - em[r] : 4.f * NEG;
-            mx = fmaxf(mx, fmaxf(x[2 * r], x[2 * r + 1]));
-        }
-        mx = block_max(mx, scratch);
-        float sum = 0.f;
-#pragma unroll
-        for (int r = 0; r < 2 * R; ++r) sum += fex2(x[r] - mx);
-        sum = block_sum(sum, scratch);
-        lt.tot = mx + flg2(sum);
-        lt.feasible = lt.tot > 0.5f * LNEG;
-    }
-    if (!is_beta) {
-        if (tid == 0) {
-            nll[b] = lt.feasible ? (float)(-((double)lt.tot + csum) * LN2) : INFINITY;
-            tot_out[b] = lt.feasible ? lt.tot : -INFINITY;
-        }
-        if (!OCC) lt.scatter(m, pm, em);                        // row m (RED mode)
-        lt.template run<false, true>(m + 1, Tb - 1 - m);       // rows m+1 .. Tb-1
-    } else {
-        // OCC mode: row m belongs to the beta CTA -- it is the only reader of alpha_m in memory, so it may overwrite it
-        if (OCC) lt.scatter(m, pm, em);
-        lt.template run<true, true>(m - 1, m);                 // rows m-1 .. 0
-    }
-}
-
 // scatter for the split lattice: occupancy formed on the fly from alpha, beta, the label emission term and tot
 template <typename GT>
 __global__ void __launch_bounds__(256) ctc_scatter_ab_kernel(const float2* __restrict__ al, const float2* __restrict__ be,
@@ -889,97 +461,11 @@ __global__ void __launch_bounds__(256) ctc_scatter_ab_kernel(const float2* __res
     }
 }
 
-template <typename T, int PASS>
-static void launch_pass(const CtcDenseParams& q, cudaStream_t st) {
-    const long rows = (long)q.T * q.nb;
-    const int chunks = (q.V + 3) / 4;
-    bool done = false;
-#define LASR_CTC_CASE(GROUP, NI)                                                                  \
-    if (!done && chunks <= GROUP * NI) {                                                          \
-        ctc_pass_kernel<T, GROUP, NI, PASS><<<ceil_div(rows, 256 / GROUP), 256, 0, st>>>(q);      \
-        done = true;                                                                              \
-    }
-    LASR_CTC_CASE(32, 1) LASR_CTC_CASE(32, 2) LASR_CTC_CASE(32, 4) LASR_CTC_CASE(32, 8)
-    LASR_CTC_CASE(256, 2) LASR_CTC_CASE(256, 4) LASR_CTC_CASE(256, 6) LASR_CTC_CASE(256, 8)
-#undef LASR_CTC_CASE
-}
-
-// Two-pass pipeline (default for vectorisable layouts with V <= 8192):
-//   pass 1 (stream order, all SMs)  per-row log-sum-exp + lattice inputs          reads the logits once
-//   lattice (2 CTAs per utterance)  meet-in-the-middle sweeps, occupancies replace alpha in the workspace
-//   pass 3 (all SMs)                grad = s * (softmax - occupancy)               reads the logits again, writes the gradient
-// Large problems are split into utterance groups: the latency-bound lattice of group g runs on a side stream while pass 1 of
-// the later groups and pass 3 of the earlier groups keep HBM busy on the caller's stream (fork / join with events, legal
-// under stream capture).  No read-modify-write of the gradient in DRAM, no separate scatter pass.
-static const int CTC_MAX_GROUPS = 8;
 template <typename T>
-static int ctc_launch_twopass(CtcDenseParams p, float2* ab, float2* be, float* tot, int* flags, float* nll, cudaStream_t st) {
-    const int W = p.lmax + 1;
-    p.occ = ab;
-    int G = 1;
-    if ((double)p.T * p.B * p.V >= 6.4e7 && p.B >= 16) G = p.B / 8 < CTC_MAX_GROUPS ? p.B / 8 : CTC_MAX_GROUPS;
-    static cudaStream_t side[CTC_MAX_GROUPS];
-    static cudaEvent_t e1[CTC_MAX_GROUPS], e2[CTC_MAX_GROUPS];
-    static bool pool = false;
-    if (G > 1 && !pool) {
-        for (int i = 0; i < CTC_MAX_GROUPS; ++i) {
-            if (cudaStreamCreateWithFlags(&side[i], cudaStreamNonBlocking) != cudaSuccess ||
-                cudaEventCreateWithFlags(&e1[i], cudaEventDisableTiming) != cudaSuccess ||
-                cudaEventCreateWithFlags(&e2[i], cudaEventDisableTiming) != cudaSuccess)
-                return check_launch("ctc stream pool");
-        }
-        pool = true;
-    }
-    if (cudaMemsetAsync(flags, 0, 2 * (size_t)p.B * sizeof(int), st) != cudaSuccess) return check_launch("ctc flags");
-    const int per = ceil_div(p.B, G);
-    for (int g = 0; g < G; ++g) {
-        CtcDenseParams q = p;
-        q.b0 = g * per;
-        q.nb = p.B - q.b0 < per ? p.B - q.b0 : per;
-        if (q.nb <= 0) break;
-        launch_pass<T, 1>(q, st);
-        if (G > 1 && cudaEventRecord(e1[g], st) != cudaSuccess) return check_launch("ctc event");
-    }
-    int rc = check_launch("ctc_pass1");
-    if (rc) return rc;
-    for (int g = 0; g < G; ++g) {
-        const int b0 = g * per, nb = p.B - b0 < per ? p.B - b0 : per;
-        if (nb <= 0) break;
-        cudaStream_t sg = G > 1 ? side[g] : st;
-        if (G > 1 && cudaStreamWaitEvent(sg, e1[g], 0) != cudaSuccess) return check_launch("ctc wait");
-#define LASR_MEET(R, PFW, NW)                                                                                                  \
-    ctc_lattice_meet_kernel<T, R, PFW, NW, true><<<2 * nb, 32 * NW, 0, sg>>>(p.lp_ext, ab, be, p.targets, p.in_len, p.tgt_len, nll, tot, flags, \
-                                                                              p.grad, p.gst, p.gsb, p.blank, p.grad_scale, p.upstream, p.T, p.lmax, b0)
-        if (W <= 32) LASR_MEET(1, 8, 1);
-        else if (W <= 64) LASR_MEET(2, 8, 1);
-        else if (W <= 128) LASR_MEET(2, 8, 2);
-        else if (W <= 256) LASR_MEET(2, 8, 4);
-        else if (W <= 512) LASR_MEET(2, 8, 8);
-        else LASR_MEET(4, 4, 8);
-#undef LASR_MEET
-        if (G > 1 && cudaEventRecord(e2[g], sg) != cudaSuccess) return check_launch("ctc event");
-    }
-    rc = check_launch("ctc_lattice_meet");
-    if (rc) return rc;
-    for (int g = 0; g < G; ++g) {
-        CtcDenseParams q = p;
-        q.b0 = g * per;
-        q.nb = p.B - q.b0 < per ? p.B - q.b0 : per;
-        if (q.nb <= 0) break;
-        if (G > 1 && cudaStreamWaitEvent(st, e2[g], 0) != cudaSuccess) return check_launch("ctc wait");
-        launch_pass<T, 3>(q, st);
-    }
-    return check_launch("ctc_pass3");
-}
-
-template <typename T>
-static int ctc_launch(const CtcDenseParams& p, float2* ab, float2* be, float* tot, int* flags, float* nll, cudaStream_t st) {
+static int ctc_launch(const CtcDenseParams& p, float2* ab, float2* be, float* tot, float* nll, cudaStream_t st) {
     const long rows = (long)p.T * p.B;
     const bool vec = ((reinterpret_cast<uintptr_t>(p.logits) | reinterpret_cast<uintptr_t>(p.grad)) % (4 * sizeof(T)) == 0) &&
                      p.st % 4 == 0 && p.sb % 4 == 0 && p.gst % 4 == 0 && p.gsb % 4 == 0;
-    static int pipe = -1;  // LASR_CTC_PIPE=0: developer switch back to the single-pass gather + separate scatter
-    if (pipe < 0) { const char* e = getenv("LASR_CTC_PIPE"); pipe = e ? atoi(e) : 0; }
-    if (pipe && vec && (p.V + 3) / 4 <= 2048) return ctc_launch_twopass<T>(p, ab, be, tot, flags, nll, st);
     bool done = false;
     if (vec) {
         const int chunks = (p.V + 3) / 4;
@@ -995,40 +481,22 @@ static int ctc_launch(const CtcDenseParams& p, float2* ab, float2* be, float* to
     if (!done) ctc_softmax_gather_generic<T><<<(unsigned)rows, 256, 0, st>>>(p);
     int rc = check_launch("ctc_softmax_gather");
     if (rc) return rc;
+    // R state pairs per thread, NW warps per sweep (32 R NW >= W)
     const int W = p.lmax + 1;
-    {
-        // R state pairs per thread, NW warps per sweep (32 R NW >= W)
-        static int fused = -1;  // LASR_CTC_FUSED=0: developer switch back to separate sweeps + scatter kernel
-        if (fused < 0) { const char* e = getenv("LASR_CTC_FUSED"); fused = e ? atoi(e) : 0; }
-        if (fused) {
-            if (cudaMemsetAsync(flags, 0, 2 * (size_t)p.B * sizeof(int), st) != cudaSuccess) return check_launch("ctc flags");
-#define LASR_MEET(R, PFW, NW)                                                                                                  \
-    ctc_lattice_meet_kernel<T, R, PFW, NW, false><<<2 * p.B, 32 * NW, 0, st>>>(p.lp_ext, ab, be, p.targets, p.in_len, p.tgt_len, nll, tot, flags, \
-                                                                                p.grad, p.gst, p.gsb, p.blank, p.grad_scale, p.upstream, p.T, p.lmax, 0)
-            if (W <= 32) LASR_MEET(1, 8, 1);
-            else if (W <= 64) LASR_MEET(2, 8, 1);
-            else if (W <= 128) LASR_MEET(2, 8, 2);
-            else if (W <= 256) LASR_MEET(2, 8, 4);
-            else if (W <= 512) LASR_MEET(2, 8, 8);
-            else LASR_MEET(4, 4, 8);
-#undef LASR_MEET
-            return check_launch("ctc_lattice_meet");
-        }
-        dim3 grid(p.B, 2);
+    dim3 grid(p.B, 2);
 #define LASR_LATTICE(R, PFW, NW) \
     ctc_lattice_warp_kernel<R, PFW, NW><<<grid, 32 * NW, 0, st>>>(p.lp_ext, ab, be, p.targets, p.in_len, p.tgt_len, nll, tot, p.T, p.lmax)
-        if (W <= 32) LASR_LATTICE(1, 8, 1);
-        else if (W <= 64) LASR_LATTICE(2, 8, 1);
-        else if (W <= 128) LASR_LATTICE(2, 8, 2);
-        else if (W <= 256) LASR_LATTICE(2, 8, 4);
-        else if (W <= 512) LASR_LATTICE(2, 8, 8);
-        else LASR_LATTICE(4, 4, 8);
+    if (W <= 32) LASR_LATTICE(1, 8, 1);
+    else if (W <= 64) LASR_LATTICE(2, 8, 1);
+    else if (W <= 128) LASR_LATTICE(2, 8, 2);
+    else if (W <= 256) LASR_LATTICE(2, 8, 4);
+    else if (W <= 512) LASR_LATTICE(2, 8, 8);
+    else LASR_LATTICE(4, 4, 8);
 #undef LASR_LATTICE
-        rc = check_launch("ctc_lattice_warp");
-        if (rc) return rc;
-        ctc_scatter_ab_kernel<T><<<ceil_div(rows, 8), 256, 0, st>>>(ab, be, p.lp_ext, tot, p.grad, p.gst, p.gsb, p.targets, p.in_len,
-                                                                   p.tgt_len, p.T, p.B, p.lmax, p.blank, p.grad_scale, p.upstream);
-    }
+    rc = check_launch("ctc_lattice_warp");
+    if (rc) return rc;
+    ctc_scatter_ab_kernel<T><<<ceil_div(rows, 8), 256, 0, st>>>(ab, be, p.lp_ext, tot, p.grad, p.gst, p.gsb, p.targets, p.in_len,
+                                                               p.tgt_len, p.T, p.B, p.lmax, p.blank, p.grad_scale, p.upstream);
     return check_launch("ctc_scatter_ab");
 }
 
@@ -1038,8 +506,8 @@ extern "C" {
 
 size_t lasr_ctc_workspace_bytes(int T, int B, int lmax) {
     const size_t w = (size_t)(lmax < 1 ? 1 : lmax) + 1;
-    // alpha (float2) + beta (float2) + gathered lattice inputs (float) per (t, b, state pair); tot + two meeting flags per utterance
-    return (size_t)T * B * w * (sizeof(float) + 2 * sizeof(float2)) + (size_t)B * (sizeof(float) + 2 * sizeof(int)) + (size_t)T * B * sizeof(float) + 1024;
+    // alpha (float2) + beta (float2) + gathered lattice inputs (float) per (t, b, state pair); tot per utterance
+    return (size_t)T * B * w * (sizeof(float) + 2 * sizeof(float2)) + (size_t)B * sizeof(float) + 1024;
 }
 
 int lasr_ctc_fwdbwd(const void* logits, int dtype, int64_t st, int64_t sb, const int64_t* targets, const int64_t* in_len,
@@ -1061,12 +529,9 @@ int lasr_ctc_fwdbwd(const void* logits, int dtype, int64_t st, int64_t sb, const
     float2* be = reinterpret_cast<float2*>(base + (size_t)T * B * w * sizeof(float2));
     p.lp_ext = reinterpret_cast<float*>(base + 2 * (size_t)T * B * w * sizeof(float2));
     float* tot = reinterpret_cast<float*>(base + (size_t)T * B * w * (2 * sizeof(float2) + sizeof(float)));
-    int* flags = reinterpret_cast<int*>(tot + B);  // meeting flags of the alpha / beta CTA pairs
-    p.lse = reinterpret_cast<float*>(flags + 2 * B);
-    p.b0 = 0; p.nb = B; p.occ = nullptr;
     p.T = T; p.B = B; p.V = V; p.lmax = lmax; p.blank = blank; p.grad_scale = grad_scale; p.upstream = upstream;
-    if (dtype == LASR_F32) return ctc_launch<float>(p, ab, be, tot, flags, nll, (cudaStream_t)stream);
-    if (dtype == LASR_BF16) return ctc_launch<bf16>(p, ab, be, tot, flags, nll, (cudaStream_t)stream);
+    if (dtype == LASR_F32) return ctc_launch<float>(p, ab, be, tot, nll, (cudaStream_t)stream);
+    if (dtype == LASR_BF16) return ctc_launch<bf16>(p, ab, be, tot, nll, (cudaStream_t)stream);
     set_error("ctc: unsupported dtype %d", dtype);
     return LASR_ERR_UNSUPPORTED;
 }

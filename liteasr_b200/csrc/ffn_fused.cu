@@ -69,7 +69,6 @@ struct Params {
     int M, D, F;
     int tiles;
     long long* trace;  // developer aid: 8 clock64 stamps per chunk of CTA 0's first tile (lasr_ffn_bwd_set_trace)
-    int dbg;  // developer experiments (LASR_FFN_DBG bit mask): 16 no chunk rotation, 32 wait for every first MMA chain (trace)
 };
 
 __device__ __forceinline__ uint4 ldg_pred_u4(const void* p, bool pred) {
@@ -166,7 +165,7 @@ ffn_bwd_kernel(const __grid_constant__ CUtensorMap m_w2, const __grid_constant__
     // Every CTA walks the f chunks in its own rotation (chunk jj of a tile is column block (jj + rot) % NC): with a common
     // order all 148 SMs would ask the L2 for the SAME 64 KB of weights at the same moment (one line -> one slice -> 148 requests
     // in a row); rotated, the requests of a moment spread over the whole 2 MB of W1 and W2
-    const int rot = (p.dbg & 16) ? 0 : (int)((blockIdx.x * 7u) % (unsigned)NC);
+    const int rot = (int)((blockIdx.x * 7u) % (unsigned)NC);
 
     if (warp == 0 && lane == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&m_w2) : "memory");
@@ -237,11 +236,6 @@ ffn_bwd_kernel(const __grid_constant__ CUtensorMap m_w2, const __grid_constant__
                         tc_mma_bf16_ts(td, ta + kb * 32 + kk * 8, db + (uint64_t)((kb * 8192 + kk * 2048) >> 4), id1, (kb | kk) ? 1u : 0u);
                 tc_commit(bars + W2_EMPTY + ws1);
                 tc_commit(bars + ACC1_FULL + a);
-                if (p.dbg & 32) {  // developer experiment: how long does the first MMA chain really take (issue -> barrier completion)?
-                    const long long ti = clock64();
-                    mbar_wait(bars + ACC1_FULL + a, aph);
-                    if (p.trace && blockIdx.x == 0 && c1 < 32) { p.trace[c1 * 8 + 0] = ti; p.trace[c1 * 8 + 1] = clock64(); }
-                }
                 ++c1;
                 if (++ws1 == W2S) { ws1 = 0; wp1 ^= 1u; }
             };
@@ -812,7 +806,6 @@ int lasr_ffn_bwd(const void* dy, int64_t lddy, const void* g, int64_t ldg, const
     p.colsum = colsum; p.alpha = alpha;
     p.M = M; p.D = d; p.F = f;
     p.tiles = (M + ffn::TM - 1) / ffn::TM;
-    { const char* e = getenv("LASR_FFN_DBG"); p.dbg = e ? atoi(e) : 0; }
     p.trace = g_ffn_trace;
     static int sms = 0;
     if (!sms) {

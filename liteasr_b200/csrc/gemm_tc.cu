@@ -38,15 +38,14 @@ constexpr int A_BYTES = BM * BK * 2;
 constexpr int MAX_STAGES = 8;
 constexpr int ACC_COLS = 256;  // TMEM columns per accumulator buffer (2 buffers = the whole 512-column TMEM)
 
+constexpr int CW = 32;  // epilogue chunk width in fp32 columns (one tcgen05.ld 32x32b.x32 per chunk)
+
 // shared-memory carve-up (offsets from the 1024-aligned base): epilogue staging (EPI_WARPS x 32 rows x CW fp32 columns),
-// mbarriers + TMEM slot, then the operand ring.  CW = 32 in the streaming kernels; the B-stationary kernels stage 16 columns
-// at a time (32 KB instead of 64 KB) to make room for a resident weight tile.
-constexpr int sm_bars(int cw) { return EPI_WARPS * 32 * cw * 4; }
-constexpr int sm_ring(int cw) { return sm_bars(cw) + 1024; }
+// mbarriers + TMEM slot, then the operand ring.
+constexpr int SM_BARS = EPI_WARPS * 32 * CW * 4;
+constexpr int SM_RING = SM_BARS + 1024;
 constexpr int SM_MAX_DYNAMIC = 232448;   // 227 KB
-constexpr int sm_ring_budget(int cw) { return SM_MAX_DYNAMIC - sm_ring(cw) - 1024 /*alignment slack*/; }
-constexpr int SM_RING = sm_ring(32);
-constexpr int SM_RING_BUDGET = sm_ring_budget(32);
+constexpr int SM_RING_BUDGET = SM_MAX_DYNAMIC - SM_RING - 1024 /*alignment slack*/;
 
 struct TcParams {
     void* c;
@@ -76,10 +75,6 @@ struct TcParams {
     // implicit-GEMM 3x3 stride-2 convolution over parity planes (see conv2_tc_dispatch): only the TMA producer changes
     int tma_epi;       // epilogue stores through TMA (row-per-thread math, swizzled staging, bulk tensor store / reduce-add)
     int c_b1, c_b2;    // 1 if C really advances along that batch level (TMA store coordinates)
-    int b_stationary;  // K <= 256 GEMMs: every CTA keeps ONE N tile of B resident in shared memory and streams A tiles only
-    int bsta_bytes;    // size of that resident tile
-    int dual;          // recompute mode: a second accumulator A2.B2^T (K-major operands) at TMEM columns [128, 128 + bn) of the buffer
-    const float* bias2;  // bias of the recomputed Linear
     int conv_mode;     // 0 plain GEMM | 1 forward | 2 input gradient (one parity class) | 3 weight gradient
     int conv_kbt;      // K blocks per tap (= channels / 64)
     int conv_d;        // channels
@@ -179,15 +174,13 @@ __device__ __forceinline__ void store4(CT* dst, const float4& f) {
 
 // Epilogue modes: the column phase is specialised so that its inner loop carries no run-time flag tests.
 enum { EPI_PLAIN = 0, EPI_RELU = 1, EPI_SWISH = 2, EPI_RES = 3, EPI_ACC = 4, EPI_GENERIC = 5, EPI_DSWISH = 6, EPI_DRELU = 7,
-       EPI_DUAL_DSWISH = 8, EPI_DUAL_DRELU = 9,  // DUAL: act'(.) of a pre-activation recomputed into a second accumulator
-       EPI_DMUL = 10 };                          // C = alpha * acc * saved factor (the forward pass saved act'() itself: aux_deriv)
+       EPI_DMUL = 10 };  // C = alpha * acc * saved factor (the forward pass saved act'() itself: aux_deriv)
 
-// CW = staged chunk width in fp32 columns (32, or 16 in the B-stationary kernels).  The staging buffer holds 32 rows x CW
-// columns; a row is PIECES = CW/4 16-byte pieces, XOR-swizzled so that both the row-per-thread writes and the row-contiguous
-// reads are bank-conflict free: piece j of row r lives at r*128 + ((j ^ (r & 7)) << 4) for CW = 32 and at
-// r*64 + ((j ^ ((r >> 1) & 3)) << 4) for CW = 16.  In the column phase PIECES lanes own one row segment and a warp covers
-// RGRP = 32 / PIECES rows per instruction.
-template <typename CT, int MODE, int CW, bool DROP>
+// The staging buffer holds 32 rows x CW columns; a row is PIECES = CW/4 16-byte pieces, XOR-swizzled so that both the
+// row-per-thread writes and the row-contiguous reads are bank-conflict free: piece j of row r lives at
+// r*128 + ((j ^ (r & 7)) << 4).  In the column phase PIECES lanes own one row segment and a warp covers RGRP = 32 / PIECES
+// rows per instruction.
+template <typename CT, int MODE, bool DROP>
 __device__ __forceinline__ void epilogue_unit(const TcParams& p, const Unit& w, uint32_t tmem_acc, uint8_t* stage, int q, int part,
                                               int lane) {
     constexpr int PIECES = CW / 4, RGRP = 32 / PIECES, ITERS = 32 / RGRP, ROWB = CW * 4;
@@ -205,10 +198,10 @@ __device__ __forceinline__ void epilogue_unit(const TcParams& p, const Unit& w, 
     float* csbase = p.colsum ? p.colsum + (long)w.b1 * p.cs1 + (long)w.b2 * p.cs2 : nullptr;
     constexpr bool DACT = (MODE == EPI_DSWISH || MODE == EPI_DRELU || MODE == EPI_DMUL);
     uint8_t* wr = stage + lane * ROWB;
-    const int wx = (CW == 32) ? ((lane & 7) << 4) : (((lane >> 1) & 3) << 4);
-    // CW = 32: rows 4i + rsub alternate between two swizzle phases (i even / odd); CW = 16: rows 8i + rsub share one
-    const uint8_t* rd0 = (CW == 32) ? stage + rsub * 128 + ((chunk ^ rsub) << 4) : stage + rsub * 64 + ((chunk ^ ((rsub >> 1) & 3)) << 4);
-    const uint8_t* rd1 = (CW == 32) ? stage + rsub * 128 + (((chunk ^ rsub) ^ 4) << 4) : rd0;
+    const int wx = (lane & 7) << 4;
+    // rows 4i + rsub alternate between two swizzle phases (i even / odd)
+    const uint8_t* rd0 = stage + rsub * 128 + ((chunk ^ rsub) << 4);
+    const uint8_t* rd1 = stage + rsub * 128 + (((chunk ^ rsub) ^ 4) << 4);
     const bool drop_on = DROP && p.drop.thr != 0;  // warp-uniform; DROP = false kernels carry none of the dropout code
     DropKey dk = {};
     if (drop_on) dk = drop_key(p.drop);
@@ -246,22 +239,7 @@ __device__ __forceinline__ void epilogue_unit(const TcParams& p, const Unit& w, 
         // row phase: thread = accumulator row
         {
             float v[CW];
-            if constexpr (CW == 32) tc_ld32(taddr + (uint32_t)cc, v);
-            else tc_ld16(taddr + (uint32_t)cc, v);
-            if constexpr (MODE == EPI_DUAL_DSWISH || MODE == EPI_DUAL_DRELU) {
-                // C = alpha * acc * act'(acc2 + bias2): the recomputed pre-activation sits 128 TMEM columns further; its bias is
-                // the same 32 floats for every lane (warp-uniform loads)
-                float pre[32];
-                tc_ld32(taddr + 128u + (uint32_t)cc, pre);
-                const int c0 = w.n0 + cc;
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const float b = (p.bias2 && c0 + j < p.n) ? __ldg(p.bias2 + c0 + j) : 0.f;
-                    const float x = pre[j] + b;
-                    if constexpr (MODE == EPI_DUAL_DSWISH) v[j] *= dswish_scaled(x, 0.5f * alpha);
-                    else v[j] = x > 0.f ? alpha * v[j] : 0.f;
-                }
-            }
+            tc_ld32(taddr + (uint32_t)cc, v);
             __syncwarp();  // the previous chunk's column phase has finished reading the staging buffer
 #pragma unroll
             for (int j = 0; j < PIECES; ++j)
@@ -328,9 +306,6 @@ __device__ __forceinline__ void epilogue_unit(const TcParams& p, const Unit& w, 
                         }
                         store4<CT>(crow, f);
                         cs.x += f.x; cs.y += f.y; cs.z += f.z; cs.w += f.w;
-                    } else if constexpr (MODE == EPI_DUAL_DSWISH || MODE == EPI_DUAL_DRELU) {
-                        store4<CT>(crow, f);  // finished in the row phase
-                        cs.x += f.x; cs.y += f.y; cs.z += f.z; cs.w += f.w;
                     } else if constexpr (MODE == EPI_RES) {
                         if (drop_on) {  // res + keep * scale * (alpha * acc + alpha * bias)
                             f.x = fmaf(fmaf(f.x, alpha, ba.x), kx, r4[i].x); f.y = fmaf(fmaf(f.y, alpha, ba.y), ky, r4[i].y);
@@ -375,7 +350,7 @@ __device__ __forceinline__ void epilogue_unit(const TcParams& p, const Unit& w, 
                 }
                 off += rstride;
             }
-            if constexpr (MODE == EPI_PLAIN || DACT || MODE == EPI_DUAL_DSWISH || MODE == EPI_DUAL_DRELU) {
+            if constexpr (MODE == EPI_PLAIN || DACT) {
                 if (csbase) {  // warp-uniform: fold the row groups (lanes with the same piece), then one vector red per 4 columns
 #pragma unroll
                     for (int o = PIECES; o < 32; o <<= 1) {
@@ -390,8 +365,7 @@ __device__ __forceinline__ void epilogue_unit(const TcParams& p, const Unit& w, 
             for (int i = 0; i < ITERS; ++i) {
                 const int row = RGRP * i + rsub;
                 const int grow = row_base + row;
-                const int swz = (CW == 32) ? (row & 7) : ((row >> 1) & 3);
-                const float4 f4 = *reinterpret_cast<const float4*>(stage + row * ROWB + ((chunk ^ swz) << 4));
+                const float4 f4 = *reinterpret_cast<const float4*>(stage + row * ROWB + ((chunk ^ (row & 7)) << 4));
                 const float f[4] = {f4.x + b4.x, f4.y + b4.y, f4.z + b4.z, f4.w + b4.w};
                 if (grow >= p.m) continue;
 #pragma unroll 1
@@ -424,39 +398,22 @@ __device__ __forceinline__ void epilogue_unit(const TcParams& p, const Unit& w, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// TMA-store epilogue (default whenever C / aux / bias / res / dact meet the 16-byte alignment rules).
+// TMA-store epilogue of the PLAIN / RELU / SWISH / ACC modes without colsum (whenever C / aux / bias meet the 16-byte
+// alignment rules: setup_tma_epilogue).
 // The accumulator row a thread reads from TMEM (32 consecutive columns) is finished IN PLACE -- bias as warp-uniform float4
-// loads, residual / saved activation as row-contiguous 16-byte loads -- converted, written to a swizzled 32 x 32 staging box
+// loads -- converted, written to a swizzled 32 x 32 staging box
 // (SWIZZLE_64B for bf16, SWIZZLE_128B for fp32: the same XOR patterns that make the row-per-thread 16-byte stores conflict
 // free) and handed to ONE bulk tensor store (or reduce-add) per box.  Compared with the register -> smem -> register ->
 // global column phase this removes every LDS, STG, 64-bit address computation and edge predicate from the 16 epilogue warps
 // (the FFN fc1 + Swish kernel was issue-bound: 59 % issue-slot utilisation, 58 % LSU wavefronts, tensor pipe 21 %); the TMA
 // unit clips rows >= M and columns >= N, so ragged shapes (N = 299, V = 4233) take the same path.
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float col_sums_32(float (&v)[32], int lane) {
-    // transpose-reduce: after the five exchange stages lane c holds the sum over the 32 lanes (rows) of column c
-#pragma unroll
-    for (int s = 16; s >= 1; s >>= 1) {
-        const bool up = (lane & s) != 0;
-#pragma unroll
-        for (int i = 0; i < s; ++i) {
-            const float send = up ? v[i] : v[i + s];
-            const float keep = up ? v[i + s] : v[i];
-            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, s);
-        }
-    }
-    return v[0];
-}
-
 template <typename CT, int MODE, bool DROP>
 __device__ __forceinline__ void epilogue_unit_tma(const TcParams& p, const Unit& w, uint32_t tmem_acc, uint8_t* stage, int q, int part,
                                                   int lane, const CUtensorMap* mc, const CUtensorMap* mx, int& buf) {
     constexpr bool BF = sizeof(CT) == 2;
-    constexpr bool DACT = (MODE == EPI_DSWISH || MODE == EPI_DRELU || MODE == EPI_DMUL);
-    const long boff = (long)w.b1 * p.sc1 + (long)w.b2 * p.sc2;
     const int col_limit = min(p.n_store, w.n0 + p.bn);
     const int row0 = w.m0 + q * 32, row = row0 + lane;
-    const bool row_ok = row < p.m;
     const uint32_t taddr = tmem_acc + ((uint32_t)(q * 32) << 16);
     const float alpha = p.alpha;
     const bool has_aux = p.aux != nullptr;   // warp-uniform
@@ -474,34 +431,6 @@ __device__ __forceinline__ void epilogue_unit_tma(const TcParams& p, const Unit&
         // its wait: they depend on nothing the accumulator holds, so the Philox latency chain hides behind the load's
         // (two calls: packed 0xffff / 0 lane masks, mk[t] = columns col0 + 2t and col0 + 2t + 1 -- philox.cuh)
         uint32_t mk[16];
-        // row-wise global operands first (in flight while TMEM is read)
-        float4 r4[MODE == EPI_RES ? 8 : 1];
-        uint4 s4[DACT ? 4 : 1];
-        if constexpr (MODE == EPI_RES) {
-            const float* rp = p.res + boff + (long)row * p.ldres + col0;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) r4[j] = ldg_pred_f4(rp + 4 * j, row_ok && col0 + 4 * j + 3 < col_limit);
-            if (!full && row_ok && (col_limit & 3)) {  // ragged edge inside a float4: element-wise for that quad
-                const int j = (col_limit - col0) >> 2;
-                float t[4] = {0.f, 0.f, 0.f, 0.f};
-                for (int e = 0; e < (col_limit & 3); ++e) t[e] = rp[4 * j + e];
-                r4[j < 8 ? j : 7] = make_float4(t[0], t[1], t[2], t[3]);
-            }
-        }
-        if constexpr (DACT) {
-            const bf16* sp = p.dact + boff + (long)row * p.lddact + col0;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                s4[j] = make_uint4(0u, 0u, 0u, 0u);
-                if (row_ok && col0 + 8 * j + 7 < col_limit) s4[j] = *reinterpret_cast<const uint4*>(sp + 8 * j);
-                else if (row_ok && col0 + 8 * j < col_limit) {
-                    bf16 t[8];
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) t[e] = (col0 + 8 * j + e < col_limit) ? sp[8 * j + e] : __float2bfloat16_rn(0.f);
-                    s4[j] = *reinterpret_cast<const uint4*>(t);
-                }
-            }
-        }
         float v[32];
         if constexpr (DROP) {
             tc_ld32_issue(taddr + (uint32_t)cc, v);
@@ -520,25 +449,6 @@ __device__ __forceinline__ void epilogue_unit_tma(const TcParams& p, const Unit&
         if constexpr (MODE == EPI_ACC) {
 #pragma unroll
             for (int j = 0; j < 32; ++j) v[j] *= alpha;
-        } else if constexpr (DACT) {
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&s4[j]);
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    const float a0 = __low2float(h[e]), a1 = __high2float(h[e]);
-                    if constexpr (MODE == EPI_DSWISH) {
-                        v[8 * j + 2 * e] *= dswish_scaled(a0, 0.5f * alpha);
-                        v[8 * j + 2 * e + 1] *= dswish_scaled(a1, 0.5f * alpha);
-                    } else if constexpr (MODE == EPI_DMUL) {
-                        v[8 * j + 2 * e] *= alpha * a0;
-                        v[8 * j + 2 * e + 1] *= alpha * a1;
-                    } else {
-                        v[8 * j + 2 * e] = a0 > 0.f ? alpha * v[8 * j + 2 * e] : 0.f;
-                        v[8 * j + 2 * e + 1] = a1 > 0.f ? alpha * v[8 * j + 2 * e + 1] : 0.f;
-                    }
-                }
-            }
         } else {
             // bias: the same 32 floats for every lane (warp-uniform 16-byte loads, L1-resident), consumed quad by quad
             const bool has_bias = p.bias != nullptr;
@@ -556,14 +466,13 @@ __device__ __forceinline__ void epilogue_unit_tma(const TcParams& p, const Unit&
                         b.w = c + 3 < col_limit ? __ldg(p.bias + c + 3) : 0.f;
                     }
                 }
-                if constexpr (MODE == EPI_PLAIN || MODE == EPI_RES) {
+                if constexpr (MODE == EPI_PLAIN) {
                     v[4 * j] = fmaf(v[4 * j], alpha_s, alpha_s * b.x); v[4 * j + 1] = fmaf(v[4 * j + 1], alpha_s, alpha_s * b.y);
                     v[4 * j + 2] = fmaf(v[4 * j + 2], alpha_s, alpha_s * b.z); v[4 * j + 3] = fmaf(v[4 * j + 3], alpha_s, alpha_s * b.w);
-                    if (drop_on) {  // dropped -> +0 (the residual is added after the mask)
+                    if (drop_on) {  // dropped -> +0
                         v[4 * j] = drop_and(v[4 * j], drop_mask_lo(mk[2 * j])); v[4 * j + 1] = drop_and(v[4 * j + 1], drop_mask_hi(mk[2 * j]));
                         v[4 * j + 2] = drop_and(v[4 * j + 2], drop_mask_lo(mk[2 * j + 1])); v[4 * j + 3] = drop_and(v[4 * j + 3], drop_mask_hi(mk[2 * j + 1]));
                     }
-                    if constexpr (MODE == EPI_RES) { v[4 * j] += r4[j].x; v[4 * j + 1] += r4[j].y; v[4 * j + 2] += r4[j].z; v[4 * j + 3] += r4[j].w; }
                 } else {  // EPI_RELU / EPI_SWISH: pre-activation = acc + bias
                     v[4 * j] += b.x; v[4 * j + 1] += b.y; v[4 * j + 2] += b.z; v[4 * j + 3] += b.w;
                 }
@@ -651,85 +560,33 @@ __device__ __forceinline__ void epilogue_unit_tma(const TcParams& p, const Unit&
             bulk_commit();
         }
         if (dbl) buf ^= 1;
-        // ---- bias gradient of the producing Linear: column sums of what was just written (rows >= M excluded)
-        if constexpr (MODE == EPI_PLAIN || DACT) {
-            if (p.colsum) {  // warp-uniform
-#pragma unroll
-                for (int j = 0; j < 32; ++j) v[j] = row_ok ? v[j] : 0.f;
-                const float cs = col_sums_32(v, lane);
-                if (col0 + lane < col_limit) atomicAdd(p.colsum + (long)w.b1 * p.cs1 + (long)w.b2 * p.cs2 + col0 + lane, cs);
-            }
-        }
     }
 }
 
-// Work-unit walk shared by the three roles.  Streaming kernels: units blockIdx.x, + gridDim.x, ... of the (batch, split, m, n)
-// list.  B-stationary kernels: the CTA owns N tile blockIdx.x % tiles_n for its whole life and takes every
-// (gridDim.x / tiles_n)-th M tile (gridDim.x is a multiple of tiles_n).
-template <bool BS>
-struct Walk {
-    int cur, step, nt;
-    __device__ __forceinline__ explicit Walk(const TcParams& p) {
-        if (BS) {
-            nt = blockIdx.x % p.tiles_n;
-            cur = blockIdx.x / p.tiles_n;
-            step = gridDim.x / p.tiles_n;
-        } else {
-            nt = 0;
-            cur = blockIdx.x;
-            step = gridDim.x;
-        }
-    }
-    __device__ __forceinline__ bool next(const TcParams& p, Unit& w) {
-        if (BS) {
-            if (cur >= p.tiles_m) return false;
-            w.m0 = cur * BM; w.n0 = nt * p.bn; w.b1 = 0; w.b2 = 0; w.kb_begin = 0; w.num_kb = (p.k + BK - 1) / BK;
-            cur += step;
-            return true;
-        }
-        while (cur < p.total_units) {
-            w = decode_unit(p, cur);
-            cur += step;
-            if (w.num_kb > 0) return true;  // <= 0 only for trailing splits: skipped by every role
-        }
-        return false;
-    }
-};
-
 // MODE / C_F32 specialise the epilogue warps (one kernel per epilogue keeps the instruction footprint and the register
 // allocation of each variant minimal); operand majors are run-time values: they only steer the two single-thread roles.
-// BS (B-stationary, K <= 256): the weight tile of the CTA's N tile is loaded ONCE into shared memory and only 16 KB A slabs
-// stream through the ring -- a K = 256 GEMM otherwise re-fetches its 128 KB B tile for every 128 x 256 output tile and runs
-// at the L2 -> SM bandwidth, not at the tensor or HBM roofline.
-template <int MODE, bool C_F32, bool BS, bool DROP>
+// The three roles walk the same work units: blockIdx.x, + gridDim.x, ... of the (batch, split, m, n) list; a unit with no
+// K blocks (a trailing split) is skipped by every role.
+template <int MODE, bool C_F32, bool DROP>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
-               const __grid_constant__ CUtensorMap tma_c, const __grid_constant__ CUtensorMap tma_x,
-               const __grid_constant__ CUtensorMap tma_a2, const __grid_constant__ CUtensorMap tma_b2, const TcParams p) {
-    constexpr int CW = BS ? 16 : 32;
+               const __grid_constant__ CUtensorMap tma_c, const __grid_constant__ CUtensorMap tma_x, const TcParams p) {
     const bool A_MN = p.a_mn != 0, B_MN = p.b_mn != 0;
     extern __shared__ uint8_t smem_raw[];
     // align inside the shared window (keeps the address space visible to the compiler: LDS/STS, not generic LD/ST)
     uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + sm_bars(CW));
+    uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + SM_BARS);
     uint64_t* empty_bar = full_bar + MAX_STAGES;
     uint64_t* acc_full = empty_bar + MAX_STAGES;
     uint64_t* acc_empty = acc_full + 2;
-    uint64_t* b_full = acc_empty + 2;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(b_full + 1);
-    uint8_t* bsta = smem + sm_ring(CW);                         // resident B k-blocks (BS only)
-    uint8_t* ring = bsta + (BS ? p.bsta_bytes : 0);
-    const int b_kb_bytes = p.bn * BK * 2;
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
+    uint8_t* ring = smem + SM_RING;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
     if (warp == 0 && lane == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_a) : "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_b) : "memory");
-        if (p.dual) {
-            asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_a2) : "memory");
-            asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_b2) : "memory");
-        }
         if (p.tma_epi) {
             asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_c) : "memory");
             if (p.aux) asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_x) : "memory");
@@ -744,7 +601,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             mbar_init(acc_full + s, 1);
             mbar_init(acc_empty + s, EPI_WARPS);  // one arrival per epilogue warp
         }
-        mbar_init(b_full, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 2) {
@@ -766,21 +622,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
         if (lane == 0) {
             int s = 0;
             uint32_t ph = 0;
-            Walk<BS> walk(p);
-            Unit w;
-            if (BS && walk.cur < p.tiles_m) {  // the CTA's weight tile, once
-                const int total_kb = (p.k + BK - 1) / BK, n0 = walk.nt * p.bn;
-                mbar_arrive_expect_tx(b_full, (uint32_t)(total_kb * b_kb_bytes));
-                for (int kb = 0; kb < total_kb; ++kb) {
-                    uint8_t* sb = bsta + kb * b_kb_bytes;
-                    if (!B_MN) {
-                        tma_load_4d(sb, &tma_b, b_full, kb * BK, n0, 0, 0);
-                    } else {
-                        for (int j = 0; j < p.bn / 64; ++j) tma_load_4d(sb + j * 8192, &tma_b, b_full, n0 + 64 * j, kb * BK, 0, 0);
-                    }
-                }
-            }
-            while (walk.next(p, w)) {
+            for (int u = blockIdx.x; u < p.total_units; u += gridDim.x) {
+                const Unit w = decode_unit(p, u);
+                if (w.num_kb <= 0) continue;
                 const int ab1 = w.b1 * p.a_b1, ab2 = w.b2 * p.a_b2, bb1 = w.b1 * p.b_b1, bb2 = w.b2 * p.b_b2;
                 for (int i = 0; i < w.num_kb; ++i) {
                     mbar_wait(empty_bar + s, ph ^ 1);
@@ -788,7 +632,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                     uint8_t* sa = ring + s * p.stage_bytes;
                     uint8_t* sb = sa + A_BYTES;
                     const int k0 = (w.kb_begin + i) * BK;
-                    if (!BS && p.conv_mode != 0) {
+                    if (p.conv_mode != 0) {
                         const int kb = w.kb_begin + i;
                         if (p.conv_mode == 1) {         // A = h1 planes (rows shifted per tap), B = (co, tap*ci) weight, both K-major
                             const int tp = kb / p.conv_kbt, kc = kb - tp * p.conv_kbt;
@@ -815,18 +659,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                             for (int j = 0; j < BM / 64; ++j)  // box {64 m, 64 k}
                                 tma_load_4d(sa + j * 8192, &tma_a, full_bar + s, w.m0 + 64 * j, k0, ab2, ab1);
                         }
-                        if (!BS) {
-                            if (!B_MN) {
-                                tma_load_4d(sb, &tma_b, full_bar + s, k0, w.n0, bb2, bb1);  // box {64 k, BN n}
-                            } else {
-                                for (int j = 0; j < p.bn / 64; ++j)
-                                    tma_load_4d(sb + j * 8192, &tma_b, full_bar + s, w.n0 + 64 * j, k0, bb2, bb1);
-                            }
-                            if (p.dual) {  // the recomputed Linear's input and weight slabs, both K-major, behind A and B in the stage
-                                uint8_t* sa2 = sb + b_kb_bytes;
-                                tma_load_4d(sa2, &tma_a2, full_bar + s, k0, w.m0, 0, 0);
-                                tma_load_4d(sa2 + A_BYTES, &tma_b2, full_bar + s, k0, w.n0, 0, 0);
-                            }
+                        if (!B_MN) {
+                            tma_load_4d(sb, &tma_b, full_bar + s, k0, w.n0, bb2, bb1);  // box {64 k, BN n}
+                        } else {
+                            for (int j = 0; j < p.bn / 64; ++j)
+                                tma_load_4d(sb + j * 8192, &tma_b, full_bar + s, w.n0 + 64 * j, k0, bb2, bb1);
                         }
                     }
                     if (++s == p.stages) { s = 0; ph ^= 1; }
@@ -840,13 +677,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                                    ((uint32_t)(p.bn >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
             int s = 0, as = 0;
             uint32_t ph = 0, aph = 0;
-            Walk<BS> walk(p);
-            Unit w;
-            if (BS && walk.cur < p.tiles_m) {
-                mbar_wait(b_full, 0);
-                tc_fence_after();
-            }
-            while (walk.next(p, w)) {
+            for (int u = blockIdx.x; u < p.total_units; u += gridDim.x) {
+                const Unit w = decode_unit(p, u);
+                if (w.num_kb <= 0) continue;
                 mbar_wait(acc_empty + as, aph ^ 1);  // the epilogue has drained this accumulator buffer
                 tc_fence_after();
                 const uint32_t tmem_d = tmem_base + (uint32_t)(as * ACC_COLS);
@@ -854,7 +687,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                     mbar_wait(full_bar + s, ph);
                     tc_fence_after();
                     const uint32_t sa = smem_u32(ring + s * p.stage_bytes);
-                    const uint32_t sb = BS ? smem_u32(bsta + i * b_kb_bytes) : sa + A_BYTES;
+                    const uint32_t sb = sa + A_BYTES;
 #pragma unroll
                     for (int kk = 0; kk < BK / UMMA_K; ++kk) {
                         // K-major: +32 B per UMMA_K inside the 128 B swizzle row; SBO = 8 rows * 128 B.
@@ -862,11 +695,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                         const uint64_t da = A_MN ? umma_desc(sa + kk * 2048, 8192, 1024) : umma_desc(sa + kk * 32, 16, 1024);
                         const uint64_t db = B_MN ? umma_desc(sb + kk * 2048, 8192, 1024) : umma_desc(sb + kk * 32, 16, 1024);
                         tc_mma_bf16(tmem_d, da, db, idesc, (i > 0 || kk > 0) ? 1u : 0u);
-                        if (!BS && p.dual) {  // second accumulator (bn <= 128): A2.B2^T, K-major operands
-                            const uint32_t sa2 = sb + (uint32_t)b_kb_bytes;
-                            tc_mma_bf16(tmem_d + 128u, umma_desc(sa2 + kk * 32, 16, 1024), umma_desc(sa2 + A_BYTES + kk * 32, 16, 1024),
-                                        idesc & ~((1u << 15) | (1u << 16)), (i > 0 || kk > 0) ? 1u : 0u);
-                        }
                     }
                     tc_commit(empty_bar + s);  // frees the smem slot once these MMAs retire
                     if (++s == p.stages) { s = 0; ph ^= 1; }
@@ -882,16 +710,16 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
         uint8_t* stage = smem + ew * (32 * CW * 4);
         int as = 0, sbuf = 0;
         uint32_t aph = 0;
-        Walk<BS> walk(p);
-        Unit w;
         typedef typename std::conditional<C_F32, float, bf16>::type CT;
-        constexpr bool TMA_OK = !BS && MODE != EPI_GENERIC && MODE != EPI_DUAL_DSWISH && MODE != EPI_DUAL_DRELU;
+        constexpr bool TMA_OK = MODE == EPI_PLAIN || MODE == EPI_RELU || MODE == EPI_SWISH || MODE == EPI_ACC;  // setup_tma_epilogue
         const bool tma_epi = TMA_OK && p.tma_epi != 0;
         // N tiles whose 32-column chunks do not divide evenly among the four warps of a lane quarter (BN = 160: 5 chunks) leave one
         // warp with twice the work of the others in EVERY unit; rotating the chunk -> warp assignment from unit to unit spreads it
         // (the two accumulator buffers let a warp run one unit ahead of the slowest one)
         int urot = 0;
-        while (walk.next(p, w)) {
+        for (int u = blockIdx.x; u < p.total_units; u += gridDim.x) {
+            const Unit w = decode_unit(p, u);
+            if (w.num_kb <= 0) continue;
             mbar_wait(acc_full + as, aph);  // (sleeping between polls, 32-300 ns, changes nothing: the spin is not what limits the epilogue)
             tc_fence_after();
             const uint32_t tmem_acc = tmem_base + (uint32_t)(as * ACC_COLS);
@@ -899,9 +727,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             urot += p.epi_rot;
             if constexpr (TMA_OK) {
                 if (tma_epi) epilogue_unit_tma<CT, MODE, DROP>(p, w, tmem_acc, stage, q, part_u, lane, &tma_c, &tma_x, sbuf);
-                else epilogue_unit<CT, MODE, CW, DROP>(p, w, tmem_acc, stage, q, part_u, lane);
+                else epilogue_unit<CT, MODE, DROP>(p, w, tmem_acc, stage, q, part_u, lane);
             } else {
-                epilogue_unit<CT, MODE, CW, DROP>(p, w, tmem_acc, stage, q, part_u, lane);
+                epilogue_unit<CT, MODE, DROP>(p, w, tmem_acc, stage, q, part_u, lane);
             }
             tc_fence_before();
             __syncwarp();
@@ -999,21 +827,15 @@ static void setup_tma_epilogue(TcParams& p, CUtensorMap* mc, CUtensorMap* mx, in
     p.tma_epi = 0;
     p.c_b1 = (p.sc1 != 0 && nb1 > 1);
     p.c_b2 = (p.sc2 != 0 && nb2 > 1);
-    const char* env = getenv("LASR_GEMM_TMA_EPI");  // developer switch (read per call so that tests can toggle it)
-    if (env && atoi(env) == 0) return;
-    if (p.epi_mode == EPI_GENERIC || p.b_stationary || p.dual) return;
     // Row-per-thread math makes the residual / saved-activation reads 32-lines-per-instruction gathers and the column sums a
     // 31-shuffle transpose: measured slower than the column-phase epilogue (fc2 + residual 62 vs 51 us, dswish + colsum 128 vs
-    // 103 us at C2/B=126), so those modes keep it.  LASR_GEMM_TMA_EPI=2 forces the TMA path for every mode (tests).
-    const bool force = env && atoi(env) == 2;
-    if (!force && (p.epi_mode == EPI_RES || p.epi_mode == EPI_DSWISH || p.epi_mode == EPI_DRELU || p.epi_mode == EPI_DMUL || p.colsum)) return;
+    // 103 us at C2/B=126), so RES, the dact modes, colsum and GENERIC keep it (TMA_OK in gemm_tc_kernel).
+    if (!(p.epi_mode == EPI_PLAIN || p.epi_mode == EPI_RELU || p.epi_mode == EPI_SWISH || p.epi_mode == EPI_ACC) || p.colsum) return;
     // bulk tensor stores clip at 16-byte granularity (measured: tools/tma_clip_probe.py): a row whose last 16-byte chunk is
     // partial would get zeros written past column n_store, so ragged widths keep the register epilogue
     if (((long)p.n_store * (p.c_dtype == LASR_F32 ? 4 : 2)) & 15) return;
     if (p.aux && p.c_dtype == LASR_F32) return;                        // the staging set holds C + aux only for bf16
     if (p.bias && (reinterpret_cast<uintptr_t>(p.bias) & 15)) return;
-    if (p.res && ((reinterpret_cast<uintptr_t>(p.res) & 15) || (p.ldres & 3) || (p.sc1 & 3) || (p.sc2 & 3))) return;
-    if (p.dact && ((reinterpret_cast<uintptr_t>(p.dact) & 15) || (p.lddact & 7) || (p.sc1 & 7) || (p.sc2 & 7))) return;
     if (make_store_map(mc, p.c, p.c_dtype, p.n_store, p.m, p.ldc, nb2, p.sc2, nb1, p.sc1)) return;
     if (p.aux && make_store_map(mx, p.aux, p.c_dtype, p.n_store, p.m, p.ldc, nb2, p.sc2, nb1, p.sc1)) return;
     p.tma_epi = 1;
@@ -1032,13 +854,12 @@ static int pick_bn(int n, int gran) {
     return best;
 }
 
-typedef void (*TcKernel)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap,
-                         const TcParams);
+typedef void (*TcKernel)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const TcParams);
 
-template <int MODE, bool C_F32, bool BS, bool DROP = false>
+template <int MODE, bool C_F32, bool DROP = false>
 static TcKernel configured_kernel() {
     static bool configured = false;
-    TcKernel k = gemm_tc_kernel<MODE, C_F32, BS, DROP>;
+    TcKernel k = gemm_tc_kernel<MODE, C_F32, DROP>;
     if (!configured) {
         if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, SM_MAX_DYNAMIC) != cudaSuccess) return nullptr;
         configured = true;
@@ -1046,75 +867,66 @@ static TcKernel configured_kernel() {
     return k;
 }
 
-template <bool BS>
 static TcKernel pick_kernel(int mode, bool f32) {
     if (f32) {
         switch (mode) {
-            case EPI_PLAIN: return configured_kernel<EPI_PLAIN, true, BS>();
-            case EPI_RELU: return configured_kernel<EPI_RELU, true, BS>();
-            case EPI_SWISH: return configured_kernel<EPI_SWISH, true, BS>();
-            case EPI_RES: return configured_kernel<EPI_RES, true, BS>();
-            case EPI_ACC: return configured_kernel<EPI_ACC, true, BS>();
-            case EPI_DSWISH: return configured_kernel<EPI_DSWISH, true, BS>();
-            case EPI_DRELU: return configured_kernel<EPI_DRELU, true, BS>();
-            case EPI_DMUL: return configured_kernel<EPI_DMUL, true, BS>();
-            default: return configured_kernel<EPI_GENERIC, true, BS>();
+            case EPI_PLAIN: return configured_kernel<EPI_PLAIN, true>();
+            case EPI_RELU: return configured_kernel<EPI_RELU, true>();
+            case EPI_SWISH: return configured_kernel<EPI_SWISH, true>();
+            case EPI_RES: return configured_kernel<EPI_RES, true>();
+            case EPI_ACC: return configured_kernel<EPI_ACC, true>();
+            case EPI_DSWISH: return configured_kernel<EPI_DSWISH, true>();
+            case EPI_DRELU: return configured_kernel<EPI_DRELU, true>();
+            case EPI_DMUL: return configured_kernel<EPI_DMUL, true>();
+            default: return configured_kernel<EPI_GENERIC, true>();
         }
     }
     switch (mode) {
-        case EPI_PLAIN: return configured_kernel<EPI_PLAIN, false, BS>();
-        case EPI_RELU: return configured_kernel<EPI_RELU, false, BS>();
-        case EPI_SWISH: return configured_kernel<EPI_SWISH, false, BS>();
-        case EPI_DSWISH: return configured_kernel<EPI_DSWISH, false, BS>();
-        case EPI_DRELU: return configured_kernel<EPI_DRELU, false, BS>();
-        case EPI_DMUL: return configured_kernel<EPI_DMUL, false, BS>();
-        case EPI_DUAL_DSWISH: return BS ? nullptr : configured_kernel<EPI_DUAL_DSWISH, false, false>();
-        case EPI_DUAL_DRELU: return BS ? nullptr : configured_kernel<EPI_DUAL_DRELU, false, false>();
-        default: return configured_kernel<EPI_GENERIC, false, BS>();
+        case EPI_PLAIN: return configured_kernel<EPI_PLAIN, false>();
+        case EPI_RELU: return configured_kernel<EPI_RELU, false>();
+        case EPI_SWISH: return configured_kernel<EPI_SWISH, false>();
+        case EPI_DSWISH: return configured_kernel<EPI_DSWISH, false>();
+        case EPI_DRELU: return configured_kernel<EPI_DRELU, false>();
+        case EPI_DMUL: return configured_kernel<EPI_DMUL, false>();
+        default: return configured_kernel<EPI_GENERIC, false>();
     }
 }
 
-// dropout variants (streaming kernels only): separate instantiations, so that the p = 0 kernels are the round-1 kernels
+// dropout variants: separate instantiations, so that the p = 0 kernels are the round-1 kernels
 static TcKernel pick_drop_kernel(int mode, bool f32) {
     if (f32) {
         switch (mode) {
-            case EPI_PLAIN: return configured_kernel<EPI_PLAIN, true, false, true>();
-            case EPI_RELU: return configured_kernel<EPI_RELU, true, false, true>();
-            case EPI_SWISH: return configured_kernel<EPI_SWISH, true, false, true>();
-            case EPI_RES: return configured_kernel<EPI_RES, true, false, true>();
-            default: return configured_kernel<EPI_GENERIC, true, false, true>();
+            case EPI_PLAIN: return configured_kernel<EPI_PLAIN, true, true>();
+            case EPI_RELU: return configured_kernel<EPI_RELU, true, true>();
+            case EPI_SWISH: return configured_kernel<EPI_SWISH, true, true>();
+            case EPI_RES: return configured_kernel<EPI_RES, true, true>();
+            default: return configured_kernel<EPI_GENERIC, true, true>();
         }
     }
     switch (mode) {
-        case EPI_PLAIN: return configured_kernel<EPI_PLAIN, false, false, true>();
-        case EPI_RELU: return configured_kernel<EPI_RELU, false, false, true>();
-        case EPI_SWISH: return configured_kernel<EPI_SWISH, false, false, true>();
-        default: return configured_kernel<EPI_GENERIC, false, false, true>();
+        case EPI_PLAIN: return configured_kernel<EPI_PLAIN, false, true>();
+        case EPI_RELU: return configured_kernel<EPI_RELU, false, true>();
+        case EPI_SWISH: return configured_kernel<EPI_SWISH, false, true>();
+        default: return configured_kernel<EPI_GENERIC, false, true>();
     }
 }
 
 static int launch_tc(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mc, const CUtensorMap& mx, const TcParams& p,
-                     cudaStream_t st, const CUtensorMap* ma2 = nullptr, const CUtensorMap* mb2 = nullptr) {
+                     cudaStream_t st) {
     const bool f32 = p.c_dtype == LASR_F32;
     TcKernel kern;
     if (p.drop.thr != 0) {
-        if (p.b_stationary || p.dual || p.epi_mode == EPI_ACC || p.epi_mode == EPI_DSWISH || p.epi_mode == EPI_DRELU || p.epi_mode == EPI_DMUL) {
+        if (p.epi_mode == EPI_ACC || p.epi_mode == EPI_DSWISH || p.epi_mode == EPI_DRELU || p.epi_mode == EPI_DMUL) {
             set_error("gemm_tc: dropout is not available with this epilogue");
             return LASR_ERR_UNSUPPORTED;
         }
         kern = pick_drop_kernel(p.epi_mode, f32);
     } else {
-        kern = p.b_stationary ? pick_kernel<true>(p.epi_mode, f32) : pick_kernel<false>(p.epi_mode, f32);
+        kern = pick_kernel(p.epi_mode, f32);
     }
     if (!kern) return check_launch("gemm_tc smem attr");
-    int smem_bytes, grid;
-    if (p.b_stationary) {
-        smem_bytes = sm_ring(16) + p.bsta_bytes + p.stages * p.stage_bytes + 1024;
-        grid = sm_count() / p.tiles_n * p.tiles_n;
-    } else {
-        smem_bytes = SM_RING + p.stages * p.stage_bytes + 1024;
-        grid = p.total_units < sm_count() ? p.total_units : sm_count();
-    }
+    const int smem_bytes = SM_RING + p.stages * p.stage_bytes + 1024;
+    const int grid = p.total_units < sm_count() ? p.total_units : sm_count();
     static int pdl = -1;  // LASR_PDL=0: developer switch
     if (pdl < 0) { const char* e = getenv("LASR_PDL"); pdl = e ? atoi(e) : 1; }
     cudaLaunchConfig_t cfg = {};
@@ -1127,31 +939,22 @@ static int launch_tc(const CUtensorMap& ma, const CUtensorMap& mb, const CUtenso
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = pdl ? 1 : 0;
-    if (cudaLaunchKernelEx(&cfg, kern, ma, mb, mc, mx, ma2 ? *ma2 : ma, mb2 ? *mb2 : mb, p) != cudaSuccess) return check_launch("gemm_tc launch");
+    if (cudaLaunchKernelEx(&cfg, kern, ma, mb, mc, mx, p) != cudaSuccess) return check_launch("gemm_tc launch");
     return check_launch("gemm_tc");
 }
 
 int gemm_tc_dispatch(const lasr_gemm_args* a, cudaStream_t st) {
     const int n_store = a->n_store ? a->n_store : a->n;
     // N tiles are multiples of 32 columns: the TMA-store epilogue writes whole 32-column boxes, clipped only at the tensor edge
-    // recompute mode: two accumulators share a 256-column TMEM buffer -> N tiles of at most 128 columns
-    int bn = a->a2 ? (n_store >= 128 ? 128 : pick_bn(n_store, 64)) : pick_bn(n_store, a->trans_b ? 64 : 32);
-    if (!a->a2) {
-        // Few row tiles (the decoder: 126 x 41 = 5166 rows = 41 tiles for 148 SMs): narrower N tiles until the work units cover at
-        // least half of the SMs -- the A tile is re-read from L2 by more units, but a unit then takes proportionally less time
-        // and 41-unit launches ran on 28 % of the machine.  LASR_GEMM_FILL=0 keeps the widest tile (developer switch).
-        static int fill = -1;
-        if (fill < 0) { const char* e = getenv("LASR_GEMM_FILL"); fill = e ? atoi(e) : 1; }
-        const int gran = a->trans_b ? 64 : 32;
-        const long per_n = (long)ceil_div(a->m, BM) * (a->split_k < 1 ? 1 : a->split_k) * a->batch1 * a->batch2;
-        while (fill && per_n * ceil_div(n_store, bn) * 2 <= sm_count() && bn % (2 * gran) == 0 && bn / 2 >= 64) bn /= 2;
-    }
-    CUtensorMap ma, mb, ma2, mb2;
+    const int gran = a->trans_b ? 64 : 32;
+    int bn = pick_bn(n_store, gran);
+    // Few row tiles (the decoder: 126 x 41 = 5166 rows = 41 tiles for 148 SMs): narrower N tiles until the work units cover at
+    // least half of the SMs -- the A tile is re-read from L2 by more units, but a unit then takes proportionally less time
+    // and 41-unit launches ran on 28 % of the machine.
+    const long per_n = (long)ceil_div(a->m, BM) * (a->split_k < 1 ? 1 : a->split_k) * a->batch1 * a->batch2;
+    while (per_n * ceil_div(n_store, bn) * 2 <= sm_count() && bn % (2 * gran) == 0 && bn / 2 >= 64) bn /= 2;
+    CUtensorMap ma, mb;
     int rc;
-    if (a->a2) {
-        if ((rc = make_map(&ma2, a->a2, a->k2, a->m, a->lda2, 1, 0, 1, 0, BK, BM))) return rc;
-        if ((rc = make_map(&mb2, a->b2, a->k2, a->n, a->ldb2, 1, 0, 1, 0, BK, bn))) return rc;
-    }
     if (!a->trans_a) rc = make_map(&ma, a->a, a->k, a->m, a->lda, a->batch2, a->sa2, a->batch1, a->sa1, BK, BM);
     else rc = make_map(&ma, a->a, a->m, a->k, a->lda, a->batch2, a->sa2, a->batch1, a->sa1, 64, BK);
     if (rc) return rc;
@@ -1180,19 +983,12 @@ int gemm_tc_dispatch(const lasr_gemm_args* a, cudaStream_t st) {
     p.colsum = a->colsum; p.cs1 = a->cs1; p.cs2 = a->cs2;
     if (a->dact) p.vec_ok = p.vec_ok && ((reinterpret_cast<uintptr_t>(a->dact) & 7) == 0) && ((a->lddact * 2) % 8 == 0) && al16(a->sc1, 2) && al16(a->sc2, 2);
     if (a->colsum) p.vec_ok = p.vec_ok && ((reinterpret_cast<uintptr_t>(a->colsum) & 15) == 0) && al16(a->cs1, 4) && al16(a->cs2, 4);
-    p.dual = a->a2 ? 1 : 0;
-    p.bias2 = a->bias2;
     p.drop.state = reinterpret_cast<const unsigned long long*>(a->drop_state);
     p.drop.site = a->drop_site; p.drop.thr = a->drop_thr; p.drop.scale = a->drop_scale;
     p.drop_mark = a->drop_mark_aux;
     p.aux_deriv = a->aux_deriv;
-    {
-        static int rot = -1;  // LASR_GEMM_ROT=0: developer switch
-        if (rot < 0) { const char* e = getenv("LASR_GEMM_ROT"); rot = e ? atoi(e) : 1; }
-        p.epi_rot = (rot && ((bn + 31) / 32) % (EPI_WARPS / 4) != 0) ? 1 : 0;
-    }
-    if (a->a2) p.epi_mode = a->act == LASR_ACT_SWISH ? EPI_DUAL_DSWISH : EPI_DUAL_DRELU;
-    else if (a->accumulate) p.epi_mode = EPI_ACC;
+    p.epi_rot = ((bn + 31) / 32) % (EPI_WARPS / 4) != 0 ? 1 : 0;
+    if (a->accumulate) p.epi_mode = EPI_ACC;
     else if (a->dact && a->act == LASR_ACT_SWISH) p.epi_mode = EPI_DSWISH;
     else if (a->dact && a->act == LASR_ACT_RELU) p.epi_mode = EPI_DRELU;
     else if (a->dact && a->act == LASR_ACT_MUL) p.epi_mode = EPI_DMUL;
@@ -1203,7 +999,7 @@ int gemm_tc_dispatch(const lasr_gemm_args* a, cudaStream_t st) {
     else if (!a->res && !a->aux && a->act == LASR_ACT_NONE) p.epi_mode = EPI_PLAIN;
     else p.epi_mode = EPI_GENERIC;
     p.bn = bn;
-    p.stage_bytes = (A_BYTES + bn * BK * 2) * (p.dual ? 2 : 1);
+    p.stage_bytes = A_BYTES + bn * BK * 2;
     p.stages = SM_RING_BUDGET / p.stage_bytes;
     if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
     p.tiles_m = ceil_div(a->m, BM);
@@ -1220,37 +1016,8 @@ int gemm_tc_dispatch(const lasr_gemm_args* a, cudaStream_t st) {
     p.a_mn = a->trans_a ? 1 : 0;
     p.b_mn = a->trans_b ? 1 : 0;
     if (a->c_dtype != LASR_F32 && (p.epi_mode == EPI_RES || p.epi_mode == EPI_ACC)) p.epi_mode = EPI_GENERIC;
-    // B-stationary: short-K, unbatched, many M tiles per CTA, and an even split of the M tiles over the CTAs of an N tile
-    p.b_stationary = 0;
-    p.bsta_bytes = 0;
-    {
-        // Off by default: measured SLOWER than the streaming kernel on every C2 shape it applies to (fc1 forward 86 vs 80 us,
-        // its input gradient 131 vs 102 us at B = 126) although it moves 37 % less through L2 -- those GEMMs are bound by the
-        // epilogue / HBM write stream, not by operand fetch, and the 16-column staging doubles the TMEM-load count.
-        // LASR_GEMM_BS=1 selects it (read per call so that tests can toggle it).
-        const char* bs_env = getenv("LASR_GEMM_BS");
-        const int bs_on = bs_env ? atoi(bs_env) : 0;
-        const int total_kb = (a->k + BK - 1) / BK;
-        if (bs_on && !p.dual && p.drop.thr == 0 && total_kb <= 4 && p.split_k == 1 && !a->accumulate && a->batch1 * a->batch2 == 1 && p.tiles_n <= sm_count() / 2) {
-            const int per_n = sm_count() / p.tiles_n;                  // CTAs per N tile
-            const int rounds = (p.tiles_m + per_n - 1) / per_n;        // M tiles of the busiest CTA
-            const double eff = (double)p.tiles_m / ((double)rounds * per_n);
-            const int bsta = total_kb * bn * BK * 2;
-            const int stages = (sm_ring_budget(16) - bsta) / A_BYTES;
-            if (rounds >= 2 && eff >= 0.9 && stages >= 3) {
-                p.b_stationary = 1;
-                p.bsta_bytes = bsta;
-                p.stage_bytes = A_BYTES;
-                p.stages = stages > MAX_STAGES ? MAX_STAGES : stages;
-            }
-        }
-    }
     CUtensorMap mc, mx;
     setup_tma_epilogue(p, &mc, &mx, a->batch1, a->batch2);
-    if (p.dual) {
-        if (p.vec_ok == 0 || p.stages < 2 || (a->n & 3)) { set_error("gemm_tc: recompute mode needs 16-byte aligned C / colsum and N % 4 == 0"); return LASR_ERR_UNSUPPORTED; }
-        return launch_tc(ma, mb, mc, mx, p, st, &ma2, &mb2);
-    }
     return launch_tc(ma, mb, mc, mx, p, st);
 }
 
@@ -1328,7 +1095,7 @@ int conv2_tc_dispatch(int mode, int plane_class, const void* h1p, const void* w2
         return LASR_ERR_BAD_ARG;
     }
     p.bn = bn;
-    p.stage_bytes = (A_BYTES + bn * BK * 2) * (p.dual ? 2 : 1);
+    p.stage_bytes = A_BYTES + bn * BK * 2;
     p.stages = SM_RING_BUDGET / p.stage_bytes;
     if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
     p.tiles_m = ceil_div(p.m, BM);

@@ -406,9 +406,7 @@ int lasr_conv2_dgrad(const void* dy2p, const void* w2k, const void* h1p, void* d
 int lasr_conv2_wgrad(const void* dy2p, const void* h1p, float* dw2k, int B, int T, int F, int d, void* stream) {
     LASR_REQUIRE(dy2p && h1p && dw2k && planes_ok(d), "conv2_wgrad: bad args");
     const int T1 = (T - 3) / 2 + 1, F1 = (F - 3) / 2 + 1, U = (T1 + 1) / 2, V = (F1 + 1) / 2, T2 = (T1 - 3) / 2 + 1;
-    static int pair = -1;  // LASR_CONV2_WGRAD2=0: developer switch back to the single-CTA kernel
-    if (pair < 0) { const char* e = getenv("LASR_CONV2_WGRAD2"); pair = e ? atoi(e) : 1; }
-    if (pair && d % 256 == 0) return conv2_wgrad2_dispatch(h1p, dy2p, dw2k, B, U, V, T2, d, (cudaStream_t)stream);  // CTA pairs (gemm2_wgrad.cu)
+    if (d % 256 == 0) return conv2_wgrad2_dispatch(h1p, dy2p, dw2k, B, U, V, T2, d, (cudaStream_t)stream);  // CTA pairs (gemm2_wgrad.cu)
     return conv2_tc_dispatch(3, 0, h1p, nullptr, nullptr, dy2p, dw2k, B, U, V, T2, d, 1, (cudaStream_t)stream);
 }
 

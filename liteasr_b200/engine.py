@@ -45,20 +45,11 @@ class Engine:
         # attention score tensors that still round-trip through HBM (dprobs of every attention backward; ac / bd of the unfused
         # forward: decoder attentions, T' > 320): the operand dtype in bf16 mode -- what torch autocast's matmul hands to the softmax
         # in the reference's bf16 run -- which halves their traffic (183 -> 91 MB per tensor at C2/B=126; 0.9 % of the step).
-        # LASR_SCORES_BF16=0 keeps them in fp32.
-        self.sdt = store.adt if (store.adt == torch.bfloat16 and os.environ.get("LASR_SCORES_BF16", "1") != "0") else torch.float32
+        self.sdt = store.adt
         self.dev = store.device
         # LASR_FUSED_ATTN=0: developer switch back to GEMM -> softmax kernel -> GEMM for the rel-pos attention forward
         self.fused_attn = os.environ.get("LASR_FUSED_ATTN", "1") != "0"
         self.fused_attn_bwd = os.environ.get("LASR_FUSED_ATTN_BWD", "1") != "0"
-        self.wgrad2 = store.adt == torch.bfloat16 and os.environ.get("LASR_WGRAD2", "1") != "0"
-        # LASR_FFN_RECOMPUTE=1 (developer switch, off): fc1 of a Swish FFN does not save its pre-activation and the backward GEMM
-        # recomputes it into a second TMEM accumulator.  Saves 154 MB written + 135 MB read per FFN at C2/B=126 but measured
-        # SLOWER (32.0 vs 30.7 ms per step): two accumulators force 128-column N tiles, and at K = 256 the four operand slabs of a
-        # tile (256 KB for a 128 x 128 output) make the GEMM L2 -> shared-memory bound (1.2 GB per launch against 0.45 GB).
-        self.ffn_recompute = store.adt == torch.bfloat16 and os.environ.get("LASR_FFN_RECOMPUTE", "0") == "1"
-        # LASR_FUSED_FFN=0: developer switch back to the two separate backward GEMMs of a feed-forward block (csrc/ffn_fused.cu)
-        self.fused_ffn = store.adt == torch.bfloat16 and os.environ.get("LASR_FUSED_FFN", "1") != "0"
         # off by default: correct but measured slower than the GEMM pair (csrc/ffn_fused.cu, "STATUS")
         self.fused_ffn_fwd = store.adt == torch.bfloat16 and os.environ.get("LASR_FUSED_FFN_FWD", "0") == "1"
 
@@ -143,7 +134,7 @@ class Engine:
         """gw (N_out, K_in) += alpha * dy^T x   (split-K tcgen05 / SIMT GEMM with red.add)."""
         m, n = dy.shape
         k = x.shape[1]
-        if (self.wgrad2 and dy.dtype == torch.bfloat16 and x.dtype == torch.bfloat16 and ops.wgrad2_supported(n, k) and m >= 1024
+        if (dy.dtype == torch.bfloat16 and x.dtype == torch.bfloat16 and ops.wgrad2_supported(n, k) and m >= 1024
                 and dy.stride(0) % 8 == 0 and x.stride(0) % 8 == 0 and gw.stride(0) % 4 == 0):
             # CTA pairs (tcgen05.mma.cta_group::2): each SM stages half of both operands of a 256 x 256 tile (csrc/gemm2_wgrad.cu);
             # one work unit per pair, split-K so that the units cover the 74 pairs of the machine
@@ -153,16 +144,14 @@ class Engine:
         ops.gemm(dy, x, gw, n, k, m, lda=dy.stride(0), ldb=x.stride(0), ldc=gw.stride(0), ta=True, tb=True, accumulate=True,
                  split_k=self._split_k(n, k, m), alpha=alpha)
 
-    def dgrad(self, dy, w, *, out_dtype=None, alpha=1.0, dx_res=None, dact=None, act=ACT_NONE, colsum=None, recompute=None,
-              drop=None):
+    def dgrad(self, dy, w, *, out_dtype=None, alpha=1.0, dx_res=None, dact=None, act=ACT_NONE, colsum=None, drop=None):
         """dx = alpha * dy @ W (W stored (N_out, K_in)); optional fused activation backward (``dact``/``act``), bias-gradient
         column sum of the result (``colsum``) and fp32 accumulation into ``dx_res``."""
         m, n = dy.shape
         k = w.shape[1]
         dx = _empty((m, k), self.adt if out_dtype is None else out_dtype, self.dev) if dx_res is None else dx_res
         ops.gemm(dy, w, dx, m, k, n, lda=dy.stride(0), ldb=w.stride(0), ldc=dx.stride(0), tb=True, alpha=alpha,
-                 res=dx_res, ldres=(dx_res.stride(0) if dx_res is not None else 0), dact=dact, act=act, colsum=colsum,
-                 recompute=recompute, drop=drop)
+                 res=dx_res, ldres=(dx_res.stride(0) if dx_res is not None else 0), dact=dact, act=act, colsum=colsum, drop=drop)
         return dx
 
     def linear_bwd(self, dy, x, wname, *, need_dx=True, dx_dtype=None, bias=True, dbias_done=False, alpha=1.0, w=None,
@@ -188,10 +177,8 @@ class Engine:
         swish' (it is instruction-bound), and the inner dropout mask needs no regeneration either -- ``g`` is 0 at dropped
         elements (ReLU: the saved output is 0 there)."""
         ln = self.layernorm(x, pfx_norm, self.adt)
-        if act == ACT_SWISH and d_in is not None and self.ffn_recompute:
-            raise NotImplementedError("LASR_FFN_RECOMPUTE=1 cannot be combined with FFN dropout (the mask lives in the saved pre-activation)")
         w1, w2 = self.st.w(pfx_ff + ".fc1.weight"), self.st.w(pfx_ff + ".fc2.weight")
-        if (act == ACT_SWISH and not self.ffn_recompute and self.fused_ffn_fwd and ops.ffn_fwd_supported(w1.shape[1], w1.shape[0])
+        if (act == ACT_SWISH and self.fused_ffn_fwd and ops.ffn_fwd_supported(w1.shape[1], w1.shape[0])
                 and ln.y.stride(0) % 8 == 0 and x.stride(0) % 4 == 0):
             # ONE kernel: a and g = swish'(h) are written once, the second contraction reads a from shared memory (csrc/ffn_fused.cu)
             m, f = ln.y.shape[0], w1.shape[0]
@@ -200,9 +187,9 @@ class Engine:
             ops.ffn_fwd(ln.y, w1, self.st.p(pfx_ff + ".fc1.bias"), w2, self.st.p(pfx_ff + ".fc2.bias"), x, a, h, out, alpha=scale,
                         drop_in=d_in, drop_out=d_out)
             return NS(out=out, ln=ln, a=a, h=h, act=act, scale=scale, pfx=pfx_ff, d_in=d_in, d_out=d_out)
-        if act == ACT_SWISH and not self.ffn_recompute:
+        if act == ACT_SWISH:
             a, h = self.linear(ln.y, pfx_ff + ".fc1", self.adt, act=act, aux=True, drop=d_in, drop_mark_aux=True, aux_deriv=True)
-        else:  # ReLU: act'(.) from the output; Swish in bf16 mode: the pre-activation is recomputed in the backward GEMM
+        else:  # ReLU: act'(.) from the output
             a, h = self.linear(ln.y, pfx_ff + ".fc1", self.adt, act=act, drop=d_in), None
         out = self.linear(a, pfx_ff + ".fc2", torch.float32, res=x, alpha=scale, drop=d_out)
         return NS(out=out, ln=ln, a=a, h=h, act=act, scale=scale, pfx=pfx_ff, d_in=d_in, d_out=d_out)
@@ -215,12 +202,7 @@ class Engine:
         # dh = scale * (dy @ W2) * act'(.)  and  db1 += colsum(dh), both in the dgrad epilogue; with inner dropout the 1/(1-p)
         # factor rides on alpha and the mask is implied by the saved tensor (marker / zero)
         s_in = c.scale * (c.d_in.scale if c.d_in is not None else 1.0)
-        if c.act == ACT_SWISH and c.h is None:
-            # fc1's pre-activation is recomputed on the tensor cores inside this GEMM (second TMEM accumulator) instead of being
-            # written by the forward pass and read back: 154 MB less written and 135 MB less read per FFN at C2/B=126
-            dh = self.dgrad(dy, st.w(c.pfx + ".fc2.weight"), alpha=c.scale, act=c.act, colsum=st.g(c.pfx + ".fc1.bias"),
-                            recompute=(c.ln.y, st.w(c.pfx + ".fc1.weight"), st.p(c.pfx + ".fc1.bias")))
-        elif (c.act == ACT_SWISH and self.fused_ffn and ops.ffn_bwd_supported(dy.shape[1], c.h.shape[1]) and c.h.stride(0) % 8 == 0
+        if (c.act == ACT_SWISH and self.adt == torch.bfloat16 and ops.ffn_bwd_supported(dy.shape[1], c.h.shape[1]) and c.h.stride(0) % 8 == 0
               and dy.stride(0) % 8 == 0):
             # ONE kernel: dh = s (dy @ W2) * g, db1 += colsum(dh), dln = dh @ W1 -- dh is written once (the fc1 weight gradient
             # needs it) and never read back by the second contraction
@@ -250,9 +232,8 @@ class Engine:
         scale = dk ** -0.5
         fused = (qv is not None and drop is None and Tq == Tk and self.adt == torch.bfloat16 and self.fused_attn
                  and ops.rel_attn_fwd_supported(Tk, dk) and q.stride(0) == qv.stride(0) and k.stride(0) == v.stride(0))
-        if fused and os.environ.get("LASR_ATTN_LD64", "1") != "0":
-            ld = _ceil(Tk, 64)  # 128-byte aligned probability rows: every 128-byte piece the kernel stores is a whole line
         if fused:
+            ld = _ceil(Tk, 64)  # 128-byte aligned probability rows: every 128-byte piece the kernel stores is a whole line
             # one tcgen05 kernel: both score contractions, rel_shift, scale, mask, softmax and probs.V (csrc/attn_fused.cu)
             probs = _empty((B, H, Tq, ld), self.adt, self.dev)
             o = _empty((B * Tq, d), self.adt, self.dev)

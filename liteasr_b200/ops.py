@@ -44,7 +44,6 @@ def gemm(a: torch.Tensor, b: torch.Tensor, c: torch.Tensor, m: int, n: int, k: i
          accumulate: bool = False, split_k: int = 1, batch: Tuple[int, int] = (1, 1), sa: Tuple[int, int] = (0, 0),
          sb: Tuple[int, int] = (0, 0), sc: Tuple[int, int] = (0, 0), dact: Optional[torch.Tensor] = None,
          colsum: Optional[torch.Tensor] = None, cs: Tuple[int, int] = (0, 0), n_store: int = 0,
-         recompute: Optional[Tuple[torch.Tensor, torch.Tensor, Optional[torch.Tensor]]] = None,
          drop=None, drop_mark_aux: bool = False, aux_deriv: bool = False) -> None:
     """C[b1,b2] = alpha * act(A.B^T + bias) (+ res); see include/lasr.h ``lasr_gemm``.  ``drop`` = ``Drop`` (dropout on the
     output before the residual add) or None."""
@@ -70,14 +69,6 @@ def gemm(a: torch.Tensor, b: torch.Tensor, c: torch.Tensor, m: int, n: int, k: i
     g.colsum = colsum.data_ptr() if colsum is not None else None
     g.cs1, g.cs2 = cs
     g.n_store = n_store
-    if recompute is not None:  # (x, W, bias) of the forward Linear whose pre-activation is recomputed in the epilogue
-        x2, w2, b2 = recompute
-        _require_cuda(x2, w2, b2)
-        if x2.dtype != a.dtype or w2.dtype != a.dtype or x2.stride(1) != 1 or w2.stride(1) != 1:
-            raise TypeError("recompute operands must be row-major tensors of the operand dtype")
-        g.a2, g.b2 = x2.data_ptr(), w2.data_ptr()
-        g.bias2 = b2.data_ptr() if b2 is not None else None
-        g.lda2, g.ldb2, g.k2 = x2.stride(0), w2.stride(0), x2.shape[1]
     if drop is not None and drop.thr:
         g.drop_state, g.drop_site, g.drop_thr, g.drop_scale = drop.state.data_ptr(), drop.site, drop.thr, drop.scale
         g.drop_mark_aux = int(drop_mark_aux)

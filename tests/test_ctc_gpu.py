@@ -210,16 +210,19 @@ def test_ctc_c4_grid_vs_torch_float64(T, L, V):
     assert (grad[~live] == 0).all()
 
 
-VARIANT_SCRIPT = r'''
-import sys, torch
-sys.path.insert(0, ROOT)
-from liteasr_b200 import ops
-for (T, B, V, L) in ((300, 8, 1000, 60), (800, 64, 5000, 100), (97, 5, 333, 12)):
+@pytest.mark.parametrize("T,B,V,L", [(300, 8, 1000, 60), (800, 64, 5000, 100), (97, 5, 333, 12)])
+def test_ctc_mixed_shapes_vs_torch_float64(T, B, V, L):
+    """Batch sizes and vocabularies off the C4 grid (odd T, V not a multiple of 4, a repeated label in utterance 1)
+    against torch's float64 CTC, with a NaN-filled workspace."""
+    from liteasr_b200 import ops
     g = torch.Generator(device="cuda").manual_seed(T + V)
     x = torch.randn(T, B, V, generator=g, device="cuda")
-    il = torch.randint(int(0.6 * T), T + 1, (B,), generator=g, device="cuda"); il[0] = T
-    tl = torch.randint(L // 2, L + 1, (B,), generator=g, device="cuda"); tl[0] = L
-    tg = torch.randint(1, V, (B, L), generator=g, device="cuda"); tg[1, 1] = tg[1, 0]
+    il = torch.randint(int(0.6 * T), T + 1, (B,), generator=g, device="cuda")
+    il[0] = T
+    tl = torch.randint(L // 2, L + 1, (B,), generator=g, device="cuda")
+    tl[0] = L
+    tg = torch.randint(1, V, (B, L), generator=g, device="cuda")
+    tg[1, 1] = tg[1, 0]
     ws = torch.full((ops.ctc_workspace_bytes(T, B, L),), 0xFF, dtype=torch.uint8, device="cuda")
     nll, grad = ops.ctc_fwdbwd(x, tg, il, tl, time_major=True, workspace=ws)
     x64 = x.double().requires_grad_(True)
@@ -228,19 +231,3 @@ for (T, B, V, L) in ((300, 8, 1000, 60), (800, 64, 5000, 100), (97, 5, 333, 12))
     assert torch.isfinite(grad).all()
     assert ((nll.double() - l64).abs() / l64.abs()).max().item() < 1e-6
     assert (grad.double() - x64.grad).abs().max().item() < max(1e-4, 2e-6 * T), (T, V)
-print("VARIANT-OK")
-'''
-
-
-@pytest.mark.parametrize("env", [{"LASR_CTC_PIPE": "1"}, {"LASR_CTC_FUSED": "1"}], ids=["two_pass_pipeline", "meet_in_the_middle"])
-def test_ctc_off_by_default_variants_stay_correct(env):
-    """The two alternative CTC pipelines in csrc/ctc.cu (developer switches, both measured slower than the default: DESIGN.md)
-    are kept only as long as they are correct: each runs in a subprocess (the switch is read once per process) against
-    torch's float64 CTC."""
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    e = dict(os.environ)
-    e.update(env)
-    r = subprocess.run([sys.executable, "-c", f"ROOT = {root!r}\n" + VARIANT_SCRIPT], capture_output=True, text=True, timeout=600, env=e)
-    assert r.returncode == 0 and "VARIANT-OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]

@@ -211,49 +211,74 @@ def test_gemm_n_store_pads_with_zeros(dtype):
     assert (c[..., T:] == 0).all()
 
 
-@pytest.mark.parametrize("act", ["swish", "relu"])
-@pytest.mark.parametrize("m,n,k", [(333, 320, 256), (1000, 2048, 256), (77, 100, 64), (129, 128, 128), (4000, 1024, 256)])
-def test_gemm_recomputed_preactivation_backward(act, m, n, k):
-    """Recompute mode (bf16): C = alpha * (dy @ W2) * act'(x @ W1^T + b1) with the pre-activation rebuilt by a second MMA into
-    a second TMEM accumulator of the same tile, colsum += sum_rows C -- the FFN backward of nets/feed_forward.py:18-19 without a
-    saved pre-activation tensor.  Reference: plain torch fp32 on the same bf16-rounded operands."""
+def _swish(v):
+    return v * torch.sigmoid(v)
+
+
+def _dswish(v):
+    s = torch.sigmoid(v)
+    return s * (1 + v * (1 - s))
+
+
+# The row count of the C2 FFN GEMMs at B = 126 (m = 37 674) with K <= 256: many M tiles per CTA, for every fused epilogue.
+@pytest.mark.parametrize("m,n,k", [(37674, 256, 256), (37674, 2048, 256), (37674, 512, 200), (56000, 256, 64), (37674, 4233, 256)])
+@pytest.mark.parametrize("tb", [False, True])
+def test_gemm_c2_rows_plain_bias_bf16_and_f32(m, n, k, tb):
     from liteasr_b200 import ops
-    dtype = torch.bfloat16
     g = torch.Generator(device="cuda").manual_seed(m + n + k)
-    dy, w2 = _mk(m, k, dtype, g), _mk(k, n, dtype, g)    # W2 stored (N_out=k, K_in=n): dh = dy @ W2
-    x, w1 = _mk(m, k, dtype, g), _mk(n, k, dtype, g)     # fc1: pre = x @ W1^T + b1, W1 stored (n, k)
-    b1 = torch.randn(n, generator=g, device="cuda") * 0.3
-    cs = torch.randn(n, generator=g, device="cuda")
-    cs0 = cs.clone()
-    ld = (n + 7) // 8 * 8
-    out = torch.full((m, ld), float("nan"), device="cuda", dtype=dtype)[:, :n]
-    code = ops.ACT_SWISH if act == "swish" else ops.ACT_RELU
-    ops.gemm(dy, w2, out, m, n, k, lda=dy.stride(0), ldb=w2.stride(0), ldc=ld, tb=True, alpha=0.5, act=code, colsum=cs,
-             recompute=(x, w1, b1))
-    pre = x.float() @ w1.float().t() + b1
-    sg = torch.sigmoid(pre)
-    dact = sg * (1 + pre * (1 - sg)) if act == "swish" else (pre > 0).float()
-    ref = 0.5 * (dy.float() @ w2.float()) * dact
-    assert torch.isfinite(out.float()).all()
-    err = (out.float() - ref).abs()
-    if act == "relu":  # a pre-activation within rounding of 0 may flip the mask: exclude |pre| < 1e-3
-        err = err * (pre.abs() > 1e-3)
-        ref_cs = None
-    assert err.max().item() <= 3e-2 * max(1.0, ref.abs().max().item())
-    if act == "swish":
-        assert (cs - cs0 - ref.sum(0)).abs().max().item() <= 3e-2 * max(1.0, ref.sum(0).abs().max().item())
-    # the same values as the saved-pre-activation path it replaces (which rounds the pre-activation to bf16 first)
-    out2 = torch.empty(m, ld, device="cuda", dtype=dtype)[:, :n]
-    ops.gemm(dy, w2, out2, m, n, k, lda=dy.stride(0), ldb=w2.stride(0), ldc=ld, tb=True, alpha=0.5, dact=pre.to(dtype).contiguous(), act=code)
-    if act == "swish":
-        assert (out.float() - out2.float()).abs().max().item() <= 2e-2 * max(1.0, ref.abs().max().item())
+    x = _mk(m, k, torch.bfloat16, g)
+    w = _mk(k, n, torch.bfloat16, g) if tb else _mk(n, k, torch.bfloat16, g)
+    bias = torch.randn(n, generator=g, device="cuda")
+    ref = x.float() @ (w.float() if tb else w.float().t())
+    ldn = (n + 7) // 8 * 8
+    for cdt in (torch.bfloat16, torch.float32):
+        use_bias = not tb
+        c = torch.full((m, ldn), float("nan"), device="cuda", dtype=cdt)[:, :n]
+        ops.gemm(x, w, c, m, n, k, lda=x.stride(0), ldb=w.stride(0), ldc=c.stride(0), tb=tb, bias=bias if use_bias else None, alpha=0.5)
+        want = 0.5 * (ref + (bias if use_bias else 0.0))
+        assert torch.isfinite(c.float()).all()
+        err = (c.float() - want).abs().max().item()
+        assert err <= (3e-2 if cdt == torch.bfloat16 else 2e-3) * max(1.0, want.abs().max().item()), (cdt, err)
 
 
-def test_gemm_recompute_rejects_unsupported():
+def test_gemm_c2_rows_swish_aux_relu_res():
     from liteasr_b200 import ops
-    g = torch.Generator(device="cuda").manual_seed(0)
-    dy, w2 = _mk(64, 64, torch.float32, g), _mk(64, 128, torch.float32, g)
-    x, w1 = _mk(64, 64, torch.float32, g), _mk(128, 64, torch.float32, g)
-    out = torch.empty(64, 128, device="cuda")
-    with pytest.raises(RuntimeError):  # fp32 (SIMT) mode has no recompute path
-        ops.gemm(dy, w2, out, 64, 128, 64, lda=64, ldb=128, ldc=128, tb=True, act=ops.ACT_SWISH, recompute=(x, w1, None))
+    g = torch.Generator(device="cuda").manual_seed(11)
+    m, n, k = 37674, 2048, 256
+    x, w = _mk(m, k, torch.bfloat16, g), _mk(n, k, torch.bfloat16, g)
+    bias = torch.randn(n, generator=g, device="cuda")
+    pre = x.float() @ w.float().t() + bias
+    out = torch.empty(m, n, device="cuda", dtype=torch.bfloat16)
+    aux = torch.empty(m, n, device="cuda", dtype=torch.bfloat16)
+    ops.linear(x, w, out, bias=bias, aux=aux, act=ops.ACT_SWISH)
+    assert (aux.float() - pre).abs().max().item() <= 3e-2 * pre.abs().max().item()
+    assert (out.float() - _swish(pre)).abs().max().item() <= 3e-2 * pre.abs().max().item()
+    ops.linear(x, w, out, bias=bias, act=ops.ACT_RELU, alpha=2.0)
+    assert (out.float() - 2.0 * torch.relu(pre)).abs().max().item() <= 3e-2 * 2 * pre.abs().max().item()
+    # fp32 C with residual (N = 256: one N tile)
+    n2 = 256
+    w2 = _mk(n2, k, torch.bfloat16, g)
+    res = torch.randn(m, n2, generator=g, device="cuda")
+    o32 = torch.empty(m, n2, device="cuda")
+    ops.linear(x, w2, o32, bias=bias[:n2].contiguous(), res=res, alpha=0.5)
+    want = 0.5 * (x.float() @ w2.float().t() + bias[:n2]) + res
+    assert (o32 - want).abs().max().item() <= 2e-2 * want.abs().max().item()
+
+
+@pytest.mark.parametrize("act", ["swish", "relu"])
+def test_gemm_c2_rows_fused_activation_backward_and_colsum(act):
+    from liteasr_b200 import ops
+    g = torch.Generator(device="cuda").manual_seed(13)
+    m, n, k = 37674, 2048, 256
+    dy = _mk(m, k, torch.bfloat16, g)
+    w = _mk(k, n, torch.bfloat16, g)  # (N_out = k, K_in = n) weight, MN-major B
+    saved = _mk(m, n, torch.bfloat16, g)
+    dx = torch.empty(m, n, device="cuda", dtype=torch.bfloat16)
+    cs = torch.zeros(n, device="cuda")
+    ops.gemm(dy, w, dx, m, n, k, lda=dy.stride(0), ldb=w.stride(0), ldc=n, tb=True, alpha=0.5, dact=saved,
+             act=ops.ACT_SWISH if act == "swish" else ops.ACT_RELU, colsum=cs)
+    d = _dswish(saved.float()) if act == "swish" else (saved.float() > 0).float()
+    want = 0.5 * (dy.float() @ w.float()) * d
+    assert (dx.float() - want).abs().max().item() <= 3e-2 * max(1.0, want.abs().max().item())
+    ref_cs = want.sum(0)
+    assert (cs - ref_cs).abs().max().item() <= 2e-2 * max(1.0, ref_cs.abs().max().item()) + 0.5
