@@ -402,6 +402,7 @@ int lasr_zero(void* ptr, size_t bytes, void* stream);
  *                     exp / log (<= 1 ulp): scores may differ from the host function's in the last bits, and two hypotheses
  *                     whose scores lie within a few ulps may come out in the other order.
  * CTC Viterbi forced alignment (token timestamps) of a ragged batch: declared in include/lasr_align.h.
+ * Kaldi-compatible log-mel filterbank features of a padded batch of waveforms: declared in include/lasr_fbank.h.
  * ------------------------------------------------------------------------------------------------ */
 int lasr_logsoftmax_topk(const void* logits, int dtype, int64_t ld, int64_t rows, int V, int K, float* lse, float* logp_full,
                          int64_t ldf, float* top_val, int32_t* top_idx, void* stream);

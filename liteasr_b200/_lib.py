@@ -10,8 +10,10 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("LASR_LIB_PATH") or os.path.join(_HERE, "liblasr.so")  # LASR_LIB_PATH: developer A/B builds
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "lasr.h")
 ALIGN_HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "lasr_align.h")
+FBANK_HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "lasr_fbank.h")
 
 F32, BF16 = 0, 1
+I16 = 2  # int16 samples (include/lasr_fbank.h: LASR_I16)
 ACT_NONE, ACT_RELU, ACT_SWISH, ACT_MUL = 0, 1, 2, 3
 
 

@@ -17,6 +17,8 @@
 * ``align``                   CTC Viterbi forced alignment of known transcripts on the same encoder pass: the most likely CTC
                               path per utterance in one device launch (``lasr_ctc_forced_align``), token spans in frames and
                               seconds (defined from nets/ctc.py:25-26; the reference ships no aligner).
+* ``transcribe``              raw audio in: Kaldi-compatible log-mel features on the device (``features.fbank``, one launch),
+                              then ``decode_batch``.
 
 ``greedy_ctc(xs, xlens)`` keeps the reference's padded-batch semantics (mask mode 3, the padded rows inside the depthwise conv
 window), so its tokens can differ from those of a batch-1 call; ``decode_batch(...)["greedy"]`` has per-utterance semantics and
@@ -34,6 +36,8 @@ from torch import Tensor
 
 from . import functions as F
 from . import ops
+from .features import FbankConfig
+from .features import fbank as _fbank
 
 BEAM = 10          # models/u2.py:223 (hard-coded in the reference)
 CTC_WEIGHT = 0.5   # models/u2.py:312
@@ -199,14 +203,15 @@ def _rescore_padded(model, nbest, h: Tensor, tps: Sequence[int]):
     return _rescore(model, nbest, h.index_select(0, idx), torch.tensor([tps[u] for u in utt], dtype=torch.int64).to(dev))
 
 
-def decode_batch(model, xs: Tensor, xlens, beam: int = BEAM, timestamps: bool = False):
+def decode_batch(model, xs: Tensor, xlens, beam: int = BEAM, timestamps: bool = False, frame_shift: float = 0.01):
     """Decode a padded batch xs (B,T,F) fp32 with lengths xlens (B,): the batch-1 inference of every utterance (models/u2.py:
     221-317 on xs[b, :xlens[b]]) in one encoder pass, one top-K, one device prefix search and one decoder pass.
     -> one dict per utterance: ``best`` (token list), ``hyps`` [(prefix tuple, CTC score)], ``scores`` (rescoring scores) and
     ``greedy`` (greedy CTC tokens of the same rows, = ``greedy_ctc(x_b, None)``).  CTC scores are float64 with CUDA's exp / log:
     they may differ from the host search's in the last bits (see ``lasr_ctc_prefix_beam_search_batch``).
     ``timestamps=True`` adds ``timestamps``: ``align``'s ``tokens`` for ``best`` (token, first frame, last frame, start s, end s
-    at a 10 ms frame shift), from the same encoder pass and CTC logits (one more device launch); the other keys do not change.
+    at ``frame_shift`` seconds per input frame), from the same encoder pass and CTC logits (one more device launch); the other
+    keys do not change.
     Raises RuntimeError in training mode, ValueError for an utterance shorter than 7 frames or longer than T."""
     h, tv, ti, tps, sub, Tp, logits, lse = _ragged_topk(model, xs, xlens, beam, want_lse=timestamps)
     toks, lens, scores, count = ops.ctc_prefix_beam_search_batch(tv, ti, sub, Tp, beam=beam, blank=model.blank)
@@ -220,10 +225,28 @@ def decode_batch(model, xs: Tensor, xlens, beam: int = BEAM, timestamps: bool = 
         ys = np.full((len(best), max(len(b) for b in best)), -1, dtype=np.int64)
         for b, hy in enumerate(best):
             ys[b, : len(hy)] = hy
-        al = _align_rows(model, logits, lse, ys, [len(b) for b in best], sub, tps, Tp, 0.01)
+        al = _align_rows(model, logits, lse, ys, [len(b) for b in best], sub, tps, Tp, frame_shift)
         for o, a in zip(out, al):
             o["timestamps"] = a["tokens"]
     return out
+
+
+def transcribe(model, waves, nsamp=None, cfg: FbankConfig = FbankConfig(), beam: int = BEAM, timestamps: bool = False):
+    """Decode raw audio: ``features.fbank(waves, nsamp, cfg)`` (Kaldi-compatible log-mel features in one device launch; waves a
+    padded (B, Nmax) CUDA int16 / fp32 tensor in int16 scale with lengths nsamp, or a list of 1-D CUDA tensors), then
+    ``decode_batch`` on the features.  -> what ``decode_batch`` returns; with ``timestamps=True`` the seconds use
+    ``cfg.frame_shift``.
+    Raises ValueError when cfg.num_mel_bins differs from the encoder's input size or an utterance gives fewer than 7 feature
+    frames, and what ``features.fbank`` and ``decode_batch`` raise."""
+    if cfg.num_mel_bins != model.encoder.i_dim:
+        raise ValueError(f"cfg.num_mel_bins = {cfg.num_mel_bins}, but the encoder takes {model.encoder.i_dim} features per frame")
+    feats, flens = _fbank(waves, nsamp, cfg)
+    fl = flens.cpu()
+    for b, f in enumerate(fl.tolist()):
+        if f < 7:
+            raise ValueError(f"utterance {b} gives {f} feature frames; the encoder needs >= 7 "
+                             f"({cfg.frame_length + 6 * cfg.frame_shift:g} ms of audio)")
+    return decode_batch(model, feats, fl, beam=beam, timestamps=timestamps, frame_shift=cfg.frame_shift / 1000)
 
 
 # ----------------------------------------------------------------------------------------------

@@ -624,3 +624,29 @@ def ctc_forced_align(logits: torch.Tensor, lse: torch.Tensor, targets: torch.Ten
                                        _ptr(frames), _i(B), _i(Tmax), _i(lmax), _i(V), _i(blank), _ptr(state), _ptr(logp), _ptr(score),
                                        _ptr(spans), _ptr(ws), C.c_size_t(ws.numel()), _stream()), "ctc_forced_align")
     return state, logp, score, spans
+
+
+def fbank(wave: torch.Tensor, nsamp: torch.Tensor, frame_len: int, frame_shift: int, window: torch.Tensor, mel_lo: torch.Tensor,
+          mel_off: torch.Tensor, mel_w: torch.Tensor) -> torch.Tensor:
+    """DEVICE Kaldi log-mel filterbank of a padded batch (include/lasr_fbank.h, one launch, no host synchronisation).
+    wave (B, Nmax) int16 | fp32 in int16 scale, row stride >= Nmax; nsamp (B,) int64; frame_len / frame_shift in samples;
+    window (frame_len,) fp32; the sparse mel bank mel_lo (nb,) int32, mel_off (nb+1,) int32, mel_w (mel_off[nb],) fp32.
+    -> (B, Fmax, nb) fp32, Fmax = the frame count of Nmax, rows past each utterance's frames 0."""
+    _require_cuda(wave, nsamp, window, mel_lo, mel_off, mel_w)
+    assert wave.dim() == 2 and wave.stride(1) == 1 and nsamp.dtype == torch.int64 and nsamp.numel() == wave.shape[0]
+    assert window.dtype == torch.float32 and mel_w.dtype == torch.float32 and mel_lo.dtype == torch.int32 and mel_off.dtype == torch.int32
+    assert mel_off.numel() == mel_lo.numel() + 1
+    if wave.dtype == torch.int16:
+        code = _lib.I16
+    elif wave.dtype == torch.float32:
+        code = F32
+    else:
+        raise TypeError(f"fbank takes int16 or fp32 samples, not {wave.dtype}")
+    B, nmax = wave.shape
+    nb = mel_lo.numel()
+    fmax = 0 if nmax < frame_len else 1 + (nmax - frame_len) // frame_shift
+    out = torch.empty((B, fmax, nb), dtype=torch.float32, device=wave.device)
+    _lib.check(_lib.lib().lasr_fbank(_ptr(wave), _i(code), _l(wave.stride(0) if B > 1 else nmax), _ptr(nsamp.contiguous()), _i(B), _l(nmax),
+                                     _i(frame_len), _i(frame_shift), _ptr(window.contiguous()), _i(nb), _ptr(mel_lo.contiguous()),
+                                     _ptr(mel_off.contiguous()), _ptr(mel_w.contiguous()), _ptr(out), _stream()), "fbank")
+    return out
